@@ -3,6 +3,7 @@
 synthetic 10x-shaped data, 30,000 cells x 33,694 genes, ContinuousCellBiGan, Z = 3.
 
     python bench.py --gpus N --steps K --warmup W [--batch B] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one `trainings_step` (six RMSprop updates + two predicts, reference
 src/bigan_classify.py:126-155) on one batch of B cells per GPU.  Prints ONE JSON line.
@@ -286,6 +287,30 @@ def workload_config(args, batch):
 
 
 # ------------------------------------------------------------------------------ GPU arm
+def dump_outputs(out_dir, losses, engine, rank, sample=1 << 20):
+    """Write what the timed trainings_steps computed, for comparing two builds on the same
+    inputs: `losses.npy`, the last step's (g, e, d) losses (float64), and `<G|E|D>_weights.npy`,
+    each network's parameters after that step (float32) -- a fixed, seeded sample of `sample`
+    entries of its weight arrays (Net.get_weights order) flattened and concatenated."""
+    import numpy as np
+    out = {"losses": np.asarray(losses, dtype=np.float64)}
+    for name, n in engine.nets.items():
+        ws = n.get_weights()          # collective in data-parallel runs: every rank calls it
+        offs = np.cumsum([0] + [w.size for w in ws])
+        pos = np.sort(np.random.default_rng(0).choice(offs[-1], min(sample, offs[-1]),
+                                                      replace=False))
+        which = np.searchsorted(offs, pos, side="right") - 1
+        picked = np.empty(len(pos), dtype=np.float32)
+        for i, w in enumerate(ws):
+            m = which == i
+            picked[m] = w.reshape(-1)[pos[m] - offs[i]]
+        out[f"{name}_weights"] = picked
+    if rank == 0:
+        os.makedirs(out_dir, exist_ok=True)
+        for k, v in out.items():
+            np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -322,15 +347,16 @@ def run_ours(args):
     classify = args.workload == "classify"
     Z = Z_CLASSIFY if classify else 3
     # the public API takes the GLOBAL batch: every rank draws the same permutation(N)[:B*world]
-    # and trains on its contiguous B rows (CellTraining.run / trainings_step)
-    if classify:
-        from cellcomm_b200.bigan_classify import ClassifyCellBiGan
-        trainer = CellTraining.__new__(CellTraining)     # the reference's trainer builds the
-        trainer.batch_size, trainer.data = B * world, data   # Continuous variant only
-        trainer.batches_per_iteration = 10
-        trainer.network = ClassifyCellBiGan(Z, gene_size=args.genes)
-    else:
-        trainer = CellTraining(data, batch_size=B * world, encoding_size=Z)
+    # and trains on its contiguous B rows (CellTraining.run / trainings_step).  The trainer is
+    # assembled here rather than by CellTraining(), which builds an unseeded Continuous variant
+    # only: a fixed seed gives every run the same initial weights and device RNG key, so the
+    # outputs of two builds can be compared (--dump-outputs).
+    from cellcomm_b200.bigan_classify import ClassifyCellBiGan
+    from cellcomm_b200.bigan_cont import ContinuousCellBiGan
+    trainer = CellTraining.__new__(CellTraining)
+    trainer.batch_size, trainer.data, trainer.batches_per_iteration = B * world, data, 10
+    trainer.network = (ClassifyCellBiGan if classify else ContinuousCellBiGan)(
+        Z, gene_size=args.genes, seed=0)
     net = trainer.network
     e = net._engine
     rowptr, colidx, values = data.device_csr(dev)
@@ -397,6 +423,8 @@ def run_ours(args):
         launches = graphed.launches_per_replay * args.steps
     ms_resident = max_over_ranks(ev0.elapsed_time(ev1))
     last_losses = [float(v) for v in losses]
+    if args.dump_outputs:         # before anything else trains the networks further
+        dump_outputs(args.dump_outputs, last_losses, e, rank)
 
     # ---- the same step at the reference's default batch of 128 cells (src/__main__.py:44):
     # weight / optimiser streaming regime, HBM-bound; device-resident, same engine
@@ -1101,7 +1129,14 @@ def main():
                     help="train numbers only (tuning sweeps); the driver's runs never pass this")
     ap.add_argument("--graph", type=int, default=int(os.environ.get("CELLCOMM_BENCH_GRAPH", "1")),
                     help="1: run the device-resident loop as one CUDA graph per step")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="train / classify: after the timed steps, write the last step's losses "
+                         "and a seeded sample of the updated weights to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload not in ("train", "classify")):
+        ap.error("--dump-outputs needs --impl ours and --workload train or classify")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     if args.workload == "loader":
         run_loader(args)

@@ -43,6 +43,50 @@ def test_loader_workload_matches_the_reference_body():
     assert d["cpu_baseline"]["kind"] == "reference" and d["value"] > 0 and d["gpu_launches"] == 0
 
 
+def test_argument_checks():
+    for args in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"],
+                 ["--workload", "encode", "--dump-outputs", "d"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *args], cwd=ROOT,
+                           capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and r.stdout == "", (args, r.stderr)
+
+
+def test_dump_outputs_writes_a_fixed_sample_of_every_network(tmp_path):
+    """bench.dump_outputs on stand-in networks whose every weight holds its own flat index:
+    the sample is the same positions on every call, sorted, drawn across all arrays."""
+    import numpy as np
+    import bench
+
+    class Net:
+        def __init__(self, shapes):
+            self.arrays, n = [], 0
+            for s in shapes:
+                size = int(np.prod(s))
+                self.arrays.append(np.arange(n, n + size, dtype=np.float32).reshape(s))
+                n += size
+
+        def get_weights(self):
+            return [a.copy() for a in self.arrays]
+
+    class Engine:
+        nets = {"G": Net([(300, 200), (200,), (40,)]), "E": Net([(7, 5), (5,)]), "D": Net([(9,)])}
+
+    a, b = tmp_path / "a", tmp_path / "b"
+    bench.dump_outputs(str(a), [0.5, 0.25, 2.0], Engine(), 0, sample=1000)
+    bench.dump_outputs(str(b), [0.5, 0.25, 2.0], Engine(), 0, sample=1000)
+    assert sorted(os.listdir(a)) == ["D_weights.npy", "E_weights.npy", "G_weights.npy", "losses.npy"]
+    losses = np.load(a / "losses.npy")
+    assert losses.dtype == np.float64 and losses.tolist() == [0.5, 0.25, 2.0]
+    g = np.load(a / "G_weights.npy")
+    assert g.dtype == np.float32 and len(g) == 1000 and (np.diff(g) > 0).all()
+    assert g.max() >= 300 * 200                         # reaches past the first array
+    assert np.load(a / "E_weights.npy").tolist() == list(range(40))   # smaller than the sample
+    for name in os.listdir(a):
+        assert np.array_equal(np.load(a / name), np.load(b / name))
+    bench.dump_outputs(str(tmp_path / "c"), [0.0] * 3, Engine(), 1)   # other ranks write nothing
+    assert not (tmp_path / "c").exists()
+
+
 def test_stdout_is_parked_on_stderr_while_libraries_initialise():
     """bench.stdout_to_stderr: C-level (buffered printf) and Python-level writes made inside the
     block land on stderr; stdout keeps only what is printed afterwards."""
