@@ -10,7 +10,11 @@ The module-level names other code may import are kept (`SOURCE_IDS`, `SOURCES`, 
 `DATA_SOURCES`, `run_training`, `create_interceptors`, `check_log_dir`,
 `store_converted_cell_file`).  Environment knobs the reference does not have:
 CELLCOMM_DATA_DIR (directory of the `<source>_matrix.mtx / _barcodes.tsv / _genes.tsv`
-files, default `<repo>/data`), CELLCOMM_ITERATIONS, CELLCOMM_BATCH_SIZE.
+files, default `<repo>/data`), CELLCOMM_ITERATIONS, CELLCOMM_BATCH_SIZE, CELLCOMM_SEED.
+
+Reproducible runs: CELLCOMM_SEED=<int> seeds numpy's global state (the batch sampler) and the
+network (weights, device RNG key, host priors).  With CELLCOMM_B200_DETERMINISTIC=1 as well,
+two runs on the same data, GPU count and build write identical losses (DESIGN.md section 2).
 
 Data parallel: `torchrun --nproc-per-node N -m cellcomm_b200` (or `... src`) runs one process
 per GPU.  Every rank loads the matrix and trains on its contiguous share of each global
@@ -22,6 +26,8 @@ import os
 import signal
 import sys
 import time
+
+import numpy as np
 
 from . import intercepts
 from .cell_type_training import CellTraining, load_matrix
@@ -83,10 +89,19 @@ def init_data_parallel():
     return dist.get_rank(), dist.get_world_size()
 
 
+def env_seed():
+    """CELLCOMM_SEED as an int, or None when unset or empty."""
+    v = os.environ.get('CELLCOMM_SEED', '').strip()
+    return int(v) if v else None
+
+
 def run_training(batch_size=128):
     rank, world = init_data_parallel()
     cells = load_matrix(DATA_SOURCES['matrix'], verbose=rank == 0)
-    trainer = CellTraining(cells, batch_size=batch_size, encoding_size=ENCODING_SIZE)
+    seed = env_seed()
+    if seed is not None:
+        np.random.seed(seed)      # the batch sampler draws from numpy's global state
+    trainer = CellTraining(cells, batch_size=batch_size, encoding_size=ENCODING_SIZE, seed=seed)
     # side effects (log directory, Mongo documents, stdout) belong to rank 0 alone
     interceptors = create_interceptors(ENCODING_SIZE, trainer, DATA_SOURCES) if rank == 0 else None
     trainer.run(_env_int('CELLCOMM_ITERATIONS', 1), interceptors)

@@ -124,9 +124,13 @@ SIGNATURES = {
                                  C.POINTER(c_i32), C.POINTER(vp), C.POINTER(c_i64), vp, c_i64,
                                  c_i32, c_f32, vp, c_i64, c_i32, vp, c_i64, vp]),
     "cc_dense_wgrad": (C.c_int, [c_i32, c_i32, c_i32, vp, c_i64, vp, c_i64, vp, c_i64, c_i32, vp]),
+    "cc_reduce_ws_floats": (c_i64, [c_i64, c_i64]),
     "cc_colsum": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, c_i32, c_i32, vp]),
+    "cc_colsum_ws": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, c_i32, c_i32, vp, c_i64, vp]),
     "cc_bias_grad": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, c_i32, vp, c_i32, vp, c_i64, vp,
                                c_i64, c_i32, vp]),
+    "cc_bias_grad_ws": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, c_i32, vp, c_i32, vp, c_i64,
+                                  vp, c_i64, c_i32, vp, c_i64, vp]),
     "cc_split_bf16": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, c_i32, vp]),
     "cc_dropout": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, c_f32, vp, c_i64, c_u64, vp,
                              c_u32, c_i32, vp]),
@@ -136,11 +140,14 @@ SIGNATURES = {
     "cc_act_bwd": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, c_i32, c_i32, vp]),
     "cc_copy2d": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, c_i32, c_f32, c_i32, vp]),
     "cc_bn_stats": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, c_i32, vp]),
+    "cc_bn_stats_ws": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, c_i32, vp, c_i64, vp]),
     "cc_bn_train_apply": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, vp, c_i64, vp, vp, c_f32,
                                     c_f32, vp, vp, vp, vp, c_i32, vp]),
     "cc_bn_infer": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, vp, vp, vp, vp, c_f32, c_i32,
                               vp]),
     "cc_bn_bwd_stats": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, vp, vp, vp, c_i32, vp]),
+    "cc_bn_bwd_stats_ws": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, vp, vp, vp, c_i32, vp,
+                                     c_i64, vp]),
     "cc_bn_bwd_apply": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, vp, vp, vp, vp,
                                   c_i64, vp, vp, c_i32, vp]),
     "cc_bn_infer_bwd": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, vp, vp, c_f32, c_i32, vp]),
@@ -149,6 +156,8 @@ SIGNATURES = {
     "cc_bce_fwd_bwd": (C.c_int, [vp, c_i64, c_i64, c_i32, c_f32, c_i64, vp, vp, c_i64, c_i32, vp]),
     "cc_mse_fwd_bwd": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, c_i64, vp, vp, c_i64, c_i32,
                                  vp]),
+    "cc_mse_fwd_bwd_ws": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, c_i64, vp, vp, c_i64,
+                                    c_i32, vp, c_i64, vp]),
     "cc_round_half_even": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, c_i32, vp]),
     "cc_argmax_onehot": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, vp]),
     "cc_rmsprop_step": (C.c_int, [vp, vp, vp, vp, vp, c_i64, c_i64, c_i64, c_f32, c_f32, c_f32,

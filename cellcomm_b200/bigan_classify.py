@@ -66,8 +66,16 @@ class ClassifyCellBiGan(BasicBiGan):
                  generator_factory: Callable[[int, int], object] = _build_generator,
                  encoder_factory: Callable[[int, int], object] = _build_encoder,
                  discriminator_factory: Callable[[int, int], object] = _build_discriminator,
-                 device=None, seed=None, dist=None):
+                 device=None, seed=None, dist=None, deterministic=None):
+        """seed: the weights, the device RNG key and the host prior stream (None: random).
+        deterministic: fixed-order reductions, so that the same seed and data give the same
+        bits on every run (BiGanEngine); None reads CELLCOMM_B200_DETERMINISTIC (default 0)."""
         super().__init__(encoding_size, gene_size, generator_factory, encoder_factory, discriminator_factory)
+        if seed is not None:
+            self._prior_rng = np.random.default_rng([int(seed), 1])
+        if deterministic is None:
+            deterministic = os.environ.get("CELLCOMM_B200_DETERMINISTIC", "0") == "1"
+        self.deterministic = bool(deterministic)
         self.gene_size = gene_size
         discr_optimizer = RMSprop(learning_rate=0.0075, rho=0.85, momentum=0.1)
         self._optimizer = discr_optimizer
@@ -81,7 +89,8 @@ class ClassifyCellBiGan(BasicBiGan):
                 dist = _engine.default_dist()
             self._engine = _engine.BiGanEngine(
                 self.VARIANT, encoding_size, gene_size, max_batch=1, device=device, seed=seed,
-                dist=dist, graphs={"G": G.graph, "E": E.graph, "D": D.graph})
+                dist=dist, graphs={"G": G.graph, "E": E.graph, "D": D.graph},
+                deterministic=self.deterministic)
             for m in (G, E, D):
                 m._bind(self, self._engine)
             z = (None, encoding_size)

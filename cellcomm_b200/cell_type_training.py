@@ -225,7 +225,8 @@ def load_cells(cells_file, verbose=False):
 
 
 class CellTraining:
-    def __init__(self, data, batch_size, encoding_size, batches_per_iteration=10):
+    def __init__(self, data, batch_size, encoding_size, batches_per_iteration=10, *, seed=None):
+        """seed (not in the reference): seeds the network's weights, device RNG and priors."""
         try:
             from .bigan_cont import ContinuousCellBiGan
         except ImportError:  # imported as a top-level module (PYTHONPATH=src style)
@@ -233,7 +234,8 @@ class CellTraining:
         self.batch_size = batch_size
         self.data = data
         self.batches_per_iteration = batches_per_iteration
-        self.network = ContinuousCellBiGan(encoding_size, gene_size=self.data.shape[1])
+        kwargs = {} if seed is None else {"seed": seed}
+        self.network = ContinuousCellBiGan(encoding_size, gene_size=self.data.shape[1], **kwargs)
 
     def sample_cell_data(self, random_seed=None):
         return self.data.sample(self.batch_size, random_state=random_seed)

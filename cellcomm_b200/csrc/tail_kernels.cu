@@ -361,12 +361,19 @@ __device__ __forceinline__ void store_quad(const Mat& m, long long r, long long 
 // out[c] = sum_r f0(r,c), out[cols + c] = sum_r f1(r,c).  A block of 32 x 8 threads owns 128
 // columns (four adjacent columns per thread: a warp reads 512 B (fp32) / 256 B (bf16) of a
 // row per instruction) and strides over a slab of rows, four rows' loads in flight per
-// thread; slabs combine with atomics only when there is more than one slab (grid.y > 1).
+// thread.  With more than one slab (grid.y > 1) the slabs combine either with atomics
+// (part == nullptr: run-dependent order) or in fixed order: every CTA stores its per-column
+// partials to part[y][c] (second moment at part[grid.y + y][c]), then takes a ticket from its
+// column block's counter; the CTA that draws the last ticket sums the grid.y partials in slab
+// order 0..grid.y-1, writes (or adds to) out, and re-zeroes the counter.  No CTA waits for
+// another, so the scheme cannot deadlock on CTAs that are not resident; only WHICH CTA
+// finalises depends on timing, never the order of the additions.
 template <int MODE>  // 0: x (1 output)  1: x, x^2   2: dy, dy*xhat   3: dy*act'(y) (1 output)
 __global__ void __launch_bounds__(256)
 colreduce_kernel(const Mat a, const Mat b, long long rows, long long cols,
                  const float* __restrict__ mean, const float* __restrict__ rstd,
-                 float* __restrict__ out, int accumulate, int act,
+                 float* __restrict__ out, int accumulate, int act, float* __restrict__ part,
+                 unsigned int* __restrict__ tickets,
                  const Mat dz = Mat{nullptr, 0, 0}, const Mat dzlo = Mat{nullptr, 0, 0}) {
   __shared__ float s0[8][128], s1[8][128];
   const int tx = threadIdx.x, ty = threadIdx.y;
@@ -436,10 +443,11 @@ colreduce_kernel(const Mat a, const Mat b, long long rows, long long cols,
     s1[ty][tx * 4 + i] = acc1[i];
   }
   __syncthreads();
-  if (ty < 4) {
-    const int j = ty * 32 + tx;
-    const long long cc_ = (long long)blockIdx.x * 128 + j;
-    if (cc_ < cols && out != nullptr) {
+  constexpr bool two = MODE == 1 || MODE == 2;
+  const int j = ty * 32 + tx;  // ty < 4: one column of the block per thread
+  const long long cc_ = (long long)blockIdx.x * 128 + j;
+  if (part == nullptr) {
+    if (ty < 4 && cc_ < cols && out != nullptr) {
       float t0 = 0.f, t1 = 0.f;
 #pragma unroll
       for (int y = 0; y < 8; ++y) {
@@ -448,23 +456,60 @@ colreduce_kernel(const Mat a, const Mat b, long long rows, long long cols,
       }
       if (gridDim.y > 1 || accumulate) {
         atomicAdd(out + cc_, t0);
-        if (MODE == 1 || MODE == 2) atomicAdd(out + cols + cc_, t1);
+        if (two) atomicAdd(out + cols + cc_, t1);
       } else {
         out[cc_] = t0;
-        if (MODE == 1 || MODE == 2) out[cols + cc_] = t1;
+        if (two) out[cols + cc_] = t1;
       }
     }
+    return;
   }
+  // fixed-order combine of the slabs (out != nullptr and gridDim.y > 1 here)
+  if (ty < 4 && cc_ < cols) {
+    float t0 = 0.f, t1 = 0.f;
+#pragma unroll
+    for (int y = 0; y < 8; ++y) {
+      t0 += s0[y][j];
+      t1 += s1[y][j];
+    }
+    part[(long long)blockIdx.y * cols + cc_] = t0;
+    if (two) part[(long long)(gridDim.y + blockIdx.y) * cols + cc_] = t1;
+  }
+  __threadfence();  // partials visible device-wide before the ticket is taken
+  __syncthreads();
+  __shared__ bool last;
+  if (tx == 0 && ty == 0) last = atomicAdd(tickets + blockIdx.x, 1u) == gridDim.y - 1;
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  if (ty < 4 && cc_ < cols) {
+    float t0 = 0.f, t1 = 0.f;
+    for (unsigned y = 0; y < gridDim.y; ++y) {
+      t0 += __ldcg(part + (long long)y * cols + cc_);
+      if (two) t1 += __ldcg(part + (long long)(gridDim.y + y) * cols + cc_);
+    }
+    if (accumulate) {  // the only writer of these columns: a plain read-add-write
+      out[cc_] += t0;
+      if (two) out[cols + cc_] += t1;
+    } else {
+      out[cc_] = t0;
+      if (two) out[cols + cc_] = t1;
+    }
+  }
+  if (tx == 0 && ty == 0) tickets[blockIdx.x] = 0u;  // ready for the next launch / graph replay
 }
 
-template <int MODE>
-static int launch_colreduce(const Mat& a, const Mat& b, long long rows, long long cols,
-                            const float* mean, const float* rstd, float* out, int accumulate,
-                            cudaStream_t st, int act = 0, const Mat dz = Mat{nullptr, 0, 0},
-                            const Mat dzlo = Mat{nullptr, 0, 0}) {
-  const unsigned gx = (unsigned)((cols + 127) / 128);
+// Fixed-order reduction workspace (cc_reduce_ws_floats): reduce_tickets() uint32 counters
+// first, then the partials.  Only launches with more than one slab use it, and those have fewer
+// than 2 * SMs column blocks, so every column-block counter index is below reduce_tickets()
+// whatever the shape; the partials of one call never overlap the counters of another.
+static long long reduce_tickets() { return 2ll * num_sms(); }
+
+// the slab geometry of launch_colreduce: (column blocks, row slabs)
+static void colreduce_grid(long long rows, long long cols, unsigned& gx, unsigned& gy) {
+  gx = (unsigned)((cols + 127) / 128);
   // enough row slabs to cover ~2 waves of the machine when there are few column blocks
-  unsigned gy = 1;
+  gy = 1;
   const unsigned target = 2u * (unsigned)num_sms();
   if (gx < target) {
     gy = (target + gx - 1) / gx;
@@ -472,13 +517,44 @@ static int launch_colreduce(const Mat& a, const Mat& b, long long rows, long lon
     if (gy > maxy) gy = maxy;
     if (gy < 1) gy = 1;
   }
-  if (gy > 1 && !accumulate && out != nullptr) {
-    const long long n = ((MODE == 0 || MODE == 3) ? 1 : 2) * cols;
+}
+
+// floats of workspace one fixed-order colreduce launch uses (0: it needs none)
+static long long colreduce_ws_floats(long long rows, long long cols, int outputs) {
+  unsigned gx, gy;
+  colreduce_grid(rows, cols, gx, gy);
+  return gy > 1 ? reduce_tickets() + (long long)outputs * gy * cols : 0;
+}
+
+static long long mse_blocks(long long rows, long long cols) {
+  return ew_grid(rows * ((cols + 7) / 8), 256);
+}
+
+// ws == nullptr: slabs combine with atomics; else in fixed order through ws (ws_floats long)
+template <int MODE>
+static int launch_colreduce(const Mat& a, const Mat& b, long long rows, long long cols,
+                            const float* mean, const float* rstd, float* out, int accumulate,
+                            float* ws, long long ws_floats, cudaStream_t st, int act = 0,
+                            const Mat dz = Mat{nullptr, 0, 0}, const Mat dzlo = Mat{nullptr, 0, 0}) {
+  constexpr int outputs = (MODE == 0 || MODE == 3) ? 1 : 2;
+  unsigned gx, gy;
+  colreduce_grid(rows, cols, gx, gy);
+  // one slab, or nothing to sum (a dz-only bias_grad): each column has a single writer already
+  const bool fixed = ws != nullptr && gy > 1 && out != nullptr;
+  if (fixed) {
+    const long long need = colreduce_ws_floats(rows, cols, outputs);
+    CC_REQUIRE(ws_floats >= need,
+               "column reduction of [%lld, %lld]: workspace of %lld floats, needs %lld "
+               "(cc_reduce_ws_floats)", rows, cols, (long long)ws_floats, need);
+  } else if (gy > 1 && !accumulate && out != nullptr) {
+    const long long n = outputs * cols;
     fill_f32_kernel<<<ew_grid(n, 256), 256, 0, st>>>(out, 0.f, n);
     CC_CHECK_LAUNCH();
   }
-  colreduce_kernel<MODE><<<dim3(gx, gy), dim3(32, 8), 0, st>>>(a, b, rows, cols, mean, rstd, out,
-                                                               accumulate, act, dz, dzlo);
+  colreduce_kernel<MODE><<<dim3(gx, gy), dim3(32, 8), 0, st>>>(
+      a, b, rows, cols, mean, rstd, out, accumulate, act,
+      fixed ? ws + reduce_tickets() : nullptr, fixed ? reinterpret_cast<unsigned int*>(ws) : nullptr,
+      dz, dzlo);
   CC_CHECK_LAUNCH();
   return 0;
 }
@@ -664,8 +740,13 @@ __global__ void bce_kernel(const float* __restrict__ x, long long ldx, long long
   if (threadIdx.x == 0) atomicAdd(loss_out, acc * inv_n);
 }
 
+// part == nullptr: every block adds its partial loss with an atomic (run-dependent order);
+// else the blocks combine in fixed order like colreduce_kernel: partial to part[block], ticket,
+// and the block with the last ticket sums part[] (thread t: blocks t, t + 256, ... in order,
+// then the fixed block_sum tree), adds the total to loss_out and re-zeroes the ticket.
 __global__ void mse_kernel(const Mat pred, const Mat target, long long rows, long long cols,
-                           float inv_total, float* __restrict__ loss_out, const Mat dpred) {
+                           float inv_total, float* __restrict__ loss_out, const Mat dpred,
+                           float* __restrict__ part, unsigned int* __restrict__ ticket) {
   float acc = 0.f;
   for_each_chunk8(rows, cols, [&](long long r, long long c0, int n) {
     float a[8], t[8];
@@ -681,7 +762,26 @@ __global__ void mse_kernel(const Mat pred, const Mat target, long long rows, lon
     if (dpred.p) store8(dpred, r, c0, n, g);
   });
   acc = block_sum(acc);
-  if (threadIdx.x == 0) atomicAdd(loss_out, acc * inv_total);
+  if (part == nullptr) {
+    if (threadIdx.x == 0) atomicAdd(loss_out, acc * inv_total);
+    return;
+  }
+  __shared__ bool last;
+  if (threadIdx.x == 0) {
+    part[blockIdx.x] = acc;
+    __threadfence();
+    last = atomicAdd(ticket, 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (!last) return;
+  __threadfence();
+  float t = 0.f;
+  for (unsigned i = threadIdx.x; i < gridDim.x; i += blockDim.x) t += __ldcg(part + i);
+  t = block_sum(t);
+  if (threadIdx.x == 0) {
+    *loss_out += t * inv_total;
+    *ticket = 0u;
+  }
 }
 
 // ------------------------------------------------------------------ RMSprop (Keras, momentum>0)
@@ -772,8 +872,28 @@ using namespace cc;
     return 0;                                                                           \
   } while (0)
 
+extern "C" int64_t cc_reduce_ws_floats(int64_t rows, int64_t cols) {
+  // the largest need of any colreduce (two outputs) or MSE launch of at most rows x cols: the
+  // slab count depends on the column-block count, so every column-block count up to cols'
+  // is visited (multi-slab launches have fewer than 2 * SMs of them)
+  if (rows <= 0 || cols <= 0) return 0;
+  long long need = reduce_tickets() + mse_blocks(rows, cols);
+  const long long gx_max = (cols + 127) / 128;
+  for (long long gx = 1; gx <= gx_max && gx < reduce_tickets(); ++gx) {
+    const long long n = colreduce_ws_floats(rows, gx == gx_max ? cols : gx * 128, 2);
+    if (n > need) need = n;
+  }
+  return need;
+}
+
 extern "C" int cc_colsum(const void* x, int64_t ld, int64_t rows, int64_t cols, float* out,
                          int32_t beta, int32_t dtypes, cc_stream_t stream) {
+  return cc_colsum_ws(x, ld, rows, cols, out, beta, dtypes, nullptr, 0, stream);
+}
+
+extern "C" int cc_colsum_ws(const void* x, int64_t ld, int64_t rows, int64_t cols, float* out,
+                            int32_t beta, int32_t dtypes, float* ws, int64_t ws_floats,
+                            cc_stream_t stream) {
   if (cols <= 0) return 0;
   if (rows <= 0) {
     if (!beta) {
@@ -783,13 +903,21 @@ extern "C" int cc_colsum(const void* x, int64_t ld, int64_t rows, int64_t cols, 
     return 0;
   }
   return launch_colreduce<0>(mat(x, ld, F32(dtypes, 0)), mat(nullptr, 0, 0), rows, cols, nullptr,
-                             nullptr, out, beta, ST(stream));
+                             nullptr, out, beta, ws, ws_floats, ST(stream));
 }
 
 extern "C" int cc_bias_grad(const void* dy, int64_t lddy, const void* y, int64_t ldy, int64_t rows,
                             int64_t cols, int32_t act, float* out, int32_t beta, void* dz,
                             int64_t lddz, void* dz_lo, int64_t lddz_lo, int32_t dtypes,
                             cc_stream_t stream) {
+  return cc_bias_grad_ws(dy, lddy, y, ldy, rows, cols, act, out, beta, dz, lddz, dz_lo, lddz_lo,
+                         dtypes, nullptr, 0, stream);
+}
+
+extern "C" int cc_bias_grad_ws(const void* dy, int64_t lddy, const void* y, int64_t ldy,
+                               int64_t rows, int64_t cols, int32_t act, float* out, int32_t beta,
+                               void* dz, int64_t lddz, void* dz_lo, int64_t lddz_lo,
+                               int32_t dtypes, float* ws, int64_t ws_floats, cc_stream_t stream) {
   if (cols <= 0) return 0;
   CC_REQUIRE(out != nullptr || dz != nullptr, "cc_bias_grad: nothing to compute");
   CC_REQUIRE(dz_lo == nullptr || (dz != nullptr && !F32(dtypes, 2)),
@@ -802,7 +930,7 @@ extern "C" int cc_bias_grad(const void* dy, int64_t lddy, const void* y, int64_t
     return 0;
   }
   return launch_colreduce<3>(mat(dy, lddy, F32(dtypes, 0)), mat(y, ldy, F32(dtypes, 1)), rows, cols,
-                             nullptr, nullptr, out, beta, ST(stream), act,
+                             nullptr, nullptr, out, beta, ws, ws_floats, ST(stream), act,
                              mat(dz, lddz, F32(dtypes, 2)), mat(dz_lo, lddz_lo, 0));
 }
 
@@ -859,10 +987,15 @@ extern "C" int cc_copy2d(const void* src, int64_t lds, void* dst, int64_t ldd, i
 
 extern "C" int cc_bn_stats(const void* x, int64_t ld, int64_t rows, int64_t cols, float* sums,
                            int32_t dtypes, cc_stream_t stream) {
+  return cc_bn_stats_ws(x, ld, rows, cols, sums, dtypes, nullptr, 0, stream);
+}
+
+extern "C" int cc_bn_stats_ws(const void* x, int64_t ld, int64_t rows, int64_t cols, float* sums,
+                              int32_t dtypes, float* ws, int64_t ws_floats, cc_stream_t stream) {
   if (cols <= 0) return 0;
   CC_REQUIRE(rows > 0, "cc_bn_stats: empty batch");
   return launch_colreduce<1>(mat(x, ld, F32(dtypes, 0)), mat(nullptr, 0, 0), rows, cols, nullptr,
-                             nullptr, sums, 0, ST(stream));
+                             nullptr, sums, 0, ws, ws_floats, ST(stream));
 }
 
 extern "C" int cc_bn_train_apply(const void* x, int64_t ldx, void* y, int64_t ldy, int64_t rows,
@@ -892,10 +1025,18 @@ extern "C" int cc_bn_bwd_stats(const void* dy, int64_t lddy, const void* x, int6
                                int64_t rows, int64_t cols, const float* save_mean,
                                const float* save_rstd, float* sums2, int32_t dtypes,
                                cc_stream_t stream) {
+  return cc_bn_bwd_stats_ws(dy, lddy, x, ldx, rows, cols, save_mean, save_rstd, sums2, dtypes,
+                            nullptr, 0, stream);
+}
+
+extern "C" int cc_bn_bwd_stats_ws(const void* dy, int64_t lddy, const void* x, int64_t ldx,
+                                  int64_t rows, int64_t cols, const float* save_mean,
+                                  const float* save_rstd, float* sums2, int32_t dtypes, float* ws,
+                                  int64_t ws_floats, cc_stream_t stream) {
   if (cols <= 0) return 0;
   CC_REQUIRE(rows > 0, "cc_bn_bwd_stats: empty batch");
   return launch_colreduce<2>(mat(dy, lddy, F32(dtypes, 0)), mat(x, ldx, F32(dtypes, 1)), rows, cols,
-                             save_mean, save_rstd, sums2, 0, ST(stream));
+                             save_mean, save_rstd, sums2, 0, ws, ws_floats, ST(stream));
 }
 
 extern "C" int cc_bn_bwd_apply(const void* dy, int64_t lddy, const void* x, int64_t ldx, void* dx,
@@ -956,13 +1097,29 @@ extern "C" int cc_bce_fwd_bwd(const float* x32, int64_t ldx, int64_t rows, int32
 extern "C" int cc_mse_fwd_bwd(const void* pred, int64_t ldp, const void* target, int64_t ldt,
                               int64_t rows, int64_t cols, int64_t n_total, float* loss_out,
                               void* dpred, int64_t lddp, int32_t dtypes, cc_stream_t stream) {
+  return cc_mse_fwd_bwd_ws(pred, ldp, target, ldt, rows, cols, n_total, loss_out, dpred, lddp,
+                           dtypes, nullptr, 0, stream);
+}
+
+extern "C" int cc_mse_fwd_bwd_ws(const void* pred, int64_t ldp, const void* target, int64_t ldt,
+                                 int64_t rows, int64_t cols, int64_t n_total, float* loss_out,
+                                 void* dpred, int64_t lddp, int32_t dtypes, float* ws,
+                                 int64_t ws_floats, cc_stream_t stream) {
   CC_REQUIRE(target != nullptr, "cc_mse_fwd_bwd: no target");
   if (rows <= 0 || cols <= 0) return 0;
   const float inv_total = 1.f / ((float)n_total * (float)cols);
-  const long long work = (long long)rows * ((cols + 7) / 8);
-  mse_kernel<<<ew_grid(work, 256), 256, 0, ST(stream)>>>(
+  const long long blocks = mse_blocks(rows, cols);
+  if (ws != nullptr) {
+    const long long need = reduce_tickets() + blocks;
+    CC_REQUIRE(ws_floats >= need,
+               "cc_mse_fwd_bwd_ws of [%lld, %lld]: workspace of %lld floats, needs %lld "
+               "(cc_reduce_ws_floats)", (long long)rows, (long long)cols, (long long)ws_floats,
+               need);
+  }
+  mse_kernel<<<(unsigned)blocks, 256, 0, ST(stream)>>>(
       mat(pred, ldp, F32(dtypes, 0)), mat(target, ldt, F32(dtypes, 1)), rows, cols, inv_total,
-      loss_out, mat(dpred, lddp, F32(dtypes, 2)));
+      loss_out, mat(dpred, lddp, F32(dtypes, 2)), ws ? ws + reduce_tickets() : nullptr,
+      reinterpret_cast<unsigned int*>(ws));
   CC_CHECK_LAUNCH();
   return 0;
 }

@@ -360,6 +360,17 @@ def default_dist():
     return _NoDist()
 
 
+def _on_main_stream(reduce_kw, opt_stream):
+    """reduce_kw for a reduction about to be enqueued.  Deterministic mode shares ONE workspace
+    between all reductions of a step, which is safe only because they all run on the main
+    stream; the optimiser side stream must never run one (two reductions in flight at once
+    would mix their partials and tickets)."""
+    if reduce_kw and opt_stream is not None:
+        assert torch.cuda.current_stream(opt_stream.device) != opt_stream, \
+            "a fixed-order reduction was enqueued on the optimiser side stream"
+    return reduce_kw
+
+
 class Net:
     """One network (G, E or D): parameters in flat fused-layout buffers, activation buffers for
     up to `max_rows` rows, forward / backward / RMSprop."""
@@ -396,6 +407,12 @@ class Net:
         self._needs_cache = {}
         self._ctx = None
         self.logits32 = None
+        # {"ws": workspace} in deterministic mode (BiGanEngine): passed to every column
+        # reduction, which then sums its partials in a fixed order; {} keeps the atomic path
+        self.reduce_kw = {}
+
+    def _reduce_args(self):
+        return _on_main_stream(self.reduce_kw, self.opt_stream)
 
     # ------------------------------------------------------------------ parameters
     def _alloc_params(self, generator):
@@ -963,7 +980,7 @@ class Net:
                 y = self._buf(self.act, out)[:rows]
                 if width > 0:
                     if bn_train:
-                        ops.bn_stats(x, L["sums"])
+                        ops.bn_stats(x, L["sums"], **self._reduce_args())
                         self.dist.all_reduce(L["sums"])
                         ops.bn_train_apply(x, y, L["sums"], n_total, L["gamma"], L["beta"],
                                            BN_EPS, BN_MOMENTUM, L["moving_mean"], L["moving_var"],
@@ -1082,11 +1099,11 @@ class Net:
                     # product, in ONE pass over dy and y (frozen layers: no bias gradient)
                     dz_lo = self._buf(self.split_lo, ("dz", out))[:rows]
                     ops.bias_grad(dy, A[out], act, L["db"] if train else None, dz=dz, beta=1,
-                                  dz_lo=dz_lo)
+                                  dz_lo=dz_lo, **self._reduce_args())
                     dzs = [dz, dz_lo]
                 elif train:
                     # one pass over dy and y: dz for the GEMMs and the bias gradient
-                    ops.bias_grad(dy, A[out], act, L["db"], dz=dz, beta=1)
+                    ops.bias_grad(dy, A[out], act, L["db"], dz=dz, beta=1, **self._reduce_args())
                     dzs = [dz]
                 else:
                     ops.act_bwd(dy, A[out], dz, act)
@@ -1158,7 +1175,8 @@ class Net:
                     continue
                 x = A[i]
                 if c["bn_train"]:
-                    ops.bn_bwd_stats(dy, x, L["save_mean"], L["save_rstd"], L["sums2"])
+                    ops.bn_bwd_stats(dy, x, L["save_mean"], L["save_rstd"], L["sums2"],
+                                     **self._reduce_args())
                     if train:
                         # dgamma / dbeta from the LOCAL sums: the flat gradient all-reduce in
                         # apply_rmsprop() adds the other ranks' shares
@@ -1538,10 +1556,17 @@ class BiGanEngine:
                     8: ("D",)}
 
     def __init__(self, variant, encoding_size, gene_size, max_batch=128, device="cuda", seed=None,
-                 dist=None, graphs=None):
+                 dist=None, graphs=None, deterministic=False):
         """variant 'cont' | 'classify' picks the reference graphs and whether sub-step 7 feeds
         one_hot(argmax) (classify, src/bigan_classify.py:121-124) or the raw encoding (cont,
-        src/bigan_cont.py:55-56) to D.  `graphs` = {"G","E","D": GraphBuilder} overrides them."""
+        src/bigan_cont.py:55-56) to D.  `graphs` = {"G","E","D": GraphBuilder} overrides them.
+
+        deterministic=True: every column reduction (bias gradients, BatchNormalization
+        statistics and backward sums) and the MSE losses sum their partials in a fixed order
+        through one workspace, so a run is a pure function of its inputs and seed on a given
+        GPU count and build (DESIGN.md section 2).  One workspace serves the whole step because
+        every reduction runs on the current (main) stream; the optimiser side stream runs only
+        RMSprop sweeps and gradient exchanges."""
         if variant not in ("cont", "classify"):
             raise ValueError(f"unknown variant {variant}")
         self.variant, self.Z, self.Gn = variant, int(encoding_size), int(gene_size)
@@ -1591,8 +1616,13 @@ class BiGanEngine:
                     n.sync_compute_copy()
         self._rank_stream = (self.dist.rank & 0xFFF) << 12
         self.rng_counter = torch.zeros(1, dtype=torch.int64, device=self.device)
+        self.deterministic = bool(deterministic)
+        self.reduce_kw = {}
         self.max_batch = 0
         self.reserve(max_batch)
+
+    def _reduce_args(self):
+        return _on_main_stream(self.reduce_kw, self.G.opt_stream)   # one side stream for all nets
 
     def set_fused_optimizer(self, on, keep_grads=False):
         """Single-GPU: apply RMSprop to every Dense kernel inside its wgrad GEMM epilogue.
@@ -1619,6 +1649,15 @@ class BiGanEngine:
         self.gen_cells = None
         self.gen_enc16 = ops.alloc2d(mb, Z, device=dev)
         self.gen_enc32 = ops.alloc2d(mb, Z, dtype=torch.float32, device=dev)
+        if self.deterministic:
+            # fixed-order reduction workspace for batches of up to mb rows and the widest
+            # tensor of the three networks; zeroed, as its ticket counters must start at 0
+            widest = max(max(n.g.widths) for n in self.nets.values())
+            self.reduce_ws = torch.zeros(ops.reduce_ws_floats(mb, max(widest, self.Gn, Z)),
+                                         dtype=torch.float32, device=dev)
+            self.reduce_kw = {"ws": self.reduce_ws}
+            for n in self.nets.values():
+                n.reduce_kw = self.reduce_kw
 
     # ------------------------------------------------------------------ helpers
     def _drop_args(self, substep, net, masks):
@@ -1683,7 +1722,7 @@ class BiGanEngine:
             enc = E.forward({"cell": x16}, B, bn_train=False, **self._drop_args(2, "E", masks))
             gen = G.forward({"z": enc, "r": r}, B, bn_train=True, **self._drop_args(2, "G", masks))
             dgen = G.output_grad(B)
-            ops.mse_fwd_bwd(gen, n_total, L[1:2], target=x16, dpred=dgen)
+            ops.mse_fwd_bwd(gen, n_total, L[1:2], target=x16, dpred=dgen, **self._reduce_args())
             G.backward(dgen, train=True)
             G.apply_rmsprop()
         elif k == 3:
@@ -1701,7 +1740,8 @@ class BiGanEngine:
             gen = G.forward({"z": z, "r": r}, B, bn_train=False, **self._drop_args(4, "G", masks))
             enc = E.forward({"cell": gen}, B, bn_train=True, **self._drop_args(4, "E", masks))
             denc = E.output_grad(B)
-            ops.mse_fwd_bwd(enc, n_total, L[3:4], target=self.z32[:B], dpred=denc)
+            ops.mse_fwd_bwd(enc, n_total, L[3:4], target=self.z32[:B], dpred=denc,
+                            **self._reduce_args())
             E.backward(denc, train=True)
             E.apply_rmsprop()
         elif k == 5:

@@ -287,22 +287,41 @@ def _mask(*ts):
     return m
 
 
-def colsum(x, out32, beta=0):
+def reduce_ws_floats(rows, cols):
+    """fp32 elements of a fixed-order reduction workspace that serves every `ws=` call below
+    on at most rows x cols (zero it once before the first use; one workspace per stream)."""
+    return int(_lib.load().cc_reduce_ws_floats(int(rows), int(cols)))
+
+
+def _ws(ws):
+    """(pointer, floats) of a fixed-order reduction workspace; ws=None: the atomic path"""
+    if ws is None:
+        return None, 0
+    _req(ws, torch.float32, "ws")
+    if not ws.is_contiguous():
+        raise ValueError("cellcomm_b200.ops: ws must be contiguous")
+    return ws.data_ptr(), ws.numel()
+
+
+# colsum / bias_grad / bn_stats / bn_bwd_stats / mse_fwd_bwd: with ws (a zeroed fp32 buffer of
+# reduce_ws_floats elements) the partial sums combine in a fixed order, so the result is
+# bit-identical from run to run; without it they combine with atomics.
+def colsum(x, out32, beta=0, *, ws=None):
     _req(out32, torch.float32, "out")
-    check(_lib.load().cc_colsum(_p(x), _ld(x), x.shape[0], x.shape[1], _p(out32), int(beta),
-                                _mask(x), _stream()))
+    check(_lib.load().cc_colsum_ws(_p(x), _ld(x), x.shape[0], x.shape[1], _p(out32), int(beta),
+                                   _mask(x), *_ws(ws), _stream()))
 
 
-def bias_grad(dy, y, act, out32, dz=None, beta=0, dz_lo=None):
+def bias_grad(dy, y, act, out32, dz=None, beta=0, dz_lo=None, *, ws=None):
     """out32[c] (+)= sum_r dy[r,c] * act'(y[r,c])  (Dense bias gradient from the fp32 gradient);
     dz (optional): also store dy * act'(y) there (one pass instead of act_bwd + bias_grad);
     dz_lo (optional): and its low-order bf16 term (dz then holds the high-order one).
     out32 = None: only dz (/ dz_lo) is produced."""
     _req(out32, torch.float32, "out")
     _req(dz_lo, torch.bfloat16, "dz_lo")
-    check(_lib.load().cc_bias_grad(_p(dy), _ld(dy), _p(y), _ld(y), dy.shape[0], dy.shape[1],
-                                   int(act), _p(out32), int(beta), _p(dz), _ld(dz), _p(dz_lo),
-                                   _ld(dz_lo), _mask(dy, y, dz), _stream()))
+    check(_lib.load().cc_bias_grad_ws(_p(dy), _ld(dy), _p(y), _ld(y), dy.shape[0], dy.shape[1],
+                                      int(act), _p(out32), int(beta), _p(dz), _ld(dz), _p(dz_lo),
+                                      _ld(dz_lo), _mask(dy, y, dz), *_ws(ws), _stream()))
 
 
 def split_bf16(x, hi, lo):
@@ -361,9 +380,9 @@ def cast_bf16_to_f32(src16, dst32, scale=1.0):
     copy2d(src16, dst32, scale=scale)
 
 
-def bn_stats(x, sums):
-    check(_lib.load().cc_bn_stats(_p(x), _ld(x), x.shape[0], x.shape[1], _p(sums), _mask(x),
-                                  _stream()))
+def bn_stats(x, sums, *, ws=None):
+    check(_lib.load().cc_bn_stats_ws(_p(x), _ld(x), x.shape[0], x.shape[1], _p(sums), _mask(x),
+                                     *_ws(ws), _stream()))
 
 
 def bn_train_apply(x, y, sums, n_total, gamma, beta, eps, momentum, moving_mean, moving_var,
@@ -380,10 +399,10 @@ def bn_infer(x, y, gamma, beta, moving_mean, moving_var, eps):
                                   _mask(x, y), _stream()))
 
 
-def bn_bwd_stats(dy, x, save_mean, save_rstd, sums2):
-    check(_lib.load().cc_bn_bwd_stats(_p(dy), _ld(dy), _p(x), _ld(x), dy.shape[0], dy.shape[1],
-                                      _p(save_mean), _p(save_rstd), _p(sums2), _mask(dy, x),
-                                      _stream()))
+def bn_bwd_stats(dy, x, save_mean, save_rstd, sums2, *, ws=None):
+    check(_lib.load().cc_bn_bwd_stats_ws(_p(dy), _ld(dy), _p(x), _ld(x), dy.shape[0],
+                                         dy.shape[1], _p(save_mean), _p(save_rstd), _p(sums2),
+                                         _mask(dy, x), *_ws(ws), _stream()))
 
 
 def bn_bwd_apply(dy, x, dx, gamma, save_mean, save_rstd, sums2, n_total, dgamma=None, dbeta=None):
@@ -418,11 +437,12 @@ def bce_fwd_bwd(x32, target, n_total, loss_out, dz=None, from_logits=True):
                                      _mask(dz), _stream()))
 
 
-def mse_fwd_bwd(pred, n_total, loss_out, *, target, dpred=None):
+def mse_fwd_bwd(pred, n_total, loss_out, *, target, dpred=None, ws=None):
     _req(loss_out, torch.float32, "loss_out")
-    check(_lib.load().cc_mse_fwd_bwd(_p(pred), _ld(pred), _p(target), _ld(target), pred.shape[0],
-                                     pred.shape[1], int(n_total), _p(loss_out), _p(dpred),
-                                     _ld(dpred), _mask(pred, target, dpred), _stream()))
+    check(_lib.load().cc_mse_fwd_bwd_ws(_p(pred), _ld(pred), _p(target), _ld(target),
+                                        pred.shape[0], pred.shape[1], int(n_total), _p(loss_out),
+                                        _p(dpred), _ld(dpred), _mask(pred, target, dpred),
+                                        *_ws(ws), _stream()))
 
 
 def round_half_even(x, out16=None, out32=None):

@@ -233,9 +233,28 @@ int cc_dense_wgrad(int32_t M, int32_t K, int32_t N, const void* x, int64_t ldx, 
  * lossy there, DESIGN.md "precision policy"); GEMM operands are bf16.
  */
 
+/* Fixed-order (deterministic) column reductions and MSE loss.
+ * cc_colsum, cc_bias_grad, cc_bn_stats, cc_bn_bwd_stats and cc_mse_fwd_bwd combine the partial
+ * sums of their CTAs with float atomics, so the last bits of a result depend on scheduling.
+ * Each has a `_ws` sibling taking `float* ws, int64_t ws_floats` before the stream:
+ *  - ws == NULL: the atomic path (what the plain entry point does).
+ *  - ws != NULL: every CTA stores its partials to ws, and the CTA that finishes last sums them
+ *    in a fixed order (row slab 0, 1, ... / block 0, 1, ...).  No CTA waits for another.
+ *    Results are bit-identical for identical inputs and launch geometry (same shapes and SM
+ *    count).  The same launch geometry is used as on the atomic path, and no zero-fill launch
+ *    precedes a multi-slab call with beta == 0.
+ * Workspace contract: ws holds ws_floats floats, at least cc_reduce_ws_floats(rows, cols) for
+ * any call of at most rows x cols; a smaller one fails (cc_last_error), never falls back to
+ * atomics.  Its leading counters must be zero before the first use (zero the whole buffer
+ * once); every call leaves them zero again, also across CUDA-graph replays.  One workspace per
+ * stream: two reductions that may run at the same time must not share one. */
+int64_t cc_reduce_ws_floats(int64_t rows, int64_t cols);
+
 /* column sums into fp32: db = sum_rows dZ (Dense bias grad).  dtypes: x */
 int cc_colsum(const void* x, int64_t ld, int64_t rows, int64_t cols, float* out, int32_t beta,
               int32_t dtypes, cc_stream_t stream);
+int cc_colsum_ws(const void* x, int64_t ld, int64_t rows, int64_t cols, float* out, int32_t beta,
+                 int32_t dtypes, float* ws, int64_t ws_floats, cc_stream_t stream);
 
 /* Dense bias gradient from the fp32 upstream gradient: out[c] = sum_r dy[r,c]*act'(y[r,c]).
  * (Summing the bf16 dZ instead loses the near-cancelling sums of biases that feed a
@@ -249,6 +268,10 @@ int cc_colsum(const void* x, int64_t ld, int64_t rows, int64_t cols, float* out,
 int cc_bias_grad(const void* dy, int64_t lddy, const void* y, int64_t ldy, int64_t rows,
                  int64_t cols, int32_t act, float* out, int32_t beta, void* dz, int64_t lddz,
                  void* dz_lo, int64_t lddz_lo, int32_t dtypes, cc_stream_t stream);
+int cc_bias_grad_ws(const void* dy, int64_t lddy, const void* y, int64_t ldy, int64_t rows,
+                    int64_t cols, int32_t act, float* out, int32_t beta, void* dz, int64_t lddz,
+                    void* dz_lo, int64_t lddz_lo, int32_t dtypes, float* ws, int64_t ws_floats,
+                    cc_stream_t stream);
 /* hi = bf16(x), lo = bf16(x - hi): two-term bf16 expansion of an activation, fed to cc_gemm
  * as two accumulating segments where 8 mantissa bits are too few.  dtypes: x */
 int cc_split_bf16(const void* x, int64_t ldx, void* hi, int64_t ldhi, void* lo, int64_t ldlo,
@@ -286,6 +309,8 @@ int cc_copy2d(const void* src, int64_t lds, void* dst, int64_t ldd, int64_t rows
  * The caller may all-reduce `sums` across ranks before cc_bn_train_apply.  dtypes: x */
 int cc_bn_stats(const void* x, int64_t ld, int64_t rows, int64_t cols, float* sums,
                 int32_t dtypes, cc_stream_t stream);
+int cc_bn_stats_ws(const void* x, int64_t ld, int64_t rows, int64_t cols, float* sums,
+                   int32_t dtypes, float* ws, int64_t ws_floats, cc_stream_t stream);
 /* y = gamma*(x-mean)*rstd+beta with batch stats from sums/n_total; writes
  * mean/rstd (fp32, cols each) for backward; updates moving stats:
  * moving = momentum*moving + (1-momentum)*batch (biased variance).  dtypes: x, y */
@@ -303,6 +328,10 @@ int cc_bn_infer(const void* x, int64_t ldx, void* y, int64_t ldy, int64_t rows, 
 int cc_bn_bwd_stats(const void* dy, int64_t lddy, const void* x, int64_t ldx, int64_t rows,
                     int64_t cols, const float* save_mean, const float* save_rstd, float* sums2,
                     int32_t dtypes, cc_stream_t stream);
+int cc_bn_bwd_stats_ws(const void* dy, int64_t lddy, const void* x, int64_t ldx, int64_t rows,
+                       int64_t cols, const float* save_mean, const float* save_rstd,
+                       float* sums2, int32_t dtypes, float* ws, int64_t ws_floats,
+                       cc_stream_t stream);
 /* dx = gamma*rstd*(dy - sum_dy/n - xhat*sum_dyxhat/n); dgamma = sum_dyxhat, dbeta = sum_dy
  * (dgamma/dbeta may be NULL when the BN is not being trained; dx may be NULL).
  * dtypes: dy, x, dx */
@@ -339,6 +368,10 @@ int cc_bce_fwd_bwd(const float* x32, int64_t ldx, int64_t rows, int32_t from_log
 int cc_mse_fwd_bwd(const void* pred, int64_t ldp, const void* target, int64_t ldt, int64_t rows,
                    int64_t cols, int64_t n_total, float* loss_out, void* dpred, int64_t lddp,
                    int32_t dtypes, cc_stream_t stream);
+int cc_mse_fwd_bwd_ws(const void* pred, int64_t ldp, const void* target, int64_t ldt,
+                      int64_t rows, int64_t cols, int64_t n_total, float* loss_out, void* dpred,
+                      int64_t lddp, int32_t dtypes, float* ws, int64_t ws_floats,
+                      cc_stream_t stream);
 
 /* tf.math.round (half to even) for generate_cells, src/bigan_basic.py:40-44 */
 /* dtypes: x, out */
