@@ -8,7 +8,9 @@ not exist yet; Ctrl-C ends the process with exit status 0.
 
 The module-level names other code may import are kept (`SOURCE_IDS`, `SOURCES`, `RUN_ID`,
 `DATA_SOURCES`, `run_training`, `create_interceptors`, `check_log_dir`,
-`store_converted_cell_file`).  Environment knobs the reference does not have:
+`store_converted_cell_file`).  `generate <checkpoint.npz> <source-matrix-file> <n-cells>
+<target-matrix-file>` (not in the reference) writes n generated cells of a trained checkpoint
+as a 10x .mtx with the source matrix's gene ids.  Environment knobs the reference does not have:
 CELLCOMM_DATA_DIR (directory of the `<source>_matrix.mtx / _barcodes.tsv / _genes.tsv`
 files, default `<repo>/data`), CELLCOMM_ITERATIONS, CELLCOMM_BATCH_SIZE, CELLCOMM_SEED.
 
@@ -119,6 +121,36 @@ def store_converted_cell_file(matrix_file, cell_file):
     print('done')
 
 
+def generate_matrix_file(checkpoint_file, matrix_file, n_cells, target_file):
+    """n generated cells from a checkpoint written by save_checkpoint, as a 10x .mtx file whose
+    gene ids are the source matrix's.  One process (no data-parallel group); the checkpoint's
+    host RNG states are restored, so the same checkpoint and n always write the same file."""
+    n = int(n_cells)
+    if n < 1:
+        raise ValueError(f'n-cells must be at least 1, got {n}')
+    with np.load(checkpoint_file, allow_pickle=False) as f:
+        variant = str(f['meta/variant'])
+        encoding_size = int(f['meta/encoding_size'])
+        gene_size = int(f['meta/gene_size'])
+    source = load_matrix(matrix_file)
+    if source.shape[1] != gene_size:
+        raise ValueError(f'{checkpoint_file} generates {gene_size} genes, but {matrix_file} '
+                         f'has {source.shape[1]}')
+    if variant == 'cont':
+        from .bigan_cont import ContinuousCellBiGan as Network
+    elif variant == 'classify':
+        from .bigan_classify import ClassifyCellBiGan as Network
+    else:
+        raise ValueError(f'{checkpoint_file}: unknown network variant {variant!r}')
+    network = Network(encoding_size, gene_size)
+    network.load_checkpoint(checkpoint_file)
+    encodings = network.random_encoding_vector(n)
+    cells = network.generate_cell_matrix(encodings, columns=source.columns)
+    print('storing generated cells:', target_file, '... ', end='', flush=True)
+    cells.to_mtx(target_file)
+    print('done')
+
+
 def _stop(_signum, _frame):
     print('\tstopped')
     sys.exit(0)
@@ -127,7 +159,10 @@ def _stop(_signum, _frame):
 def main(argv):
     signal.signal(signal.SIGINT, _stop)
     commands = {'convert': (2, store_converted_cell_file,
-                            'convert <source-matrix-file> <convert-target-file>')}
+                            'convert <source-matrix-file> <convert-target-file>'),
+                'generate': (4, generate_matrix_file,
+                             'generate <checkpoint.npz> <source-matrix-file> <n-cells> '
+                             '<target-matrix-file>')}
     if len(argv) < 2:
         run_training(_env_int('CELLCOMM_BATCH_SIZE', 128))
         return

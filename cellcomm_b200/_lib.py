@@ -112,6 +112,7 @@ SIGNATURES = {
     "cc_coo_barcode": (vp, [vp]),
     "cc_coo_value": (vp, [vp]),
     "cc_coo_build_csr": (C.c_int, [vp, C.POINTER(vp)]),
+    "cc_mtx_write": (C.c_int, [C.c_char_p, c_i64, c_i64, c_i64, vp, vp, vp, vp, vp]),
     "cc_encode_scratch_bytes": (c_i64, [C.POINTER(EncodePlan)]),
     "cc_encode_stream": (C.c_int, [vp, vp, vp, c_i64, c_i64, C.POINTER(EncodePlan), vp, c_i64, vp]),
     "cc_gather_rows": (C.c_int, [vp, vp, vp, vp, c_i64, c_i64, c_i64, vp, c_i64, vp, c_i64, vp]),
@@ -159,6 +160,8 @@ SIGNATURES = {
     "cc_mse_fwd_bwd_ws": (C.c_int, [vp, c_i64, vp, c_i64, c_i64, c_i64, c_i64, vp, vp, c_i64,
                                     c_i32, vp, c_i64, vp]),
     "cc_round_half_even": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, c_i32, vp]),
+    "cc_round_csr_count": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, vp]),
+    "cc_round_csr_fill": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, vp, vp, vp]),
     "cc_argmax_onehot": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, vp]),
     "cc_rmsprop_step": (C.c_int, [vp, vp, vp, vp, vp, c_i64, c_i64, c_i64, c_f32, c_f32, c_f32,
                                   c_f32, c_f32, vp]),

@@ -62,6 +62,17 @@ class BasicBiGan:
         prediction = self._generator.predict((encoding_in, random_in))
         return np.round(prediction)          # round half to even, like tf.math.round
 
+    def generate_cell_matrix(self, encoding_in, random_in=None, columns=None):
+        """generate_cells(encoding_in, random_in) as a sparse CellMatrix: cells are rows with
+        barcode ids 1..n, genes are columns with ids `columns` (default 1..gene_size).  This is
+        the definition; engine-backed subclasses stream the same numbers without a dense
+        (n, genes) intermediate."""
+        try:
+            from .cell_type_training import CellMatrix
+        except ImportError:  # imported as a top-level module (PYTHONPATH=src style)
+            from cellcomm_b200.cell_type_training import CellMatrix
+        return CellMatrix.from_dense(self.generate_cells(encoding_in, random_in), columns=columns)
+
     @abstractmethod
     def trainings_step(self, sampled_batch):
         pass

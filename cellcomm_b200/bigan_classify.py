@@ -373,6 +373,30 @@ class ClassifyCellBiGan(BasicBiGan):
             eng.discriminate(z[s:s + m].contiguous(), tile, out[s:s + m])
         return out.cpu().numpy()
 
+    def generate_cell_matrix(self, encoding_in, random_in=None, columns=None):
+        """generate_cells(encoding_in, random_in) as a CellMatrix (barcode ids 1..n, gene ids
+        `columns`: ascending, one per gene; default 1..gene_size), streamed: every 4096-cell
+        tile of generator output is rounded and compacted to CSR rows on the device
+        (BiGanEngine.generate_csr), so device memory is bounded by one tile and only the
+        non-zeros are copied to the host.  `to_numpy(np.float32)` of the result equals
+        generate_cells() bit for bit: the same draws (random_in=None draws the noise as
+        generate_cells does), the same kernels, the same tiling.  Rank-local in data-parallel
+        runs (no collective: the weights the generator reads are replicated)."""
+        if self._engine is None:
+            return super().generate_cell_matrix(encoding_in, random_in, columns)
+        if columns is None:
+            columns = np.arange(1, self.gene_size + 1, dtype=np.int64)
+        columns = np.asarray(columns, dtype=np.int64)
+        if columns.shape != (self.gene_size,) or np.any(np.diff(columns) <= 0):
+            raise ValueError(f"columns must be {self.gene_size} ascending gene ids, got "
+                             f"shape {columns.shape}")
+        if random_in is None:
+            random_in = self.random_uniform_vector(len(encoding_in))
+        enc = np.asarray(encoding_in, dtype=np.float32)
+        rowptr, colidx, values = self._engine.generate_csr(
+            enc, np.asarray(random_in, dtype=np.float32), self.PREDICT_TILE)
+        return CellMatrix(rowptr, colidx, values, np.arange(1, len(enc) + 1), columns)
+
     def evaluate_discriminator_accuracy(self, sampled_batch):
         """(true-positives, true-negatives), reference src/bigan_basic.py:50-64 -- same draws in
         the same order (random encodings, then the generator noise), but G.predict -> round ->

@@ -181,6 +181,35 @@ class CellMatrix:
                 cells = (f"{v:.1f}" for v in row) if all_int else (repr(float(v)) for v in row)
                 f.write(str(int(self.index[i])) + "," + ",".join(cells) + "\n")
 
+    def to_mtx(self, path):
+        """Write the matrix as a 10x MatrixMarket file (`gene barcode value` lines, barcode-major,
+        float64 values written exactly) and return `path`.  The file appears atomically: it is
+        written under a temporary name in the same directory and renamed into place, so a failed
+        write leaves no partial file at `path`.
+
+        `load_matrix(m.to_mtx(p))` equals `m` (ids, CSR and float64 values) when every row and
+        every column holds at least one stored entry.  Rows and columns without one are not in
+        the file, so they vanish on reload: `load_matrix` builds the matrix from the entries,
+        like the reference's pivot_table."""
+        import ctypes as C
+        import os
+        lib = _lib.load()
+        path = os.fspath(path)
+        tmp = f"{path}.{os.getpid()}.tmp"
+        try:
+            _lib.check(lib.cc_mtx_write(tmp.encode(), len(self.index), len(self.columns),
+                                        self.nnz, self.rowptr.ctypes.data_as(C.c_void_p),
+                                        self.colidx.ctypes.data_as(C.c_void_p),
+                                        self.values64.ctypes.data_as(C.c_void_p),
+                                        self.index.ctypes.data_as(C.c_void_p),
+                                        self.columns.ctypes.data_as(C.c_void_p)))
+            os.replace(tmp, path)
+        except BaseException:
+            if os.path.exists(tmp):
+                os.remove(tmp)
+            raise
+        return path
+
     # ---------------------------------------------------------------- device residency
     def device_csr(self, device="cuda"):
         """(rowptr int64, colidx int32, values float32) resident on `device` (uploaded once)."""

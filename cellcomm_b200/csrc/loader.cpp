@@ -467,6 +467,115 @@ extern "C" int cc_coo_build_csr(const cc_coo* c, cc_csr** out) {
   return build_csr(c->t.gene.get(), c->t.barcode.get(), c->t.val.get(), c->t.nnz, out);
 }
 
+// ---- writer: host CSR -> 10x .mtx (the loader's counterpart) ----
+namespace {
+
+// integer-valued and printable as int64 (NaN / inf / |v| >= 2^63 are not)
+inline bool int_valued(double v) { return v == std::nearbyint(v) && std::fabs(v) < 9.2e18; }
+
+// decimal digits of a signed integer; returns the end of the text
+inline char* put_int(char* p, int64_t v) {
+  uint64_t u = v < 0 ? (uint64_t)0 - (uint64_t)v : (uint64_t)v;
+  if (v < 0) *p++ = '-';
+  char tmp[24];
+  int n = 0;
+  do {
+    tmp[n++] = (char)('0' + u % 10);
+    u /= 10;
+  } while (u);
+  while (n) *p++ = tmp[--n];
+  return p;
+}
+
+// one "gene barcode value\n" line: at most 20 + 1 + 20 + 1 + 25 + 1 bytes
+constexpr size_t kMaxLine = 72;
+
+}  // namespace
+
+extern "C" int cc_mtx_write(const char* path, int64_t rows, int64_t cols, int64_t nnz,
+                            const int64_t* rowptr, const int32_t* colidx, const double* values,
+                            const int64_t* row_ids, const int64_t* col_ids) {
+  if (path == nullptr || rows < 0 || cols < 0 || nnz < 0 || rowptr == nullptr ||
+      (rows > 0 && row_ids == nullptr) || (cols > 0 && col_ids == nullptr) ||
+      (nnz > 0 && (colidx == nullptr || values == nullptr))) {
+    cc::set_error("cc_mtx_write: bad arguments");
+    return -1;
+  }
+  if (rowptr[0] != 0 || rowptr[rows] != nnz) {
+    cc::set_error("cc_mtx_write: rowptr runs from %lld to %lld, expected 0 to nnz = %lld",
+                  (long long)rowptr[0], (long long)rowptr[rows], (long long)nnz);
+    return -1;
+  }
+  for (int64_t r = 0; r < rows; ++r)
+    if (rowptr[r + 1] < rowptr[r]) {
+      cc::set_error("cc_mtx_write: rowptr decreases at row %lld", (long long)r);
+      return -1;
+    }
+  const unsigned nt = nnz > (1 << 16) ? worker_threads() : 1;
+  std::vector<char> bad(nt, 0), real(nt, 0);
+  parallel_ranges(nnz, nt, [&](int64_t a, int64_t b, unsigned t) {
+    for (int64_t e = a; e < b; ++e) {
+      if (colidx[e] < 0 || colidx[e] >= cols) bad[t] = 1;
+      if (!int_valued(values[e])) real[t] = 1;
+    }
+  });
+  for (unsigned t = 0; t < nt; ++t)
+    if (bad[t]) {
+      cc::set_error("cc_mtx_write: a column index lies outside [0, %lld)", (long long)cols);
+      return -1;
+    }
+  const bool is_real = std::find(real.begin(), real.end(), 1) != real.end();
+
+  FILE* f = fopen(path, "wb");
+  if (f == nullptr) {
+    cc::set_error("cc_mtx_write: cannot open %s: %s", path, strerror(errno));
+    return -1;
+  }
+  bool ok = fprintf(f, "%%%%MatrixMarket matrix coordinate %s general\n%%\n%lld %lld %lld\n",
+                    is_real ? "real" : "integer", (long long)cols, (long long)rows,
+                    (long long)nnz) > 0;
+  // blocks of entries: the threads format their slices of a block in parallel, then the
+  // slices are written in order (bounded memory, file order = CSR order)
+  const int64_t kBlock = 1 << 20;
+  std::vector<std::vector<char>> text(nt, std::vector<char>());
+  std::vector<size_t> used(nt, 0);
+  for (int64_t e0 = 0; ok && e0 < nnz; e0 += kBlock) {
+    const int64_t e1 = std::min(nnz, e0 + kBlock);
+    parallel_ranges(e1 - e0, nt, [&](int64_t a, int64_t b, unsigned t) {
+      a += e0;
+      b += e0;
+      std::vector<char>& buf = text[t];
+      if (buf.size() < (size_t)(b - a) * kMaxLine) buf.resize((size_t)(b - a) * kMaxLine);
+      char* p = buf.data();
+      // the row of entry a: last r with rowptr[r] <= a (rows may be empty)
+      int64_t r = (int64_t)(std::upper_bound(rowptr, rowptr + rows + 1, a) - rowptr) - 1;
+      for (int64_t e = a; e < b; ++e) {
+        while (rowptr[r + 1] <= e) ++r;
+        p = put_int(p, col_ids[colidx[e]]);
+        *p++ = ' ';
+        p = put_int(p, row_ids[r]);
+        *p++ = ' ';
+        const double v = values[e];
+        if (int_valued(v))
+          p = put_int(p, (int64_t)v);
+        else
+          p += snprintf(p, 32, "%.17g", v);
+        *p++ = '\n';
+      }
+      used[t] = (size_t)(p - buf.data());
+    });
+    const unsigned parts = (e1 - e0) >= 2 ? nt : 1;   // parallel_ranges' own split
+    for (unsigned t = 0; ok && t < parts; ++t)
+      ok = fwrite(text[t].data(), 1, used[t], f) == used[t];
+  }
+  if (fclose(f) != 0) ok = false;
+  if (!ok) {
+    cc::set_error("cc_mtx_write: writing %s failed: %s", path, strerror(errno));
+    return -1;
+  }
+  return 0;
+}
+
 extern "C" void cc_csr_destroy(cc_csr* csr) { delete csr; }
 extern "C" int64_t cc_csr_rows(const cc_csr* c) { return c->rows; }
 extern "C" int64_t cc_csr_cols(const cc_csr* c) { return c->cols; }

@@ -2051,6 +2051,112 @@ class BiGanEngine:
         return self.G.forward({"z": self.z32[:rows], "r": self.r32[:rows]}, rows, bn_train=False,
                               dropout="off", out32=out32)
 
+    GENERATE_TILE = 4096      # = ClassifyCellBiGan.PREDICT_TILE: split-K depends on M, so the
+                              # streamed pass must tile exactly like G.predict to match its bits
+
+    def generate_csr(self, z32, r32, tile_rows=GENERATE_TILE, consume=None):
+        """rint(G.predict(z, r)) for every row of z32 / r32 ([n, Z] fp32, host or device) as a
+        CSR, without ever holding the dense (n, genes) output.  Per tile of `tile_rows` rows
+        (from row 0, like G.predict): the generator forward (the kernels generate() runs) into
+        one fp32 tile, cc_round_csr_count, a read-back of the tile's nnz, cc_round_csr_fill,
+        and cudaMemcpyAsync of the entries into pinned host staging on a side stream, so that
+        the copy of tile i overlaps the forward of tile i+1 (two staging sets, events).
+        Device memory: the fp32 tile plus the largest tile's entries.
+
+        Engine state (weights, BN statistics, RNG counter, loss_buf) is not touched; like
+        generate(), the pass orders itself after pending side-stream optimiser updates, and it
+        issues no collective.
+
+        consume(row0, rowptr, colidx, values) receives each finished tile (rowptr: the tile's
+        m + 1 offsets from 0, numpy; colidx / values: pinned torch views valid until the call
+        returns).  consume=None: accumulate and return the host CSR
+        (rowptr int64 [n + 1], colidx int32 [nnz], values float32 [nnz]) as numpy arrays."""
+        import numpy as np
+        dev = self.device
+        if dev.type != "cuda":
+            raise RuntimeError("generate_csr needs a CUDA device (no host fallback)")
+        z32 = torch.as_tensor(z32, dtype=torch.float32).to(dev)
+        r32 = torch.as_tensor(r32, dtype=torch.float32).to(dev)
+        n = int(z32.shape[0])
+        if tuple(z32.shape) != (n, self.Z) or tuple(r32.shape) != (n, self.Z):
+            raise ValueError(f"generate_csr: z32 / r32 must both be [n, {self.Z}]")
+        tile_rows = int(tile_rows)
+        if tile_rows < 1:
+            raise ValueError("generate_csr: tile_rows must be >= 1")
+        parts = None
+        if consume is None:
+            rowptr_out = np.zeros(n + 1, dtype=np.int64)
+            parts = []
+
+            def consume(row0, rp, col, val):
+                rowptr_out[row0 + 1:row0 + len(rp)] = rowptr_out[row0] + rp[1:]
+                # pageable copies out of the staging (torch copies on host threads)
+                parts.append((torch.empty_like(col, pin_memory=False).copy_(col),
+                              torch.empty_like(val, pin_memory=False).copy_(val)))
+
+        T = max(1, min(tile_rows, n))
+        main = torch.cuda.current_stream(dev)
+        side = getattr(self, "_gen_side", None)
+        if side is None:
+            side = self._gen_side = torch.cuda.Stream(device=dev)
+        tile = ops.alloc2d(T, self.Gn, dtype=torch.float32, device=dev, zero=False)
+        rowptr_d = torch.zeros(T + 1, dtype=torch.int64, device=dev)   # [0] stays 0: tile-local
+        rowptr_h = torch.empty(T + 1, dtype=torch.int64, pin_memory=True)
+        ent_d = None                   # (colidx, values) on the device, the largest tile's size
+        stage = [None, None]           # pinned (colidx, values), alternating between tiles
+        copied = [None, None]
+        pending = None
+
+        def finish(p):
+            slot, row0, rp, nnz = p
+            copied[slot].synchronize()
+            consume(row0, rp, stage[slot][0][:nnz], stage[slot][1][:nnz])
+
+        for i, s in enumerate(range(0, n, T)):
+            m, slot = min(T, n - s), i % 2
+            self.set_latents(z32[s:s + m], r32[s:s + m], m)
+            self.generate(m, out32=tile[:m])
+            ops.round_csr_count(tile[:m], rowptr_d[:m + 1])
+            rowptr_h[:m + 1].copy_(rowptr_d[:m + 1], non_blocking=True)
+            counted = torch.cuda.Event()
+            counted.record(main)
+            if pending is not None:      # the host takes tile i-1 while the GPU runs tile i
+                finish(pending)
+                main.wait_event(copied[pending[0]])   # its entries buffer is free again
+            counted.synchronize()
+            rp = rowptr_h[:m + 1].numpy().copy()
+            nnz = int(rp[m])
+            if ent_d is None or ent_d[0].numel() < nnz:
+                ent_d = None
+                cap = max(nnz, 1)
+                ent_d = (torch.empty(cap, dtype=torch.int32, device=dev),
+                         torch.empty(cap, dtype=torch.float32, device=dev))
+            ops.round_csr_fill(tile[:m], rowptr_d[:m + 1], ent_d[0][:nnz], ent_d[1][:nnz])
+            filled = torch.cuda.Event()
+            filled.record(main)
+            if stage[slot] is None or stage[slot][0].numel() < nnz:
+                cap = max(nnz, 1)
+                stage[slot] = (torch.empty(cap, dtype=torch.int32, pin_memory=True),
+                               torch.empty(cap, dtype=torch.float32, pin_memory=True))
+            side.wait_event(filled)
+            with torch.cuda.stream(side):
+                stage[slot][0][:nnz].copy_(ent_d[0][:nnz], non_blocking=True)
+                stage[slot][1][:nnz].copy_(ent_d[1][:nnz], non_blocking=True)
+                copied[slot] = torch.cuda.Event()
+                copied[slot].record(side)
+            pending = (slot, s, rp, nnz)
+        if pending is not None:
+            finish(pending)
+            main.wait_event(copied[pending[0]])
+        if parts is None:
+            return None
+        if parts:
+            colidx = torch.cat([c for c, _ in parts]).numpy()
+            values = torch.cat([v for _, v in parts]).numpy()
+        else:
+            colidx, values = np.zeros(0, np.int32), np.zeros(0, np.float32)
+        return rowptr_out, colidx, values
+
     def discriminate(self, z16, x16, out32):
         """D.predict -> probabilities (fp32 [rows,1])."""
         return self.D.forward({"z": z16, "cell": x16}, x16.shape[0], bn_train=False, dropout="off",

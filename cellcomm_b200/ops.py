@@ -452,6 +452,32 @@ def round_half_even(x, out16=None, out32=None):
                                          _stream()))
 
 
+def _round_csr_args(x32, rowptr):
+    _req(x32, torch.float32, "x32")
+    _req(rowptr, torch.int64, "rowptr")
+    if x32.dim() != 2 or rowptr.dim() != 1 or rowptr.shape[0] != x32.shape[0] + 1:
+        raise ValueError("round_csr: x32 is [rows, cols] and rowptr has rows + 1 entries")
+    return x32.data_ptr(), _ld(x32), x32.shape[0], x32.shape[1]
+
+
+def round_csr_count(x32, rowptr):
+    """rowptr[1 + r] = rowptr[r] + nnz(rint(x32[r])) over a dense fp32 tile; rowptr[0] is the
+    base offset the caller left there (cc_round_csr_count)."""
+    x, ld, rows, cols = _round_csr_args(x32, rowptr)
+    check(_lib.load().cc_round_csr_count(x, ld, rows, cols, rowptr.data_ptr(), _stream()))
+
+
+def round_csr_fill(x32, rowptr, colidx, values):
+    """The non-zeros of rint(x32) as CSR entries: row r's go to colidx / values
+    [rowptr[r] - rowptr[0] : rowptr[r + 1] - rowptr[0]] in ascending column order
+    (cc_round_csr_fill; rowptr from round_csr_count)."""
+    x, ld, rows, cols = _round_csr_args(x32, rowptr)
+    _req(colidx, torch.int32, "colidx")
+    _req(values, torch.float32, "values")
+    check(_lib.load().cc_round_csr_fill(x, ld, rows, cols, rowptr.data_ptr(), _p(colidx),
+                                        _p(values), _stream()))
+
+
 def argmax_onehot(p32, out16=None, out32=None):
     _req(p32, torch.float32, "p32")
     check(_lib.load().cc_argmax_onehot(_p(p32), _ld(p32), _p(out16), _ld(out16), _p(out32),

@@ -87,6 +87,18 @@ const double* cc_coo_value(const cc_coo* coo);    /* nnz */
 /* the CSR of load_matrix() from already parsed triplets (no second read of the file) */
 int cc_coo_build_csr(const cc_coo* coo, cc_csr** out);
 
+/* The loader's counterpart: write a host CSR as a 10x MatrixMarket file that cc_mtx_load_csr
+ * reads back.  Header: exactly the three lines the loader skips --
+ *   "%%MatrixMarket matrix coordinate integer general" ("real" when any value is not an
+ *   integer), "%", "<cols> <rows> <nnz>" -- then one "gene_id barcode_id value" line per stored
+ * entry (explicit zeros included), barcode-major: row r's entries in stored order, with
+ * gene_id = col_ids[colidx], barcode_id = row_ids[r].  Integer values are written as integers,
+ * all others with %.17g, so a reload is bit-exact in float64.  Lines are formatted on host
+ * threads.  The file at `path` is created or truncated; the caller makes the write atomic. */
+int cc_mtx_write(const char* path, int64_t rows, int64_t cols, int64_t nnz,
+                 const int64_t* rowptr, const int32_t* colidx, const double* values,
+                 const int64_t* row_ids, const int64_t* col_ids);
+
 /* --------------------------------------------------- batch gather (device)
  * replaces: DataFrame.sample(B) dense row gather, src/cell_type_training.py:37-38,
  * and the DataFrame -> float32 tensor feed of train_on_batch/predict.
@@ -378,6 +390,23 @@ int cc_mse_fwd_bwd_ws(const void* pred, int64_t ldp, const void* target, int64_t
 int cc_round_half_even(const void* x, int64_t ldx, void* out, int64_t ldo, float* out32,
                        int64_t ldo32, int64_t rows, int64_t cols, int32_t dtypes,
                        cc_stream_t stream);
+/* Generated cells as CSR rows (csrc/generate.cu): the rounding of generate_cells() fused with
+ * the compaction of each dense generator tile, so only the non-zeros leave the device.
+ * Deterministic: row order and in-row column order come from count -> scan -> fill, with no
+ * atomics on output positions.
+ *
+ * Round-half-even (rintf, = tf.math.round / np.round) a dense fp32 tile x[rows, cols] (leading
+ * dimension ldx) and count the non-zero results per row.  rowptr[0] holds a base offset on
+ * entry (device memory, so consecutive tiles chain without the host); on return
+ * rowptr[1 + r] = rowptr[r] + nnz(row r).  Columns [cols, ldx) are never read as entries.
+ * "Non-zero" means rintf(x) != 0: -0.0 and every value in [-0.5, 0.5] count as zero. */
+int cc_round_csr_count(const float* x, int64_t ldx, int64_t rows, int64_t cols,
+                       int64_t* rowptr, cc_stream_t stream);
+/* Write the entries counted above: row r's non-zeros, in ascending column order, go to
+ * colidx[rowptr[r] - rowptr[0] + k] / values[...] (buffers are local to this call, rowptr is
+ * global).  values are the rounded fp32 numbers. */
+int cc_round_csr_fill(const float* x, int64_t ldx, int64_t rows, int64_t cols,
+                      const int64_t* rowptr, int32_t* colidx, float* values, cc_stream_t stream);
 /* to_categorical(argmax(p,-1)): src/bigan_classify.py:121-124 */
 int cc_argmax_onehot(const float* p32, int64_t ldp, void* out16, int64_t ldo, float* out32,
                      int64_t ldo32, int64_t rows, int64_t cols, cc_stream_t stream);
