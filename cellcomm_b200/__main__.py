@@ -10,9 +10,14 @@ The module-level names other code may import are kept (`SOURCE_IDS`, `SOURCES`, 
 `DATA_SOURCES`, `run_training`, `create_interceptors`, `check_log_dir`,
 `store_converted_cell_file`).  `generate <checkpoint.npz> <source-matrix-file> <n-cells>
 <target-matrix-file>` (not in the reference) writes n generated cells of a trained checkpoint
-as a 10x .mtx with the source matrix's gene ids.  Environment knobs the reference does not have:
-CELLCOMM_DATA_DIR (directory of the `<source>_matrix.mtx / _barcodes.tsv / _genes.tsv`
-files, default `<repo>/data`), CELLCOMM_ITERATIONS, CELLCOMM_BATCH_SIZE, CELLCOMM_SEED.
+as a 10x .mtx with the source matrix's gene ids.  `score <checkpoint.npz> <source-matrix-file>
+<matrix-file> <scores.csv>` (not in the reference) scores every cell of a matrix with a trained
+checkpoint: one CSV row `barcode,mse,d-real,z0,...` per cell (reconstruction error,
+discriminator probability, encoding; `BasicBiGan.score_cells`).  Environment knobs the
+reference does not have: CELLCOMM_DATA_DIR (directory of the `<source>_matrix.mtx /
+_barcodes.tsv / _genes.tsv` files, default `<repo>/data`), CELLCOMM_ITERATIONS,
+CELLCOMM_BATCH_SIZE, CELLCOMM_SEED, and CELLCOMM_VALIDATION_MATRIX=<file.mtx>: held-out cells
+(read against the same genes.tsv) scored after every iteration into `validation.csv`.
 
 Reproducible runs: CELLCOMM_SEED=<int> seeds numpy's global state (the batch sampler) and the
 network (weights, device RNG key, host priors).  With CELLCOMM_B200_DETERMINISTIC=1 as well,
@@ -59,18 +64,25 @@ def check_log_dir(log_dir):
 
 
 def create_interceptors(encoding_size, trainer, sources):
-    """stdout losses + losses.csv + the MongoDB recorder (every iteration from the first)."""
+    """stdout losses + losses.csv + the MongoDB recorder (every iteration from the first), and
+    with CELLCOMM_VALIDATION_MATRIX set, validation.csv: that matrix, aligned to the training
+    matrix's gene ids, scored after every iteration."""
+    validation_file = os.environ.get('CELLCOMM_VALIDATION_MATRIX', '').strip()
+    held_out = None
+    if validation_file:
+        held_out = load_matrix(validation_file).reindex_columns(trainer.data.columns)
     full_run_id = f"{time.strftime('%m-%d-%H%M')}_{RUN_ID}_e{encoding_size}"
     log_dir = os.path.join('logs', full_run_id)
     check_log_dir(log_dir)
     recorder = intercepts.DbRecorder(RUN_ID, sources)
     recorder.setup()
     record = intercepts.skip_iterations(1, recorder.create_interceptor(trainer))
-    return intercepts.combined_interceptors((
-        intercepts.print_losses(full_run_id),
-        intercepts.SinkIntercepts(log_dir).save_losses(),
-        intercepts.offset_iterations(0, record),
-    ))
+    sink = intercepts.SinkIntercepts(log_dir)
+    chain = [intercepts.print_losses(full_run_id), sink.save_losses(),
+             intercepts.offset_iterations(0, record)]
+    if held_out is not None:
+        chain.append(sink.save_validation(trainer, held_out))
+    return intercepts.combined_interceptors(chain)
 
 
 def init_data_parallel():
@@ -121,20 +133,18 @@ def store_converted_cell_file(matrix_file, cell_file):
     print('done')
 
 
-def generate_matrix_file(checkpoint_file, matrix_file, n_cells, target_file):
-    """n generated cells from a checkpoint written by save_checkpoint, as a 10x .mtx file whose
-    gene ids are the source matrix's.  One process (no data-parallel group); the checkpoint's
-    host RNG states are restored, so the same checkpoint and n always write the same file."""
-    n = int(n_cells)
-    if n < 1:
-        raise ValueError(f'n-cells must be at least 1, got {n}')
+def _restore_network(checkpoint_file, matrix_file, verb):
+    """-> (the network of a checkpoint written by save_checkpoint, the source matrix).  The
+    variant and sizes come from the checkpoint; the source's gene count is checked before a
+    network is built.  One process (no data-parallel group); the checkpoint's host RNG states
+    are restored with the weights, so what follows draws the same numbers every time."""
     with np.load(checkpoint_file, allow_pickle=False) as f:
         variant = str(f['meta/variant'])
         encoding_size = int(f['meta/encoding_size'])
         gene_size = int(f['meta/gene_size'])
     source = load_matrix(matrix_file)
     if source.shape[1] != gene_size:
-        raise ValueError(f'{checkpoint_file} generates {gene_size} genes, but {matrix_file} '
+        raise ValueError(f'{checkpoint_file} {verb} {gene_size} genes, but {matrix_file} '
                          f'has {source.shape[1]}')
     if variant == 'cont':
         from .bigan_cont import ContinuousCellBiGan as Network
@@ -144,10 +154,52 @@ def generate_matrix_file(checkpoint_file, matrix_file, n_cells, target_file):
         raise ValueError(f'{checkpoint_file}: unknown network variant {variant!r}')
     network = Network(encoding_size, gene_size)
     network.load_checkpoint(checkpoint_file)
+    return network, source
+
+
+def generate_matrix_file(checkpoint_file, matrix_file, n_cells, target_file):
+    """n generated cells from a checkpoint written by save_checkpoint, as a 10x .mtx file whose
+    gene ids are the source matrix's.  The same checkpoint and n always write the same file."""
+    n = int(n_cells)
+    if n < 1:
+        raise ValueError(f'n-cells must be at least 1, got {n}')
+    network, source = _restore_network(checkpoint_file, matrix_file, 'generates')
     encodings = network.random_encoding_vector(n)
     cells = network.generate_cell_matrix(encodings, columns=source.columns)
     print('storing generated cells:', target_file, '... ', end='', flush=True)
     cells.to_mtx(target_file)
+    print('done')
+
+
+def write_score_file(path, barcodes, scores):
+    """`barcode,mse,d-real,z0,...,z{Z-1}`, one row per cell; floats as %.9g (round-trips
+    float32).  The file appears atomically: written under a temporary name in the same
+    directory and renamed into place, so a failed write leaves no partial file at `path`."""
+    Z = scores.encodings.shape[1]
+    tmp = f'{path}.{os.getpid()}.tmp'
+    try:
+        with open(tmp, 'w') as f:
+            f.write(','.join(['barcode', 'mse', 'd-real'] + [f'z{k}' for k in range(Z)]) + '\n')
+            for b, m, d, z in zip(barcodes, scores.mse, scores.d_real, scores.encodings):
+                f.write(f'{int(b)},' + ','.join('%.9g' % float(v) for v in (m, d, *z)) + '\n')
+        os.replace(tmp, path)
+    except BaseException:
+        if os.path.exists(tmp):
+            os.remove(tmp)
+        raise
+    return path
+
+
+def score_matrix_file(checkpoint_file, matrix_file, cells_file, scores_file):
+    """Score every cell of `cells_file` with a checkpoint written by save_checkpoint and write
+    the CSV of write_score_file.  The cells are aligned to the source matrix's gene ids first
+    (CellMatrix.reindex_columns: genes the source lacks are dropped, missing ones are zero).
+    The same checkpoint and cells always write the same file."""
+    network, source = _restore_network(checkpoint_file, matrix_file, 'scores')
+    cells = load_matrix(cells_file).reindex_columns(source.columns)
+    scores = network.score_cells(cells)
+    print('storing cell scores:', scores_file, '... ', end='', flush=True)
+    write_score_file(scores_file, cells.index, scores)
     print('done')
 
 
@@ -162,7 +214,10 @@ def main(argv):
                             'convert <source-matrix-file> <convert-target-file>'),
                 'generate': (4, generate_matrix_file,
                              'generate <checkpoint.npz> <source-matrix-file> <n-cells> '
-                             '<target-matrix-file>')}
+                             '<target-matrix-file>'),
+                'score': (4, score_matrix_file,
+                          'score <checkpoint.npz> <source-matrix-file> <matrix-file> '
+                          '<scores.csv>')}
     if len(argv) < 2:
         run_training(_env_int('CELLCOMM_BATCH_SIZE', 128))
         return

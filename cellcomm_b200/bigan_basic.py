@@ -4,6 +4,7 @@ injected factories return (the reference's tests inject MagicMocks, test/bigans_
 12-18), so this base class only relies on `.predict`, `.summary` and `.layers`.
 """
 from abc import abstractmethod
+from collections import namedtuple
 from typing import Callable
 
 import numpy as np
@@ -13,6 +14,9 @@ try:
 except ImportError:  # pragma: no cover
     def final(f):
         return f
+
+# per-cell scores of score_cells: encodings [n, Z], mse [n], d_real [n], all float32
+CellScores = namedtuple("CellScores", ["encodings", "mse", "d_real"])
 
 
 class BasicBiGan:
@@ -72,6 +76,25 @@ class BasicBiGan:
         except ImportError:  # imported as a top-level module (PYTHONPATH=src style)
             from cellcomm_b200.cell_type_training import CellMatrix
         return CellMatrix.from_dense(self.generate_cells(encoding_in, random_in), columns=columns)
+
+    def score_cells(self, cell_data, random_in=None):
+        """Per-cell scores of a trained network on cells it may never have seen -> CellScores:
+            encodings = encoding_prediction(cell_data)                        (z)
+            mse       = mean over genes of (G.predict((z, random_in)) - x)^2  (the cycle loss of
+                        the generator-with-encoder sub-step, per cell, before rounding)
+            d_real    = D.predict((z, cell_data))                   (the real pair's probability)
+        random_in=None draws the generator noise with random_uniform_vector, as generate_cells
+        does.  This is the definition; engine-backed subclasses stream the same numbers without
+        a dense (n, genes) intermediate."""
+        encodings = self.encoding_prediction(cell_data)
+        if random_in is None:
+            random_in = self.random_uniform_vector(len(encodings))
+        prediction = self._generator.predict((encodings, random_in))
+        diff = np.asarray(prediction, dtype=np.float64) - np.asarray(cell_data, dtype=np.float64)
+        mse = np.mean(np.square(diff, out=diff), axis=-1)
+        d_real = self._discriminator.predict((encodings, cell_data))
+        return CellScores(np.asarray(encodings, dtype=np.float32), mse.astype(np.float32),
+                          np.asarray(d_real, dtype=np.float32).reshape(-1))
 
     @abstractmethod
     def trainings_step(self, sampled_batch):

@@ -15,12 +15,12 @@ from typing import Callable
 import numpy as np
 
 try:
-    from .bigan_basic import BasicBiGan
+    from .bigan_basic import BasicBiGan, CellScores
     from . import engine as _engine
     from .models import NetModel, RMSprop, losses, activations  # noqa: F401
     from .cell_type_training import CellBatch, CellMatrix
 except ImportError:  # imported as top-level modules (PYTHONPATH=src style)
-    from bigan_basic import BasicBiGan
+    from bigan_basic import BasicBiGan, CellScores
     from cellcomm_b200 import engine as _engine
     from cellcomm_b200.models import NetModel, RMSprop, losses, activations  # noqa: F401
     from cellcomm_b200.cell_type_training import CellBatch, CellMatrix
@@ -396,6 +396,35 @@ class ClassifyCellBiGan(BasicBiGan):
         rowptr, colidx, values = self._engine.generate_csr(
             enc, np.asarray(random_in, dtype=np.float32), self.PREDICT_TILE)
         return CellMatrix(rowptr, colidx, values, np.arange(1, len(enc) + 1), columns)
+
+    def score_cells(self, cell_data, random_in=None):
+        """BasicBiGan.score_cells, streamed on the device (BiGanEngine.score_stream): per
+        4096-cell tile the encoder, the generator into one fp32 tile, its squared error against
+        the exact counts (cc_recon_sqerr) and the discriminator, so device memory is bounded by
+        one tile and only the (n, Z + 2) scores are copied to the host.  A CellMatrix is scored
+        as it is; anything else (CellBatch, array, DataFrame-like) is first wrapped with
+        CellMatrix.from_dense.  encodings and d_real equal encoding_prediction /
+        D.predict((z, cells)) bit for bit (same kernels, same tiling); random_in=None draws the
+        noise as generate_cells does.  Rank-local in data-parallel runs (no collective: the
+        weights the three nets read are replicated)."""
+        if self._engine is None:
+            return super().score_cells(cell_data, random_in)
+        import torch
+        mat = cell_data if isinstance(cell_data, CellMatrix) else CellMatrix.from_dense(cell_data)
+        if mat.shape[1] != self.gene_size:
+            raise ValueError(f"expected cells with {self.gene_size} genes, got {mat.shape[1]}")
+        n = len(mat)
+        if random_in is None:
+            random_in = self.random_uniform_vector(n)
+        eng = self._engine
+        dev = eng.device
+        enc = torch.empty((n, self.encoding_size), dtype=torch.float32, device=dev)
+        mse = torch.empty(n, dtype=torch.float32, device=dev)
+        d_real = torch.empty(n, dtype=torch.float32, device=dev)
+        rowptr, colidx, values = mat.device_csr(dev)
+        eng.score_stream(rowptr, colidx, values, 0, n, np.asarray(random_in, dtype=np.float32),
+                         enc, mse, d_real, self.PREDICT_TILE)
+        return CellScores(enc.cpu().numpy(), mse.cpu().numpy(), d_real.cpu().numpy())
 
     def evaluate_discriminator_accuracy(self, sampled_batch):
         """(true-positives, true-negatives), reference src/bigan_basic.py:50-64 -- same draws in

@@ -163,6 +163,28 @@ class CellMatrix:
     def to_numpy(self, dtype=np.float64):
         return self.dense_rows(np.arange(len(self)), dtype)
 
+    def reindex_columns(self, columns):
+        """This matrix with gene ids exactly `columns` (ascending): the entries of genes not in
+        `columns` are dropped, and genes of `columns` the matrix lacks become empty columns --
+        the CSR of DataFrame.reindex(columns=columns, fill_value=0), float64 values unchanged.
+        Gene ids are the .mtx gene indices, so this aligns matrices read against one genes.tsv
+        (e.g. a held-out sample to the training matrix's genes).  Host only."""
+        columns = np.ascontiguousarray(columns, dtype=np.int64)
+        if columns.ndim != 1 or np.any(np.diff(columns) <= 0):
+            raise ValueError("reindex_columns: columns must be ascending, unique gene ids")
+        # old column j -> its position in `columns`, or -1 when the gene is dropped
+        pos = np.searchsorted(columns, self.columns)
+        hit = pos < len(columns)
+        hit[hit] = columns[pos[hit]] == self.columns[hit]
+        new_col = np.where(hit, pos, -1)
+        mapped = new_col[self.colidx]
+        keep = mapped >= 0
+        kept_before = np.zeros(self.nnz + 1, dtype=np.int64)      # kept entries before entry e
+        np.cumsum(keep, out=kept_before[1:])
+        rowptr = kept_before[self.rowptr]
+        # the old and new ids are both ascending, so the map keeps every row's column order
+        return CellMatrix(rowptr, mapped[keep], self.values64[keep], self.index.copy(), columns)
+
     @property
     def values(self):
         return self.to_numpy()

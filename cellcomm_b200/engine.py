@@ -2157,6 +2157,57 @@ class BiGanEngine:
             colidx, values = np.zeros(0, np.int32), np.zeros(0, np.float32)
         return rowptr_out, colidx, values
 
+    def score_stream(self, rowptr, colidx, values, row_begin, row_end, r32, enc_out, mse_out,
+                     d_out, tile_rows=GENERATE_TILE):
+        """Per-cell scores of rows [row_begin, row_end) of a device CSR with gene_size columns:
+            enc_out[i] = E.predict(x)                      ([n, Z] fp32, device)
+            mse_out[i] = mean_c (G.predict(z, r) - x)^2    ([n] fp32, device; G's fp32 output
+                                                            against the exact fp32 counts)
+            d_out[i]   = D.predict(z, x)                   ([n] or [n, 1] fp32, device)
+        with z = enc_out[i] and r = r32[i] ([n, Z] fp32, host or device).  Per tile of
+        `tile_rows` rows from row_begin (the tiling of E / G / D.predict, so the bits match):
+        encode_stream into z, set_latents(z, r) + generate() into one fp32 tile,
+        cc_recon_sqerr with scale 1 / gene_size, cc_gather_rows into one bf16 cell tile, and
+        discriminate(z, x).  Device memory: those two tiles and the nets' activations for
+        tile_rows rows; nothing of size (n, genes).
+
+        Engine state (weights, BN statistics, RNG counter, loss_buf) is not touched; every
+        forward orders itself after pending side-stream optimiser updates of its net, and the
+        pass issues no collective."""
+        dev = self.device
+        if dev.type != "cuda":
+            raise RuntimeError("score_stream needs a CUDA device (no host fallback)")
+        row_begin, row_end = int(row_begin), int(row_end)
+        n = row_end - row_begin
+        if row_begin < 0 or n < 0 or row_end > rowptr.shape[0] - 1:
+            raise ValueError(f"score_stream: rows [{row_begin}, {row_end}) outside the CSR's "
+                             f"{rowptr.shape[0] - 1} rows")
+        r32 = torch.as_tensor(r32, dtype=torch.float32).to(dev)
+        if tuple(r32.shape) != (n, self.Z) or tuple(enc_out.shape) != (n, self.Z):
+            raise ValueError(f"score_stream: r32 and enc_out must be [{n}, {self.Z}]")
+        if mse_out.numel() != n or d_out.numel() != n:
+            raise ValueError(f"score_stream: mse_out and d_out must hold {n} values")
+        tile_rows = int(tile_rows)
+        if tile_rows < 1:
+            raise ValueError("score_stream: tile_rows must be >= 1")
+        if n == 0:
+            return
+        T = min(tile_rows, n)
+        pred = ops.alloc2d(T, self.Gn, dtype=torch.float32, device=dev, zero=False)
+        cells = ops.alloc2d(T, self.Gn, device=dev)     # zero padding, like the predict tiles
+        mse, d = mse_out.view(n), d_out.view(n, 1)
+        for s in range(0, n, T):
+            m, row = min(T, n - s), row_begin + s
+            z = enc_out[s:s + m]
+            self.encode_stream(rowptr, colidx, values, row, row + m, z)
+            self.set_latents(z, r32[s:s + m], m)
+            self.generate(m, out32=pred[:m])
+            ops.recon_sqerr(pred[:m], rowptr, colidx, values, row, mse[s:s + m],
+                            scale=1.0 / self.Gn)
+            ops.gather_rows(rowptr, colidx, values, self.Gn, row_start=row, n_rows=m,
+                            out16=cells[:m])
+            self.discriminate(z, cells[:m], d[s:s + m])
+
     def discriminate(self, z16, x16, out32):
         """D.predict -> probabilities (fp32 [rows,1])."""
         return self.D.forward({"z": z16, "cell": x16}, x16.shape[0], bn_train=False, dropout="off",

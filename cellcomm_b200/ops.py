@@ -478,6 +478,25 @@ def round_csr_fill(x32, rowptr, colidx, values):
                                         _p(values), _stream()))
 
 
+def recon_sqerr(pred32, rowptr, colidx, values, row0, out, scale=1.0):
+    """out[r] = scale * sum_c (pred32[r, c] - x[row0 + r, c])^2 for a dense fp32 tile against
+    rows of a device CSR with pred32.shape[1] columns (cc_recon_sqerr)."""
+    _req(pred32, torch.float32, "pred32")
+    _req(rowptr, torch.int64, "rowptr")
+    _req(colidx, torch.int32, "colidx")
+    _req(values, torch.float32, "values")
+    _req(out, torch.float32, "out")
+    if pred32.dim() != 2 or out.numel() != pred32.shape[0] or not out.is_contiguous():
+        raise ValueError("recon_sqerr: pred32 is [rows, cols] and out holds rows contiguous floats")
+    rows, cols = pred32.shape
+    if rows and int(row0) + rows >= rowptr.shape[0]:
+        raise ValueError(f"recon_sqerr: rows [{int(row0)}, {int(row0) + rows}) lie outside the "
+                         f"CSR's {rowptr.shape[0] - 1} rows")
+    check(_lib.load().cc_recon_sqerr(pred32.data_ptr(), _ld(pred32), rows, cols,
+                                     rowptr.data_ptr(), colidx.data_ptr(), values.data_ptr(),
+                                     int(row0), float(scale), out.data_ptr(), _stream()))
+
+
 def argmax_onehot(p32, out16=None, out32=None):
     _req(p32, torch.float32, "p32")
     check(_lib.load().cc_argmax_onehot(_p(p32), _ld(p32), _p(out16), _ld(out16), _p(out32),

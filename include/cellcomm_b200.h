@@ -407,6 +407,17 @@ int cc_round_csr_count(const float* x, int64_t ldx, int64_t rows, int64_t cols,
  * global).  values are the rounded fp32 numbers. */
 int cc_round_csr_fill(const float* x, int64_t ldx, int64_t rows, int64_t cols,
                       const int64_t* rowptr, int32_t* colidx, float* values, cc_stream_t stream);
+/* Per-cell reconstruction error for the score pass (csrc/score.cu):
+ *   out[r] = scale * sum_{c < cols} (pred[r, c] - x[row0 + r, c])^2,   r in [0, rows)
+ * pred: dense fp32 [rows, cols] tile, leading dimension ld (columns [cols, ld) are never
+ * counted).  x: the device CSR (rowptr int64, colidx int32, values fp32) of a matrix with
+ * `cols` columns; entries must have unique columns within a row, an explicit zero counts once.
+ * Every term is a non-negative square (no expanded form), summed in a fixed order without
+ * global atomics, so the result is a pure function of the inputs.  One CTA per row, a bitmap
+ * of the row's stored columns in shared memory: cols is capped at 262,144 (an error above). */
+int cc_recon_sqerr(const float* pred, int64_t ld, int64_t rows, int64_t cols,
+                   const int64_t* rowptr, const int32_t* colidx, const float* values, int64_t row0,
+                   float scale, float* out, cc_stream_t stream);
 /* to_categorical(argmax(p,-1)): src/bigan_classify.py:121-124 */
 int cc_argmax_onehot(const float* p32, int64_t ldp, void* out16, int64_t ldo, float* out32,
                      int64_t ldo32, int64_t rows, int64_t cols, cc_stream_t stream);
