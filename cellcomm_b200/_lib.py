@@ -163,6 +163,8 @@ SIGNATURES = {
     "cc_round_csr_count": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, vp]),
     "cc_round_csr_fill": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, vp, vp, vp]),
     "cc_recon_sqerr": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, vp, vp, c_i64, c_f32, vp, vp]),
+    "cc_col_moments": (C.c_int, [vp, c_i64, c_i64, c_i64, c_i32, vp, vp, vp, vp, c_i64, vp]),
+    "cc_col_moments_ws_bytes": (c_i64, [c_i64, c_i64]),
     "cc_argmax_onehot": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, vp]),
     "cc_rmsprop_step": (C.c_int, [vp, vp, vp, vp, vp, c_i64, c_i64, c_i64, c_f32, c_f32, c_f32,
                                   c_f32, c_f32, vp]),

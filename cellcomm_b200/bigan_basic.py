@@ -18,6 +18,101 @@ except ImportError:  # pragma: no cover
 # per-cell scores of score_cells: encodings [n, Z], mse [n], d_real [n], all float32
 CellScores = namedtuple("CellScores", ["encodings", "mse", "d_real"])
 
+# per-group, per-gene statistics of gene_statistics: cells int64 [K]; mean, var (unbiased) and
+# detected (fraction of the group's cells where the gene is non-zero) float64 [K, genes]
+GeneStatistics = namedtuple("GeneStatistics", ["cells", "mean", "var", "detected"])
+
+# compare_cells: the real cells' and the generated cells' GeneStatistics, same groups
+CellComparison = namedtuple("CellComparison", ["real", "generated"])
+
+# one row of comparison_summary per group
+GroupSummary = namedtuple("GroupSummary", [
+    "group", "real_cells", "generated_cells", "real_library_size", "generated_library_size",
+    "real_genes_detected", "generated_genes_detected", "log1p_mean_r", "detected_r"])
+
+
+def statistics_from_sums(cells, s1, s2, nonzero):
+    """GeneStatistics of K groups from their cell counts n [K] and per-gene sums S1 = sum v,
+    S2 = sum v^2 and nonzero counts [K, genes]:
+        mean = S1 / n,  var = max(S2 - S1 * S1 / n, 0) / (n - 1),  detected = nonzero / n
+    var is NaN for n <= 1, every value NaN for an empty group.  Every path (the dense
+    definitions and the streamed device passes) ends here, so they agree bit for bit whenever
+    their sums do."""
+    n = np.array(cells, dtype=np.int64).reshape(-1)
+    s1 = np.asarray(s1, dtype=np.float64)
+    s2 = np.asarray(s2, dtype=np.float64)
+    nz = np.asarray(nonzero, dtype=np.int64)
+    if s1.ndim != 2 or s1.shape[0] != len(n) or s2.shape != s1.shape or nz.shape != s1.shape:
+        raise ValueError("statistics_from_sums: cells is [K] and the sums are [K, genes]")
+    nn = n.astype(np.float64)[:, None]
+    with np.errstate(divide="ignore", invalid="ignore"):
+        mean = s1 / nn
+        var = np.maximum(s2 - s1 * s1 / nn, 0.0) / (nn - 1)
+        detected = nz / nn
+    var[n <= 1] = np.nan
+    mean[n == 0] = np.nan
+    detected[n == 0] = np.nan
+    return GeneStatistics(n, mean, var, detected)
+
+
+def group_labels(groups, n_groups, n):
+    """(int64 labels [n], K) of gene_statistics' grouping: groups=None puts every cell in group
+    0 (K = n_groups or 1); otherwise one integer label in [0, K) per cell, K = n_groups or
+    max(label) + 1."""
+    if groups is None:
+        labels = np.zeros(n, dtype=np.int64)
+        K = 1 if n_groups is None else int(n_groups)
+    else:
+        labels = np.asarray(groups)
+        if labels.ndim != 1 or len(labels) != n:
+            raise ValueError(f"groups must hold one label per cell ({n}), got shape "
+                             f"{labels.shape}")
+        if len(labels) and not np.issubdtype(labels.dtype, np.integer):
+            raise ValueError(f"groups must be integer labels, got {labels.dtype}")
+        labels = labels.astype(np.int64)
+        K = int(n_groups) if n_groups is not None else (int(labels.max()) + 1 if n else 1)
+        if n and (labels.min() < 0 or labels.max() >= K):
+            raise ValueError(f"group labels must lie in [0, {K})")
+    if K < 1:
+        raise ValueError(f"n_groups must be at least 1, got {K}")
+    return labels, K
+
+
+def require_sorted(labels):
+    """generated_gene_statistics streams its rows in order: each group must be one run."""
+    if np.any(np.diff(labels) < 0):
+        raise ValueError("generated_gene_statistics: rows must be sorted by group")
+
+
+def _pearson(a, b):
+    """Pearson r of two vectors in fp64; NaN when either holds a NaN or is constant."""
+    a = np.asarray(a, dtype=np.float64)
+    b = np.asarray(b, dtype=np.float64)
+    if len(a) < 2 or np.isnan(a).any() or np.isnan(b).any():
+        return float("nan")
+    da, db = a - a.mean(), b - b.mean()
+    den = np.sqrt(np.dot(da, da) * np.dot(db, db))
+    return float(np.dot(da, db) / den) if den > 0 else float("nan")
+
+
+def comparison_summary(comparison):
+    """One GroupSummary per group of a CellComparison: the real and generated cell counts, the
+    mean library size (sum over genes of the mean count), the mean number of genes detected
+    per cell (sum over genes of the detection rate), and the Pearson r over genes, real vs
+    generated, of log1p(mean) and of the detection rate.  NaN where a group is empty or a
+    vector is constant."""
+    real, gen = comparison
+    rows = []
+    with np.errstate(invalid="ignore"):
+        for k in range(len(real.cells)):
+            rows.append(GroupSummary(
+                k, int(real.cells[k]), int(gen.cells[k]),
+                float(np.sum(real.mean[k])), float(np.sum(gen.mean[k])),
+                float(np.sum(real.detected[k])), float(np.sum(gen.detected[k])),
+                _pearson(np.log1p(real.mean[k]), np.log1p(gen.mean[k])),
+                _pearson(real.detected[k], gen.detected[k])))
+    return rows
+
 
 class BasicBiGan:
     def __init__(self, encoding_size, gene_size,
@@ -95,6 +190,59 @@ class BasicBiGan:
         d_real = self._discriminator.predict((encodings, cell_data))
         return CellScores(np.asarray(encodings, dtype=np.float32), mse.astype(np.float32),
                           np.asarray(d_real, dtype=np.float32).reshape(-1))
+
+    def gene_statistics(self, cell_data, groups=None, n_groups=None):
+        """Per-group, per-gene statistics of cells -> GeneStatistics (statistics_from_sums):
+        groups holds one integer label in [0, K) per cell (K = n_groups or max + 1; None: one
+        group).  This is the definition, fp64 numpy over the dense cells; engine-backed
+        subclasses stream the same sums without a dense (n, genes) intermediate."""
+        x = np.asarray(cell_data, dtype=np.float64)
+        if x.ndim != 2:
+            raise ValueError(f"expected cells of shape (n, genes), got {x.shape}")
+        labels, K = group_labels(groups, n_groups, len(x))
+        s1 = np.zeros((K, x.shape[1]))
+        s2 = np.zeros((K, x.shape[1]))
+        nz = np.zeros((K, x.shape[1]), dtype=np.int64)
+        for k in range(K):
+            rows = x[labels == k]
+            s1[k] = rows.sum(0)
+            s2[k] = (rows * rows).sum(0)
+            nz[k] = np.count_nonzero(rows, axis=0)
+        return statistics_from_sums(np.bincount(labels, minlength=K), s1, s2, nz)
+
+    def generated_gene_statistics(self, encoding_in, random_in=None, groups=None,
+                                  n_groups=None):
+        """gene_statistics(generate_cells(encoding_in, random_in), groups, n_groups); the rows
+        must already be sorted by group (ValueError otherwise, before anything is drawn).
+        random_in=None draws the noise as generate_cells does.  This is the definition;
+        engine-backed subclasses stream the generator instead."""
+        labels, K = group_labels(groups, n_groups, len(encoding_in))
+        require_sorted(labels)
+        return self.gene_statistics(self.generate_cells(encoding_in, random_in), labels, K)
+
+    def compare_cells(self, cell_data):
+        """Real cells against as many generated ones, per group -> CellComparison.  The groups
+        come from _comparison_groups (one group here and in the continuous variant; the
+        classify variant groups by the encoder's class).  Group k generates as many cells as it
+        has real ones, in group order, with the encodings of _comparison_encodings drawn first
+        and then random_uniform_vector(total) for the noise, so a restored checkpoint always
+        gives the same numbers."""
+        labels, K = self._comparison_groups(cell_data)
+        real = self.gene_statistics(cell_data, labels, K)
+        encodings = self._comparison_encodings(real.cells)
+        noise = self.random_uniform_vector(len(encodings))
+        generated = self.generated_gene_statistics(
+            encodings, noise, np.repeat(np.arange(K, dtype=np.int64), real.cells), K)
+        return CellComparison(real, generated)
+
+    def _comparison_groups(self, cell_data):
+        """-> (int64 group label per cell, K) for compare_cells: every cell in one group."""
+        return np.zeros(len(cell_data), dtype=np.int64), 1
+
+    def _comparison_encodings(self, counts):
+        """Generated-cell encodings for compare_cells, counts[k] of them for group k in group
+        order: random_encoding_vector over all of them."""
+        return self.random_encoding_vector(int(np.sum(counts)))
 
     @abstractmethod
     def trainings_step(self, sampled_batch):

@@ -15,12 +15,14 @@ from typing import Callable
 import numpy as np
 
 try:
-    from .bigan_basic import BasicBiGan, CellScores
+    from .bigan_basic import (BasicBiGan, CellScores, group_labels, require_sorted,
+                              statistics_from_sums)
     from . import engine as _engine
     from .models import NetModel, RMSprop, losses, activations  # noqa: F401
     from .cell_type_training import CellBatch, CellMatrix
 except ImportError:  # imported as top-level modules (PYTHONPATH=src style)
-    from bigan_basic import BasicBiGan, CellScores
+    from bigan_basic import (BasicBiGan, CellScores, group_labels, require_sorted,
+                             statistics_from_sums)
     from cellcomm_b200 import engine as _engine
     from cellcomm_b200.models import NetModel, RMSprop, losses, activations  # noqa: F401
     from cellcomm_b200.cell_type_training import CellBatch, CellMatrix
@@ -425,6 +427,59 @@ class ClassifyCellBiGan(BasicBiGan):
         eng.score_stream(rowptr, colidx, values, 0, n, np.asarray(random_in, dtype=np.float32),
                          enc, mse, d_real, self.PREDICT_TILE)
         return CellScores(enc.cpu().numpy(), mse.cpu().numpy(), d_real.cpu().numpy())
+
+    def gene_statistics(self, cell_data, groups=None, n_groups=None):
+        """BasicBiGan.gene_statistics, streamed on the device (BiGanEngine.moments_stream): the
+        cells are taken group by group (a stable argsort of the labels) in tiles of 4096,
+        gathered to one fp32 tile and reduced by cc_col_moments, so device memory is bounded
+        by one tile and only the [K, genes] sums are copied to the host.  A CellMatrix is read
+        as it is; anything else is first wrapped with CellMatrix.from_dense.  On integer counts
+        the sums are exact, so the result equals the definition bit for bit.  Rank-local in
+        data-parallel runs (no collective)."""
+        if self._engine is None:
+            return super().gene_statistics(cell_data, groups, n_groups)
+        mat = cell_data if isinstance(cell_data, CellMatrix) else CellMatrix.from_dense(cell_data)
+        if mat.shape[1] != self.gene_size:
+            raise ValueError(f"expected cells with {self.gene_size} genes, got {mat.shape[1]}")
+        labels, K = group_labels(groups, n_groups, len(mat))
+        counts = np.bincount(labels, minlength=K)
+        bounds = np.concatenate([[0], np.cumsum(counts)])
+        order = np.argsort(labels, kind="stable").astype(np.int64)
+        sums = self._engine.moments_stream(bounds, csr=mat.device_csr(self._engine.device),
+                                           order=order, tile_rows=self.PREDICT_TILE)
+        return statistics_from_sums(counts, *(t.cpu().numpy() for t in sums))
+
+    def generated_gene_statistics(self, encoding_in, random_in=None, groups=None,
+                                  n_groups=None):
+        """BasicBiGan.generated_gene_statistics, streamed on the device: the generator runs
+        tile by tile exactly as in generate_cells (so the cells are the same bits) into one
+        fp32 tile, and cc_col_moments reduces each group's rows of it, rounded half to even
+        (BiGanEngine.moments_stream).  The rows must be sorted by group.  Only the [K, genes]
+        sums are copied to the host; rank-local in data-parallel runs."""
+        if self._engine is None:
+            return super().generated_gene_statistics(encoding_in, random_in, groups, n_groups)
+        enc = np.asarray(encoding_in, dtype=np.float32)
+        labels, K = group_labels(groups, n_groups, len(enc))
+        require_sorted(labels)
+        if random_in is None:
+            random_in = self.random_uniform_vector(len(enc))
+        counts = np.bincount(labels, minlength=K)
+        bounds = np.concatenate([[0], np.cumsum(counts)])
+        sums = self._engine.moments_stream(bounds, z32=enc,
+                                           r32=np.asarray(random_in, dtype=np.float32),
+                                           tile_rows=self.PREDICT_TILE)
+        return statistics_from_sums(counts, *(t.cpu().numpy() for t in sums))
+
+    def _comparison_groups(self, cell_data):
+        """compare_cells' grouping: K = encoding_size classes, a cell's class the argmax of its
+        encoding_prediction (NumPy's first maximum, as trainings_encoding_prediction)."""
+        prediction = np.asarray(self.encoding_prediction(cell_data))
+        return np.argmax(prediction, -1).astype(np.int64), self.encoding_size
+
+    def _comparison_encodings(self, counts):
+        """counts[k] copies of one_hot(k) for every class k, in class order (nothing drawn)."""
+        eye = np.eye(self.encoding_size, dtype=np.float32)
+        return np.repeat(eye, np.asarray(counts, dtype=np.int64), axis=0)
 
     def evaluate_discriminator_accuracy(self, sampled_batch):
         """(true-positives, true-negatives), reference src/bigan_basic.py:50-64 -- same draws in

@@ -4,10 +4,12 @@ gene_size (:7-41) and the discriminator inherited from bigan_classify."""
 import numpy as np
 
 try:
+    from .bigan_basic import BasicBiGan
     from .bigan_classify import ClassifyCellBiGan
     from . import engine as _engine
     from .models import NetModel
 except ImportError:  # imported as top-level modules (PYTHONPATH=src style)
+    from bigan_basic import BasicBiGan
     from bigan_classify import ClassifyCellBiGan
     from cellcomm_b200 import engine as _engine
     from cellcomm_b200.models import NetModel
@@ -40,3 +42,7 @@ class ContinuousCellBiGan(ClassifyCellBiGan):
 
     def trainings_encoding_prediction(self, cell_data):
         return self.encoding_prediction(cell_data)
+
+    # a continuous code has no classes: compare_cells uses one group and random encodings
+    _comparison_groups = BasicBiGan._comparison_groups
+    _comparison_encodings = BasicBiGan._comparison_encodings

@@ -2208,6 +2208,84 @@ class BiGanEngine:
                             out16=cells[:m])
             self.discriminate(z, cells[:m], d[s:s + m])
 
+    def moments_stream(self, bounds, *, csr=None, order=None, z32=None, r32=None,
+                       tile_rows=GENERATE_TILE):
+        """Per-group column moments of real or generated cells, for K groups given by `bounds`
+        (K + 1 non-decreasing host ints from 0) -> device tensors
+            sum     [K, gene_size] fp64   sum over the group's cells of v
+            sumsq   [K, gene_size] fp64   sum of v^2
+            nonzero [K, gene_size] int64  number of cells with v != 0
+        Real cells: csr = (rowptr, colidx, values) of a device CSR with gene_size columns and
+        `order` (host or device int64) its row numbers sorted by group; group k is the rows
+        order[bounds[k]:bounds[k + 1]] and v the exact fp32 count.  Per tile of at most
+        tile_rows positions of one group: cc_gather_rows(row_idx=...) into the fp32 tile, then
+        cc_col_moments into that group's accumulators.
+        Generated cells: z32 / r32 ([n, Z] fp32, host or device, n = bounds[-1]) sorted by
+        group; group k is rows [bounds[k], bounds[k + 1]) and v = rint(G.predict(z, r)).  Per
+        tile of tile_rows rows from row 0 (the tiling of G.predict, whose split-K depends on
+        the row count, so the cells are generate_cells' bit for bit): set_latents + generate()
+        into the fp32 tile, then one cc_col_moments(round_half_even=1) per group segment inside
+        the tile.
+        Device memory: the fp32 tile, the accumulators and the cc_col_moments workspace;
+        nothing of size (n, genes).  Engine state (weights, BN statistics, RNG counter,
+        loss_buf) is not touched; the generator forward orders itself after pending side-stream
+        optimiser updates, and the pass issues no collective."""
+        dev = self.device
+        if dev.type != "cuda":
+            raise RuntimeError("moments_stream needs a CUDA device (no host fallback)")
+        bounds = [int(b) for b in bounds]
+        K = len(bounds) - 1
+        if K < 1 or bounds[0] != 0 or any(b > e for b, e in zip(bounds, bounds[1:])):
+            raise ValueError("moments_stream: bounds must be K + 1 >= 2 non-decreasing "
+                             "offsets from 0")
+        if (csr is None) == (z32 is None):
+            raise ValueError("moments_stream: give either csr and order (real cells) or z32 "
+                             "and r32 (generated cells)")
+        n = bounds[-1]
+        tile_rows = int(tile_rows)
+        if tile_rows < 1:
+            raise ValueError("moments_stream: tile_rows must be >= 1")
+        Gn = self.Gn
+        sums = torch.zeros((K, Gn), dtype=torch.float64, device=dev)
+        sumsq = torch.zeros((K, Gn), dtype=torch.float64, device=dev)
+        nonzero = torch.zeros((K, Gn), dtype=torch.int64, device=dev)
+        if csr is not None:
+            rowptr, colidx, values = csr
+            order = torch.as_tensor(order, dtype=torch.int64).to(dev)
+            if order.dim() != 1 or order.numel() != n:
+                raise ValueError(f"moments_stream: order must hold bounds[-1] = {n} row numbers")
+            T = max(1, min(tile_rows, max((e - b for b, e in zip(bounds, bounds[1:])),
+                                          default=1)))
+        else:
+            z32 = torch.as_tensor(z32, dtype=torch.float32).to(dev)
+            r32 = torch.as_tensor(r32, dtype=torch.float32).to(dev)
+            if tuple(z32.shape) != (n, self.Z) or tuple(r32.shape) != (n, self.Z):
+                raise ValueError(f"moments_stream: z32 / r32 must both be [{n}, {self.Z}]")
+            T = max(1, min(tile_rows, n))
+        if n == 0:
+            return sums, sumsq, nonzero
+        tile = ops.alloc2d(T, Gn, dtype=torch.float32, device=dev, zero=False)
+        ws_bytes = ops.col_moments_ws_bytes(T, Gn)
+        ws = torch.zeros(ws_bytes, dtype=torch.uint8, device=dev) if ws_bytes else None
+        if csr is not None:
+            for k in range(K):
+                for s in range(bounds[k], bounds[k + 1], T):
+                    m = min(T, bounds[k + 1] - s)
+                    ops.gather_rows(rowptr, colidx, values, Gn, row_idx=order[s:s + m],
+                                    out32=tile[:m])
+                    ops.col_moments(tile[:m], sums[k], sumsq[k], nonzero[k], ws=ws)
+            return sums, sumsq, nonzero
+        for s in range(0, n, T):
+            m = min(T, n - s)
+            self.set_latents(z32[s:s + m], r32[s:s + m], m)
+            self.generate(m, out32=tile[:m])
+            for k in range(K):
+                lo, hi = max(bounds[k], s), min(bounds[k + 1], s + m)
+                if lo < hi:
+                    ops.col_moments(tile[lo - s:hi - s], sums[k], sumsq[k], nonzero[k],
+                                    round=True, ws=ws)
+        return sums, sumsq, nonzero
+
     def discriminate(self, z16, x16, out32):
         """D.predict -> probabilities (fp32 [rows,1])."""
         return self.D.forward({"z": z16, "cell": x16}, x16.shape[0], bn_train=False, dropout="off",

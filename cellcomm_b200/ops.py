@@ -497,6 +497,35 @@ def recon_sqerr(pred32, rowptr, colidx, values, row0, out, scale=1.0):
                                      int(row0), float(scale), out.data_ptr(), _stream()))
 
 
+def col_moments_ws_bytes(rows, cols):
+    """Bytes of a col_moments workspace that serves every call on at most rows x cols (zero it
+    once before the first use; one workspace per stream)."""
+    return int(_lib.load().cc_col_moments_ws_bytes(int(rows), int(cols)))
+
+
+def col_moments(x32, sum64, sumsq64, nonzero64, *, round=False, ws):
+    """sum64[c] += sum_r v, sumsq64[c] += sum_r v^2, nonzero64[c] += #{r : v != 0} over the
+    rows of a dense fp32 tile, v = x32[r, c] or rint(x32[r, c]) with round=True
+    (cc_col_moments: fp64, fixed order).  ws: a zeroed uint8 buffer of col_moments_ws_bytes
+    bytes, or None for calls that need none (at most 256 rows)."""
+    _req(x32, torch.float32, "x32")
+    _req(sum64, torch.float64, "sum64")
+    _req(sumsq64, torch.float64, "sumsq64")
+    _req(nonzero64, torch.int64, "nonzero64")
+    _req(ws, torch.uint8, "ws")
+    if x32.dim() != 2:
+        raise ValueError("col_moments: x32 must be [rows, cols]")
+    cols = x32.shape[1]
+    for t in (sum64, sumsq64, nonzero64):
+        if t.numel() != cols or not t.is_contiguous():
+            raise ValueError(f"col_moments: the accumulators must hold {cols} contiguous values")
+    if ws is not None and not ws.is_contiguous():
+        raise ValueError("col_moments: ws must be contiguous")
+    check(_lib.load().cc_col_moments(_p(x32), _ld(x32), x32.shape[0], cols, int(bool(round)),
+                                     sum64.data_ptr(), sumsq64.data_ptr(), nonzero64.data_ptr(),
+                                     _p(ws), 0 if ws is None else ws.numel(), _stream()))
+
+
 def argmax_onehot(p32, out16=None, out32=None):
     _req(p32, torch.float32, "p32")
     check(_lib.load().cc_argmax_onehot(_p(p32), _ld(p32), _p(out16), _ld(out16), _p(out32),

@@ -418,6 +418,23 @@ int cc_round_csr_fill(const float* x, int64_t ldx, int64_t rows, int64_t cols,
 int cc_recon_sqerr(const float* pred, int64_t ld, int64_t rows, int64_t cols,
                    const int64_t* rowptr, const int32_t* colidx, const float* values, int64_t row0,
                    float scale, float* out, cc_stream_t stream);
+/* Per-gene moments for the compare pass (csrc/moments.cu).  Adds, for every column c < cols of
+ * the fp32 tile x ([rows, ld]):
+ *   sum[c] += sum_r v,  sumsq[c] += sum_r v^2,  nonzero[c] += #{r : v != 0}
+ * with v = x[r, c], or rint(x[r, c]) (round half to even) when round_half_even != 0.  -0.0
+ * counts as zero; columns [cols, ld) are never read into a result; rows == 0 is a no-op.
+ * Accumulation is fp64 and the partials of the row slabs combine in a fixed order without
+ * float atomics (the last CTA of a column block adds them once), so identical inputs give
+ * identical bits, and integer data gives exact totals whatever the order.  cols <= 262,144.
+ * Workspace contract: ws holds ws_bytes bytes, 16-byte aligned, at least
+ * cc_col_moments_ws_bytes(rows, cols) for any call of at most rows x cols (0 for calls of at
+ * most 256 rows); a smaller one fails (cc_last_error), never falls back to atomics.  Zero it
+ * once before the first use: every call leaves its counters zero again.  One workspace per
+ * stream. */
+int cc_col_moments(const float* x, int64_t ld, int64_t rows, int64_t cols,
+                   int32_t round_half_even, double* sum, double* sumsq, int64_t* nonzero,
+                   void* ws, int64_t ws_bytes, cc_stream_t stream);
+int64_t cc_col_moments_ws_bytes(int64_t rows, int64_t cols);
 /* to_categorical(argmax(p,-1)): src/bigan_classify.py:121-124 */
 int cc_argmax_onehot(const float* p32, int64_t ldp, void* out16, int64_t ldo, float* out32,
                      int64_t ldo32, int64_t rows, int64_t cols, cc_stream_t stream);
