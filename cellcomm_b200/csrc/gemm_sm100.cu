@@ -53,13 +53,11 @@ struct EpiParams {
   bf16* rms_p16;
   long long rms_ld;
   float rms_lr, rms_rho, rms_momentum, rms_eps;
-  int rms_cs;  // evict-first (ld/st.global.cs) hints on the optimiser state stream
   // blocked optimiser-state layout (cc_gemm_desc.rms_blocked): rms_p32 / rms_ms / rms_mom are
   // the LAYER's blocked arrays, this GEMM's rows start at layer row rms_row0
   int rms_blocked;
   int rms_row0;
   bf16* rms_p16lo;  // blocked path: low-order bf16 term of the updated weight (hi + lo kernels)
-  int rms_keep_operands;  // blocked path: operand TMA loads carry an L2 evict_last policy
   // routed fp32 output (data-parallel wgrad): element `rel` of the bucket goes to the rank that
   // owns it, route_base[owner] + rel (peer-mapped staging slot; own share: local memory)
   int route_world;
@@ -89,7 +87,6 @@ struct GemmParams {
   int b_boxes;            // MN-major B: 64-column TMA boxes per stage
   int b_half_rows;        // K-major B in a 2-CTA cluster: rows of the tile each CTA loads
   int cluster;            // 1 or 2 CTAs per cluster (persistent kernel)
-  int pair;               // cluster of 2 running one cta_group::2 MMA per k-step (256-row tiles)
   unsigned int stage_tx;  // bytes TMA delivers per stage
 };
 
@@ -296,16 +293,6 @@ __device__ __forceinline__ void for_each_valid(float4 (&g)[8], int nrow, int nco
   }
 }
 
-// evict-first 16-byte load that asks L2 to fetch the whole 256-byte neighbourhood from DRAM:
-// the lane's next 32-column block of the same rows lies in it
-__device__ __forceinline__ float4 ldcs_256(const float* p) {
-  float4 v;
-  asm volatile("ld.global.cs.L2::256B.v4.f32 {%0, %1, %2, %3}, [%4];"
-               : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w)
-               : "l"(p));
-  return v;
-}
-
 template <bool MATH>
 __device__ __forceinline__ void epilogue_chunk(const EpiParams& e, float* stage /*32x36*/, int lane,
                                                int r0, int c0, const uint32_t (&raw)[32],
@@ -361,7 +348,8 @@ __device__ __forceinline__ void epilogue_chunk(const EpiParams& e, float* stage 
 
   if (e.rms_p32 != nullptr) {
     // fused Keras RMSprop(momentum): ms = rho*ms + (1-rho) g^2 ; mom = momentum*mom +
-    // lr*g/sqrt(ms+eps) ; w -= mom ; bf16 copy.  All loads are issued before the first use.
+    // lr*g/sqrt(ms+eps) ; w -= mom ; bf16 copy.  All loads are issued before the first use;
+    // the state is streamed with evict-first (.cs) hints.
     const bool vec = ncol == 4 && (e.rms_ld & 3) == 0 && ((c & 3) == 0) &&
                      ((((uintptr_t)e.rms_p32) & 15) == 0) && ((((uintptr_t)e.rms_ms) & 15) == 0) &&
                      ((((uintptr_t)e.rms_mom) & 15) == 0) &&
@@ -374,19 +362,9 @@ __device__ __forceinline__ void epilogue_chunk(const EpiParams& e, float* stage 
       for (int t = 0; t < 8; ++t) {
         if (t < nrow) {
           const long long off = off0 + t * step;
-          if (e.rms_cs & 8) {
-            w[t] = ldcs_256(e.rms_p32 + off);
-            s[t] = ldcs_256(e.rms_ms + off);
-            m[t] = ldcs_256(e.rms_mom + off);
-          } else if (e.rms_cs & 1) {
-            w[t] = __ldcs(reinterpret_cast<const float4*>(e.rms_p32 + off));
-            s[t] = __ldcs(reinterpret_cast<const float4*>(e.rms_ms + off));
-            m[t] = __ldcs(reinterpret_cast<const float4*>(e.rms_mom + off));
-          } else {
-            w[t] = *reinterpret_cast<const float4*>(e.rms_p32 + off);
-            s[t] = *reinterpret_cast<const float4*>(e.rms_ms + off);
-            m[t] = *reinterpret_cast<const float4*>(e.rms_mom + off);
-          }
+          w[t] = __ldcs(reinterpret_cast<const float4*>(e.rms_p32 + off));
+          s[t] = __ldcs(reinterpret_cast<const float4*>(e.rms_ms + off));
+          m[t] = __ldcs(reinterpret_cast<const float4*>(e.rms_mom + off));
         }
       }
       const float rho = e.rms_rho, omr = 1.f - e.rms_rho, mu = e.rms_momentum, lr = e.rms_lr,
@@ -408,15 +386,9 @@ __device__ __forceinline__ void epilogue_chunk(const EpiParams& e, float* stage 
           ww.y = w[t].y - mm.y;
           ww.z = w[t].z - mm.z;
           ww.w = w[t].w - mm.w;
-          if (e.rms_cs & 1) {
-            __stcs(reinterpret_cast<float4*>(e.rms_ms + off), ss);
-            __stcs(reinterpret_cast<float4*>(e.rms_mom + off), mm);
-            __stcs(reinterpret_cast<float4*>(e.rms_p32 + off), ww);
-          } else {
-            *reinterpret_cast<float4*>(e.rms_ms + off) = ss;
-            *reinterpret_cast<float4*>(e.rms_mom + off) = mm;
-            *reinterpret_cast<float4*>(e.rms_p32 + off) = ww;
-          }
+          __stcs(reinterpret_cast<float4*>(e.rms_ms + off), ss);
+          __stcs(reinterpret_cast<float4*>(e.rms_mom + off), mm);
+          __stcs(reinterpret_cast<float4*>(e.rms_p32 + off), ww);
           if (e.rms_p16 != nullptr) {
             __nv_bfloat162 lo = __floats2bfloat162_rn(ww.x, ww.y);
             __nv_bfloat162 hi = __floats2bfloat162_rn(ww.z, ww.w);
@@ -711,73 +683,9 @@ __device__ __forceinline__ void tma_load_2d_mc(uint32_t dst, const CUtensorMap* 
       "l"(map), "r"(bar), "r"(c0), "r"(c1), "h"(mask)
       : "memory");
 }
-// the same loads with an L2 cache policy (operands of the fused-optimiser wgrad: evict_last, so
-// that the 26 B/parameter optimiser stream -- evict_first on its side -- does not push X / dZ
-// out of L2 between the row blocks that re-read them).  CC_GEMM_RMS_KEEP_OPERANDS=1; measured
-// neutral to slightly negative at batch 512 ... 4096 (profiles/r02_fused_rmsprop_blocked_state
-// .jsonl), so off by default.
-__device__ __forceinline__ uint64_t l2_policy_evict_last() {
-  uint64_t pol;
-  asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol));
-  return pol;
-}
-__device__ __forceinline__ void tma_load_2d_pol(uint32_t dst, const CUtensorMap* map, uint32_t bar,
-                                                int c0, int c1, uint64_t pol) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint "
-      "[%0], [%1, {%3, %4}], [%2], %5;" ::"r"(dst),
-      "l"(map), "r"(bar), "r"(c0), "r"(c1), "l"(pol)
-      : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_mc_pol(uint32_t dst, const CUtensorMap* map,
-                                                   uint32_t bar, int c0, int c1, uint16_t mask,
-                                                   uint64_t pol) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes"
-      ".multicast::cluster.L2::cache_hint [%0], [%1, {%3, %4}], [%2], %5, %6;" ::"r"(dst),
-      "l"(map), "r"(bar), "r"(c0), "r"(c1), "h"(mask), "l"(pol)
-      : "memory");
-}
 __device__ __forceinline__ void umma_commit_mc(uint32_t bar, uint16_t mask) {
   asm volatile(
       "tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 "
-      "[%0], %1;" ::"r"(bar),
-      "h"(mask)
-      : "memory");
-}
-
-// ---- CTA pair (tcgen05 cta_group::2): one 256-row tile per SM pair ---------------------------
-// the cluster-space address of `local` (a shared::cta address) in CTA `cta` of the cluster
-__device__ __forceinline__ uint32_t mapa_cluster(uint32_t local, uint32_t cta) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(local), "r"(cta));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr)
-               : "memory");
-}
-// TMA load whose completion bytes are counted on a barrier of the pair's LEADER CTA
-__device__ __forceinline__ void tma_load_2d_pair(uint32_t dst, const CUtensorMap* map,
-                                                 uint32_t leader_bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes "
-      "[%0], [%1, {%3, %4}], [%2];" ::"r"(dst),
-      "l"(map), "r"(leader_bar), "r"(c0), "r"(c1)
-      : "memory");
-}
-__device__ __forceinline__ void umma_bf16_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc,
-                                               uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d),
-      "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void umma_commit_pair(uint32_t bar, uint16_t mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 "
       "[%0], %1;" ::"r"(bar),
       "h"(mask)
       : "memory");
@@ -869,24 +777,14 @@ __device__ __forceinline__ void rms_blocked_chunk(const EpiParams& e, int lane, 
 // N_FAST: consecutive tiles walk along N (the contiguous direction of the output / parameter
 // matrix), so the CTAs of one wave cover whole output rows: used by the fused-optimiser wgrad,
 // whose epilogue streams 26 B per element and wants DRAM-page-local bursts.
-//
-// PAIR (CLUSTER = 2 only): the SM pair runs ONE tcgen05 cta_group::2 MMA on a 256-row tile.  Each
-// CTA stages its own 128 rows of A and only its HALF of the B tile (the tensor cores fetch the
-// other half from the peer's shared memory), so a k-block costs 16 + 16 KB of shared memory per
-// CTA instead of 16 + 32 KB: the operand ring is 6 stages deep instead of 4 at the same L2 -> SM
-// traffic as the multicast scheme.  The leader CTA (cluster rank 0) issues every MMA; both
-// CTAs' TMA loads count on the leader's "full" barrier; tcgen05.commit is multicast to both
-// CTAs' "empty" / "accumulator full" barriers; each CTA drains its own 128 accumulator rows
-// from its own TMEM and reports "accumulator free" to the leader.
 template <int BN, int STAGES, bool A_MN, bool B_MN, bool MATH, int EPI_WARPS, bool N_FAST = false,
-          int CLUSTER = 1, bool PAIR = false, bool RMS_DIRECT = false>
+          int CLUSTER = 1, bool RMS_DIRECT = false>
 __global__ void __launch_bounds__(64 + 32 * EPI_WARPS, 1)
 gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
                                const __grid_constant__ GemmParams p,
                                const int tiles_m, const int tiles_n) {
-  static_assert(!PAIR || CLUSTER == 2, "a CTA pair is a cluster of two");
   constexpr uint32_t A_BYTES = BM * BK * 2;
-  constexpr uint32_t B_BYTES = (PAIR ? BN / 2 : BN) * BK * 2;
+  constexpr uint32_t B_BYTES = BN * BK * 2;
   constexpr uint32_t STAGE_BYTES = A_BYTES + B_BYTES;
   constexpr uint32_t TMEM_COLS = 2 * BN;  // two accumulator stages
   static_assert(TMEM_COLS <= 512, "TMEM has 512 columns");
@@ -908,7 +806,6 @@ gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
 
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
-  const int nkb = p.total_kblocks;
   // work units: one tile (CLUSTER 1) or a vertical pair of tiles (CLUSTER 2)
   const int rank = (CLUSTER == 2) ? (int)cluster_ctarank() : 0;
   const int tiles_mu = (tiles_m + CLUSTER - 1) / CLUSTER;
@@ -938,32 +835,22 @@ gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
   if (threadIdx.x == 0) {
 #pragma unroll
     for (int s = 0; s < STAGES; ++s) {
-      // pair: one arrival per CTA on the leader's barrier (plus the bytes of both)
-      mbar_init(full_bar(s), PAIR ? 2 : 1);
-      // one commit from every CTA of the cluster; pair: the leader's commit, multicast
-      mbar_init(empty_bar(s), PAIR ? 1 : CLUSTER);
+      mbar_init(full_bar(s), 1);
+      mbar_init(empty_bar(s), CLUSTER);  // one commit from every CTA of the cluster
     }
 #pragma unroll
     for (int a = 0; a < 2; ++a) {
       mbar_init(tfull_bar(a), 1);
-      // one arrival per epilogue warp (pair: of both CTAs, on the leader's barrier)
-      mbar_init(tempty_bar(a), PAIR ? 2 * EPI_WARPS : EPI_WARPS);
+      mbar_init(tempty_bar(a), EPI_WARPS);  // one arrival per epilogue warp
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
   }
   if (warp == 1) {
-    if (PAIR) {  // one warp of EACH CTA: the pair gets the same columns in both TMEMs
-      asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot),
-                   "r"(TMEM_COLS)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-    } else {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot),
-                   "r"(TMEM_COLS)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot),
+                 "r"(TMEM_COLS)
+                 : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
   }
   tcgen05_fence_before();
   __syncthreads();
@@ -971,51 +858,9 @@ gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
   tcgen05_fence_after();
   const uint32_t tmem_acc = *tmem_slot_ptr;
 
-  if (warp == 0 && PAIR) {
-    // ===================== TMA producer, CTA pair: own A rows + own half of B ================
-    uint32_t it = 0;
-    const int half = p.bn_eff / 2;
-    for (int u = unit0; u < num_units; u += unit_step) {
-      const int m0 = unit_m0(u), n0 = unit_n0(u) + rank * half;
-      int seg = 0, kb_in_seg = 0;
-      for (int i = 0; i < nkb; ++i, ++it) {
-        const int s = it % STAGES;
-        const uint32_t ph = (it / STAGES) & 1u;
-        mbar_wait(empty_bar(s), ph ^ 1u, 11);
-        if (elect_one()) {
-          const uint32_t a_dst = smem_base + s * STAGE_BYTES;
-          const uint32_t b_dst = a_dst + A_BYTES;
-          const uint32_t lbar = mapa_cluster(full_bar(s), 0);  // the leader's barrier
-          const int k0 = kb_in_seg * BK;
-          if (rank == 0) mbar_expect_tx(full_bar(s), 2 * p.stage_tx);
-          else mbar_arrive_cluster(lbar);
-          if (A_MN) {
-#pragma unroll
-            for (int j = 0; j < BM / 64; ++j)
-              tma_load_2d_pair(a_dst + j * (64 * BK * 2), &maps.a[seg], lbar, m0 + 64 * j, k0);
-          } else {
-            tma_load_2d_pair(a_dst, &maps.a[seg], lbar, k0, m0);
-          }
-          if (B_MN) {
-#pragma unroll
-            for (int j = 0; j < BN / 128; ++j)
-              if (j < p.b_boxes)
-                tma_load_2d_pair(b_dst + j * (64 * BK * 2), &maps.b[seg], lbar, n0 + 64 * j, k0);
-          } else {
-            tma_load_2d_pair(b_dst, &maps.b[seg], lbar, k0, n0);
-          }
-        }
-        __syncwarp();
-        if (++kb_in_seg >= p.kblocks[seg] && seg < p.nseg - 1) {
-          kb_in_seg = 0;
-          ++seg;
-        }
-      }
-    }
-  } else if (warp == 0) {
+  if (warp == 0) {
     // ===================== TMA producer =====================
     uint32_t it = 0;
-    const uint64_t keep = (RMS_DIRECT && p.epi.rms_keep_operands) ? l2_policy_evict_last() : 0;
     for (int u = unit0; u < num_units; u += unit_step) {
       const int m0 = unit_m0(u), n0 = unit_n0(u);
       const int nkb_u = unit_nkb(u);
@@ -1033,34 +878,14 @@ gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
           const uint32_t b_dst = a_dst + A_BYTES;
           const int k0 = kb_in_seg * BK;
           mbar_expect_tx(full_bar(s), p.stage_tx);
-          if (RMS_DIRECT && A_MN && B_MN && keep != 0) {
-            // (the fused-optimiser wgrad: both operands MN-major)
-#pragma unroll
-            for (int j = 0; j < BM / 64; ++j)
-              tma_load_2d_pol(a_dst + j * (64 * BK * 2), &maps.a[seg], full_bar(s), m0 + 64 * j, k0,
-                              keep);
-#pragma unroll
-            for (int j = 0; j < BN / 64; ++j) {
-              if (j >= p.b_boxes) continue;
-              if (CLUSTER == 2) {
-                if ((j & 1) == rank)
-                  tma_load_2d_mc_pol(b_dst + j * (64 * BK * 2), &maps.b[seg], full_bar(s),
-                                     n0 + 64 * j, k0, (uint16_t)3, keep);
-              } else {
-                tma_load_2d_pol(b_dst + j * (64 * BK * 2), &maps.b[seg], full_bar(s), n0 + 64 * j,
-                                k0, keep);
-              }
-            }
-          } else if (A_MN) {
+          if (A_MN) {
 #pragma unroll
             for (int j = 0; j < BM / 64; ++j)
               tma_load_2d(a_dst + j * (64 * BK * 2), &maps.a[seg], full_bar(s), m0 + 64 * j, k0);
           } else {
             tma_load_2d(a_dst, &maps.a[seg], full_bar(s), k0, m0);
           }
-          if (RMS_DIRECT && A_MN && B_MN && keep != 0) {
-            // (B loaded above)
-          } else if (CLUSTER == 2) {
+          if (CLUSTER == 2) {
             // this CTA's half of the B tile, delivered to both CTAs
             if (B_MN) {
 #pragma unroll
@@ -1089,9 +914,9 @@ gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
       }
     }
   } else if (warp == 1) {
-    // ===================== MMA issuer (pair: the leader CTA only) =====================
+    // ===================== MMA issuer =====================
     uint32_t it = 0, tl = 0;
-    for (int u = unit0; (!PAIR || rank == 0) && u < num_units; u += unit_step, ++tl) {
+    for (int u = unit0; u < num_units; u += unit_step, ++tl) {
       const uint32_t acc = tl & 1u, aph = (tl >> 1) & 1u;
       mbar_wait(tempty_bar(acc), aph ^ 1u, 12);  // epilogue has drained this accumulator
       tcgen05_fence_after();
@@ -1109,17 +934,11 @@ gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
           for (int k = 0; k < BK / UMMA_K; ++k) {
             const uint64_t adesc = p.adesc_hi | (uint64_t)(((a_src + k * p.a_kstep) & 0x3FFFFu) >> 4);
             const uint64_t bdesc = p.bdesc_hi | (uint64_t)(((b_src + k * p.b_kstep) & 0x3FFFFu) >> 4);
-            if (PAIR) umma_bf16_pair(d_tmem, adesc, bdesc, p.idesc, (i > 0 || k > 0) ? 1u : 0u);
-            else umma_bf16(d_tmem, adesc, bdesc, p.idesc, (i > 0 || k > 0) ? 1u : 0u);
+            umma_bf16(d_tmem, adesc, bdesc, p.idesc, (i > 0 || k > 0) ? 1u : 0u);
           }
-          if (PAIR) {
-            umma_commit_pair(empty_bar(s), (uint16_t)3);  // both CTAs may refill the stage
-            if (i == nkb - 1) umma_commit_pair(tfull_bar(acc), (uint16_t)3);
-          } else {
-            if (CLUSTER == 2) umma_commit_mc(empty_bar(s), (uint16_t)3);
-            else umma_commit(empty_bar(s));
-            if (i == nkb - 1) umma_commit(tfull_bar(acc));
-          }
+          if (CLUSTER == 2) umma_commit_mc(empty_bar(s), (uint16_t)3);
+          else umma_commit(empty_bar(s));
+          if (i == nkb - 1) umma_commit(tfull_bar(acc));
         }
         __syncwarp();
       }
@@ -1153,10 +972,7 @@ gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
       }
       tcgen05_fence_before();
       __syncwarp();
-      if (lane == 0) {
-        if (PAIR) mbar_arrive_cluster(mapa_cluster(tempty_bar(acc), 0));
-        else mbar_arrive(tempty_bar(acc));
-      }
+      if (lane == 0) mbar_arrive(tempty_bar(acc));
     }
   }
   tcgen05_fence_before();
@@ -1164,20 +980,11 @@ gemm_tcgen05_persistent_kernel(const __grid_constant__ TmaMaps maps,
   // no CTA may leave while its peer can still multicast into its smem / arrive on its barriers
   if (CLUSTER == 2) cluster_sync_all();
   if (warp == 1) {
-    if (PAIR)
-      asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc),
-                   "r"(TMEM_COLS)
-                   : "memory");
-    else
-      asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc),
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_acc),
                    "r"(TMEM_COLS)
                    : "memory");
   }
 }
-
-}  // namespace cc
-#include "wgrad_rmsprop_kernel.cuh"
-namespace cc {
 
 // Sum split-K partials and apply the epilogue.  One thread per (row, 32-col chunk).
 // One thread per (row, 4 columns): consecutive lanes read consecutive float4 of a partial row
@@ -1288,10 +1095,9 @@ struct MapKey {
   const void* ptr;
   uint64_t inner, outer, ld;
   uint32_t box_inner, box_outer;
-  uint32_t kind;  // element type / swizzle / L2 promotion
   bool operator==(const MapKey& o) const {
     return ptr == o.ptr && inner == o.inner && outer == o.outer && ld == o.ld &&
-           box_inner == o.box_inner && box_outer == o.box_outer && kind == o.kind;
+           box_inner == o.box_inner && box_outer == o.box_outer;
   }
 };
 struct MapKeyHash {
@@ -1301,24 +1107,17 @@ struct MapKeyHash {
     h ^= k.outer + 0x9E3779B97F4A7C15ull + (h << 6) + (h >> 2);
     h ^= k.ld + 0x9E3779B97F4A7C15ull + (h << 6) + (h >> 2);
     h ^= ((uint64_t)k.box_inner << 32 | k.box_outer) + 0x9E3779B97F4A7C15ull + (h << 6) + (h >> 2);
-    h ^= k.kind + 0x9E3779B97F4A7C15ull + (h << 6) + (h >> 2);
     return (size_t)h;
   }
 };
 
-enum MapKind : uint32_t {
-  MAP_BF16_SW128 = 0,   // GEMM operands
-  MAP_F32_SW128 = 1,    // optimiser state blocks (32 fp32 = one 128-byte swizzle row)
-  MAP_BF16_SW64 = 2,    // bf16 weight copy blocks (32 bf16 = one 64-byte swizzle row)
-  MAP_F32_SW128_L2_256 = 3   // state blocks fetched from DRAM in 256-byte pieces
-};
-
-// Row-major [outer, inner] tensor with leading dimension ld (elements).
-static int make_map_kind(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t outer,
-                         uint64_t ld, uint32_t box_inner, uint32_t box_outer, MapKind kind) {
+// bf16 GEMM operand: row-major [outer, inner] tensor with leading dimension ld (elements),
+// 128-byte swizzle
+static int make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t outer, uint64_t ld,
+                    uint32_t box_inner, uint32_t box_outer) {
   static std::mutex mu;
   static std::unordered_map<MapKey, CUtensorMap, MapKeyHash> cache;
-  MapKey key{ptr, inner, outer, ld, box_inner, box_outer, (uint32_t)kind};
+  MapKey key{ptr, inner, outer, ld, box_inner, box_outer};
   {
     std::lock_guard<std::mutex> g(mu);
     auto it = cache.find(key);
@@ -1327,27 +1126,19 @@ static int make_map_kind(CUtensorMap* out, const void* ptr, uint64_t inner, uint
       return 0;
     }
   }
-  const bool f32 = kind == MAP_F32_SW128 || kind == MAP_F32_SW128_L2_256;
-  const uint64_t esize = f32 ? 4 : 2;
   PFN_encodeTiled enc = get_encode_fn();
   CC_REQUIRE(enc != nullptr, "cuTensorMapEncodeTiled is unavailable (no CUDA driver?)");
   CC_REQUIRE(((uintptr_t)ptr & 15) == 0, "cc_gemm: operand base %p is not 16-byte aligned", ptr);
-  CC_REQUIRE((ld * esize) % 16 == 0, "cc_gemm: operand ld=%llu is not a multiple of 16 bytes",
+  CC_REQUIRE((ld * 2) % 16 == 0, "cc_gemm: operand ld=%llu is not a multiple of 16 bytes",
              (unsigned long long)ld);
   CC_REQUIRE(inner > 0 && outer > 0, "cc_gemm: empty operand");
   cuuint64_t dims[2] = {inner, outer};
-  cuuint64_t strides[1] = {ld * esize};
+  cuuint64_t strides[1] = {ld * 2};
   cuuint32_t box[2] = {box_inner, box_outer};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = enc(out,
-                   f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16,
-                   2, const_cast<void*>(ptr), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE,
-                   kind == MAP_BF16_SW64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
-                   (kind == MAP_BF16_SW128 || kind == MAP_F32_SW128_L2_256)
-                       ? CU_TENSOR_MAP_L2_PROMOTION_L2_256B
-                       : CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  CUresult r = enc(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(ptr), dims, strides,
+                   box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+                   CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   CC_REQUIRE(r == CUDA_SUCCESS,
              "cuTensorMapEncodeTiled failed (%d) ptr=%p inner=%llu outer=%llu ld=%llu box=%ux%u",
              (int)r, ptr, (unsigned long long)inner, (unsigned long long)outer,
@@ -1358,12 +1149,6 @@ static int make_map_kind(CUtensorMap* out, const void* ptr, uint64_t inner, uint
     cache.emplace(key, *out);
   }
   return 0;
-}
-
-// bf16 GEMM operand
-static int make_map(CUtensorMap* out, const void* ptr, uint64_t inner, uint64_t outer, uint64_t ld,
-                    uint32_t box_inner, uint32_t box_outer) {
-  return make_map_kind(out, ptr, inner, outer, ld, box_inner, box_outer, MAP_BF16_SW128);
 }
 
 // smem matrix descriptor without the start address (cute::UMMA::SmemDescriptor):
@@ -1383,32 +1168,14 @@ static int env_int(const char* name, int dflt) {
   return v ? atoi(v) : dflt;
 }
 
-// Tuning / debug knobs, read from the environment ONCE (a GEMM launch used to cost a dozen
-// getenv calls); cc_reload_env() re-reads them (tests and sweep tools change them at run time).
+// Test knobs, read from the environment ONCE (a GEMM launch should not cost getenv calls);
+// cc_reload_env() re-reads them (tests change them at run time).  The first two force a choice
+// the dispatcher otherwise makes from the shape, so that small shapes cover every choice; the
+// third selects the reference that persistent split-K is compared with.
 struct GemmEnv {
-  int sms;
-  int bn;
-  int splits;
-  int persistent;
-  int cluster;
-  int rms_cluster;
-  int bn_eff;
-  int mn_lbo;
-  int mn_sbo;
-  int mn_kstep;
-  int k_lbo;
-  int k_sbo;
-  int rms_cs;
-  int rms_warps;
-  int rms_nfast;
-  int rms_tma;
-  int rms_p16_tma;
-  int rms_interleave;
-  int rms_pair;
-  int pair;
-  int rms_l2_256;
-  int rms_keep;
-  int persistent_splitk;
+  int bn_eff;             // CC_GEMM_BN_EFF: effective tile width of the persistent kernel
+  int rms_nfast;          // CC_GEMM_RMS_NFAST: raster of the fused-optimiser wgrad
+  int persistent_splitk;  // CC_GEMM_PERSISTENT_SPLITK=0: split-K in the one-tile-per-CTA kernel
 };
 static GemmEnv g_env;
 static std::atomic<int> g_env_state{0};   // 0: not loaded
@@ -1419,28 +1186,8 @@ static const GemmEnv& gemm_env() {
   if (g_env_state.load(std::memory_order_acquire) == 0) {
     std::lock_guard<std::mutex> lock(g_env_mu);
     GemmEnv e;
-    e.sms = env_int("CC_GEMM_SMS", 0);
-    e.bn = env_int("CC_GEMM_BN", 0);
-    e.splits = env_int("CC_GEMM_SPLITS", 0);
-    e.persistent = env_int("CC_GEMM_PERSISTENT", 1);
-    e.cluster = env_int("CC_GEMM_CLUSTER", 2);
-    e.rms_cluster = env_int("CC_GEMM_RMS_CLUSTER", -1);
     e.bn_eff = env_int("CC_GEMM_BN_EFF", 0);
-    e.mn_lbo = env_int("CC_GEMM_MN_LBO", 64 * BK * 2);
-    e.mn_sbo = env_int("CC_GEMM_MN_SBO", 1024);
-    e.mn_kstep = env_int("CC_GEMM_MN_KSTEP", UMMA_K * 128);
-    e.k_lbo = env_int("CC_GEMM_K_LBO", 16);
-    e.k_sbo = env_int("CC_GEMM_K_SBO", 1024);
-    e.rms_cs = env_int("CC_GEMM_RMS_CS", 1);
-    e.rms_warps = env_int("CC_GEMM_RMS_WARPS", 8);
     e.rms_nfast = env_int("CC_GEMM_RMS_NFAST", -1);
-    e.rms_tma = env_int("CC_GEMM_RMS_TMA", -1);
-    e.rms_p16_tma = env_int("CC_GEMM_RMS_P16_TMA", 0);
-    e.rms_interleave = env_int("CC_GEMM_RMS_INTERLEAVE", 1);
-    e.rms_pair = env_int("CC_GEMM_RMS_PAIR", 0);
-    e.pair = env_int("CC_GEMM_PAIR", 0);
-    e.rms_l2_256 = env_int("CC_GEMM_RMS_L2_256", 0);
-    e.rms_keep = env_int("CC_GEMM_RMS_KEEP_OPERANDS", 0);
     e.persistent_splitk = env_int("CC_GEMM_PERSISTENT_SPLITK", 1);
     g_env = e;
     g_env_state.store(1, std::memory_order_release);
@@ -1476,21 +1223,21 @@ static int launch_major(const TmaMaps& maps, const GemmParams& p, dim3 grid, boo
   return launch_cfg<BN, STAGES, true, false>(maps, p, grid, st);
 }
 
-template <int BN, int STAGES, int EPI_WARPS, bool PAIR = false, bool RMS_DIRECT = false>
+template <int BN, int STAGES, int EPI_WARPS, bool RMS_DIRECT = false>
 static constexpr size_t smem_bytes_persistent() {
-  return (size_t)STAGES * (BM * BK * 2 + (PAIR ? BN / 2 : BN) * BK * 2) + 8 * (2 * STAGES + 6) + 16 +
+  return (size_t)STAGES * (BM * BK * 2 + BN * BK * 2) + 8 * (2 * STAGES + 6) + 16 +
          (RMS_DIRECT ? 0 : EPI_WARPS * 32 * EPI_LD * 4) + 1024;   // no transpose tiles
 }
 
 template <int BN, int STAGES, bool A_MN, bool B_MN, bool MATH, int EPI_WARPS, bool N_FAST, int CLUSTER,
-          bool PAIR = false, bool RMS_DIRECT = false>
+          bool RMS_DIRECT = false>
 static int launch_persistent_one(const TmaMaps& maps, const GemmParams& p, int mt, int nt,
                                  int num_sms, cudaStream_t st) {
   auto kern = gemm_tcgen05_persistent_kernel<BN, STAGES, A_MN, B_MN, MATH, EPI_WARPS, N_FAST, CLUSTER,
-                                             PAIR, RMS_DIRECT>;
+                                             RMS_DIRECT>;
   static bool attr_set = false;
   static int max_ctas = 0;
-  constexpr size_t smem = smem_bytes_persistent<BN, STAGES, EPI_WARPS, PAIR, RMS_DIRECT>();
+  constexpr size_t smem = smem_bytes_persistent<BN, STAGES, EPI_WARPS, RMS_DIRECT>();
   static_assert(smem <= 232448, "shared memory per CTA");
   constexpr int threads = 64 + 32 * EPI_WARPS;
   if (!attr_set) {
@@ -1535,18 +1282,9 @@ static int launch_persistent_one(const TmaMaps& maps, const GemmParams& p, int m
   return 0;
 }
 
-// stages of the CTA-pair operand ring: the smem the half-width B tile frees buys depth
-template <int BN, int STAGES, int EPI_WARPS>
-static constexpr int pair_stages() {
-  return BN == 256 ? (EPI_WARPS == 8 ? 5 : 6) : STAGES;
-}
-
 template <int BN, int STAGES, bool A_MN, bool B_MN, bool MATH, int EPI_WARPS = 4, bool N_FAST = false>
 static int launch_persistent_cfg(const TmaMaps& maps, const GemmParams& p, int mt, int nt,
                                  int num_sms, cudaStream_t st) {
-  if (BN == 256 && p.cluster == 2 && p.pair)
-    return launch_persistent_one<BN, pair_stages<BN, STAGES, EPI_WARPS>(), A_MN, B_MN, MATH, EPI_WARPS,
-                                 N_FAST, 2, BN == 256>(maps, p, mt, nt, num_sms, st);
   if (p.cluster == 2)
     return launch_persistent_one<BN, STAGES, A_MN, B_MN, MATH, EPI_WARPS, N_FAST, 2>(maps, p, mt, nt, num_sms, st);
   return launch_persistent_one<BN, STAGES, A_MN, B_MN, MATH, EPI_WARPS, N_FAST, 1>(maps, p, mt, nt, num_sms, st);
@@ -1568,58 +1306,6 @@ static int launch_persistent(const TmaMaps& maps, const GemmParams& p, int mt, i
   const bool math = e.alpha != 1.f || e.bias != nullptr || e.act != 0 || e.dact != 0;
   if (math) return launch_persistent_m<BN, STAGES, true>(maps, p, mt, nt, num_sms, a_mn, b_mn, st);
   return launch_persistent_m<BN, STAGES, false>(maps, p, mt, nt, num_sms, a_mn, b_mn, st);
-}
-
-template <bool N_FAST, int CLUSTER, bool PAIR = false>
-static int launch_rms_tma(const RmsMaps& maps, const GemmParams& p, int mt, int nt, int num_sms,
-                          cudaStream_t st) {
-  static_assert(!PAIR || CLUSTER == 2, "the CTA pair is a cluster of two");
-  void (*kern)(const RmsMaps, const GemmParams, const int, const int);
-  if (PAIR) kern = wgrad_rmsprop_pair_kernel<N_FAST>;
-  else kern = wgrad_rmsprop_tma_kernel<N_FAST, CLUSTER>;
-  static bool attr_set = false;
-  static int max_ctas = 0;
-  constexpr size_t smem = PAIR ? RMSP_SMEM_BYTES : RMS_SMEM_BYTES;
-  constexpr int threads = 64 + 32 * RMS_EPI_WARPS;
-  if (!attr_set) {
-    CC_CHECK_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    max_ctas = num_sms;
-    if (CLUSTER > 1) {
-      cudaLaunchConfig_t q{};
-      q.gridDim = dim3((unsigned)(num_sms / CLUSTER * CLUSTER));
-      q.blockDim = dim3(threads);
-      q.dynamicSmemBytes = smem;
-      cudaLaunchAttribute qa[1];
-      qa[0].id = cudaLaunchAttributeClusterDimension;
-      qa[0].val.clusterDim.x = CLUSTER;
-      qa[0].val.clusterDim.y = 1;
-      qa[0].val.clusterDim.z = 1;
-      q.attrs = qa;
-      q.numAttrs = 1;
-      int nclusters = 0;
-      CC_CHECK_CUDA(cudaOccupancyMaxActiveClusters(&nclusters, kern, &q));
-      CC_REQUIRE(nclusters >= 1, "cc_gemm: no %d-CTA cluster fits on this device", CLUSTER);
-      if (nclusters * CLUSTER < max_ctas) max_ctas = nclusters * CLUSTER;
-    }
-    attr_set = true;
-  }
-  const int units = ((mt + CLUSTER - 1) / CLUSTER) * nt;
-  int grid = units * CLUSTER < max_ctas ? units * CLUSTER : max_ctas / CLUSTER * CLUSTER;
-  cudaLaunchConfig_t cfg{};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(threads);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CLUSTER;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  CC_CHECK_CUDA(cudaLaunchKernelEx(&cfg, kern, maps, p, mt, nt));
-  count_launch();
-  return 0;
 }
 
 int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
@@ -1665,15 +1351,10 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
     int dev = 0;
     CC_CHECK_CUDA(cudaGetDevice(&dev));
     CC_CHECK_CUDA(cudaDeviceGetAttribute(&g_num_sms, cudaDevAttrMultiProcessorCount, dev));
-    // data-parallel runs leave SMs to the NCCL kernels that overlap the backward pass: a
-    // persistent GEMM launched with more CTAs than free SMs would run a second, serial wave
-    const int cap = ENV.sms;
-    if (cap >= 2 && cap < g_num_sms) g_num_sms = cap / 2 * 2;
   }
   const bool a_mn = d->a_mn_major != 0, b_mn = d->b_mn_major != 0;
 
-  int bn = d->force_bn ? d->force_bn : ENV.bn;
-  if (bn == 0) bn = (d->N > 128) ? 256 : 128;
+  const int bn = d->force_bn ? d->force_bn : (d->N > 128 ? 256 : 128);
   CC_REQUIRE(bn == 128 || bn == 256, "cc_gemm: BN=%d unsupported", bn);
 
   GemmParams p{};
@@ -1694,7 +1375,7 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
   int splits = 1;
   const long long Mpad = (long long)mt * BM, Npad = (long long)nt * bn;
   if (d->workspace != nullptr && d->rms_p32 == nullptr) {
-    int want = d->force_splits ? d->force_splits : ENV.splits;
+    int want = d->force_splits;
     if (want == 0) {
       // split-K only when the tile grid leaves more than half of the SMs idle (small batch,
       // long reduction: the weight-streaming regime of the reference's batch 128); otherwise
@@ -1730,19 +1411,15 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
   }
   // split-K inside the persistent kernel (work unit = tile x k-range): the operand ring and the
   // TMEM double buffer keep running across units, where the one-tile-per-CTA kernel runs one
-  // wave of short-lived CTAs whose prologues and partial-tile stores all coincide
-  const bool psk = splits >= 2 && ENV.persistent != 0 && ENV.persistent_splitk != 0;
-  const bool persistent =
-      (splits == 1 || psk) && (ENV.persistent != 0 || d->rms_p32 != nullptr ||
-                               d->route_world > 0);
+  // wave of short-lived CTAs whose prologues and partial-tile stores all coincide.  The
+  // one-tile-per-CTA kernel stays as the reference it is tested against.
+  const bool persistent = splits == 1 || ENV.persistent_splitk != 0;
 
   // 2-CTA clusters (B tile multicast) whenever there are at least two row tiles
   // (fused optimiser: only when the batch reduction is long enough for the shared B tile to
   // matter -- at the reference's batch 128 the epilogue is everything and coupling two CTAs'
   // operand rings only costs, profiles/r02_fused_rmsprop_blocked_state.jsonl)
-  const bool rms_cluster = ENV.rms_cluster < 0 ? total > 8 : ENV.rms_cluster != 0;
-  p.cluster = (persistent && mt >= 2 && ENV.cluster == 2 &&
-               (d->rms_p32 == nullptr || rms_cluster)) ? 2 : 1;
+  p.cluster = (persistent && mt >= 2 && (d->rms_p32 == nullptr || total > 8)) ? 2 : 1;
   // effective tile width of the persistent kernel: the candidate that minimises
   // waves x (per-tile cost); e.g. N = 3369 at batch 2048 is 224 tiles of 256 (1.51 waves on 148
   // SMs -> 2) but 288 tiles of 192 (1.95 waves -> 2, each shorter).  The per-tile cost model is
@@ -1770,21 +1447,6 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
   p.b_boxes = (bn_eff + 63) / 64;
   p.b_half_rows = bn_eff / 2;
   p.stage_tx = (unsigned)(BM * BK * 2 + (b_mn ? p.b_boxes * 64 * BK * 2 : bn_eff * BK * 2));
-  // CTA pair (tcgen05 cta_group::2): each CTA stages half of the B tile, which for an MN-major B
-  // must be whole 64-column TMA boxes
-  // Measured on B200 (profiles/r02_cta_pair_gemm_bench.json): correct in every orientation
-  // (tests/test_gemm_gpu.py::test_cta_pair_mma, bit-identical to the multicast scheme) but about
-  // half its throughput (Dx1 forward 664 vs 1,296 TFLOP/s): the MMA issuer is never stalled at
-  // issue, the operand ring is -- stage turn-around ~4 us against ~1.3 us -- and forwarding the
-  // peer's "stage landed" through a relay warp instead of remote complete_tx made it slower
-  // still, so the cost sits in the paired MMA's completion path, not in the barrier wiring.
-  // Off by default until that is understood; CC_GEMM_PAIR=1 selects it.
-  p.pair = (p.cluster == 2 && bn == 256 && ENV.pair != 0 && splits == 1 &&
-            (b_mn ? bn_eff % 128 == 0 : bn_eff % 32 == 0)) ? 1 : 0;
-  if (p.pair) {
-    p.b_boxes = bn_eff / 128;   // per CTA
-    p.stage_tx = (unsigned)(BM * BK * 2 + (bn_eff / 2) * BK * 2);   // per CTA
-  }
 
   for (int s = 0; s < d->nseg; ++s) {
     int rc;
@@ -1805,20 +1467,17 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
   // K advance = 32 B inside the swizzle row.  MN-major, 128B swizzle: 64-element MN atoms are
   // separate TMA boxes 64*BK*2 = 8192 B apart (LBO), 8-k groups 1024 B apart (SBO), K advance =
   // 16 rows * 128 B.
-  const uint32_t mn_lbo = (uint32_t)ENV.mn_lbo;
-  const uint32_t mn_sbo = (uint32_t)ENV.mn_sbo;
-  const uint32_t mn_kstep = (uint32_t)ENV.mn_kstep;
-  const uint32_t k_lbo = (uint32_t)ENV.k_lbo;
-  const uint32_t k_sbo = (uint32_t)ENV.k_sbo;
-  p.adesc_hi = a_mn ? desc_hi(mn_lbo, mn_sbo) : desc_hi(k_lbo, k_sbo);
-  p.bdesc_hi = b_mn ? desc_hi(mn_lbo, mn_sbo) : desc_hi(k_lbo, k_sbo);
-  p.a_kstep = a_mn ? mn_kstep : UMMA_K * 2;
-  p.b_kstep = b_mn ? mn_kstep : UMMA_K * 2;
+  const uint64_t mn_desc = desc_hi(64 * BK * 2, 1024), k_desc = desc_hi(16, 1024);
+  const uint32_t mn_kstep = UMMA_K * 128, k_kstep = UMMA_K * 2;
+  p.adesc_hi = a_mn ? mn_desc : k_desc;
+  p.bdesc_hi = b_mn ? mn_desc : k_desc;
+  p.a_kstep = a_mn ? mn_kstep : k_kstep;
+  p.b_kstep = b_mn ? mn_kstep : k_kstep;
   // cute::UMMA::InstrDescriptor: c_format F32 (1<<4), a/b format BF16 (1<<7, 1<<10),
   // a_major bit 15, b_major bit 16, N>>3 at [17,23), M>>4 at [24,29)
   p.idesc = (1u << 4) | (1u << 7) | (1u << 10) | ((a_mn ? 1u : 0u) << 15) |
             ((b_mn ? 1u : 0u) << 16) | ((uint32_t)((persistent ? bn_eff : bn) >> 3) << 17) |
-            ((uint32_t)(((persistent && p.pair) ? 2 * BM : BM) >> 4) << 24);
+            ((uint32_t)(BM >> 4) << 24);
 
   EpiParams& e = p.epi;
   e.M = d->M;
@@ -1846,13 +1505,9 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
   e.rms_rho = d->rms_rho;
   e.rms_momentum = d->rms_momentum;
   e.rms_eps = d->rms_eps;
-  // bit 0: evict-first hints on the optimiser-state stream; bit 3: 256-byte L2 fetch granularity
-  // for its loads (bits 1, 2: see the TMA-state epilogue below)
-  e.rms_cs = (ENV.rms_cs ? 1 : 0) | (ENV.rms_l2_256 ? 8 : 0);
   e.rms_blocked = d->rms_blocked;
   e.rms_row0 = d->rms_row0;
   e.rms_p16lo = d->rms_blocked ? (bf16*)d->rms_p16_lo : nullptr;
-  e.rms_keep_operands = ENV.rms_keep;
   e.route_world = d->route_world;
   e.route_shard = (unsigned)d->route_shard;
   e.route_off0 = d->route_off0;
@@ -1864,69 +1519,24 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
     // epilogue streams 26 B per element, so it gets 8 warps (twice the loads in flight) and
     // the main loop one stage less
     if (bn == 256 && d->rms_p32 != nullptr && a_mn && b_mn && d->alpha == 1.f &&
-        d->bias == nullptr && d->act == 0 && e.dact == 0 && ENV.rms_warps == 8) {
+        d->bias == nullptr && d->act == 0 && e.dact == 0) {
       // raster: walk along N (DRAM-page-local optimiser stream) when the whole B operand
       // (dZ, batch x N) stays L2-resident across row blocks; otherwise keep m fastest so the
       // CTAs of a wave share one B tile and A (X^T) is the L2-resident operand
       int nfast = ENV.rms_nfast;
       if (nfast < 0) nfast = ((long long)total * BK * d->N * 2 <= (48ll << 20)) ? 1 : 0;
-      // optimiser state moved by TMA (wgrad_rmsprop_kernel.cuh) whenever the parameter block is
-      // TMA-addressable: 16-byte aligned bases and row pitch
-      // (measured, profiles/r02_fused_rmsprop_tma_sweep.jsonl: ahead of the register epilogue
-      // while the batch reduction is short -- the reference's batch 128 -- and behind it when
-      // the operand ring is long, so the default follows the number of k-blocks)
       if (d->rms_blocked) {
         // blocked optimiser state: accumulators go straight from TMEM registers to 4 KB state
         // blocks (rms_blocked_chunk), no transpose tiles -> four operand stages
         if (p.cluster == 2)
-          return nfast ? launch_persistent_one<256, 4, true, true, false, 8, true, 2, false, true>(
+          return nfast ? launch_persistent_one<256, 4, true, true, false, 8, true, 2, true>(
                              maps, p, mt, nt, g_num_sms, st)
-                       : launch_persistent_one<256, 4, true, true, false, 8, false, 2, false, true>(
+                       : launch_persistent_one<256, 4, true, true, false, 8, false, 2, true>(
                              maps, p, mt, nt, g_num_sms, st);
-        return nfast ? launch_persistent_one<256, 4, true, true, false, 8, true, 1, false, true>(
+        return nfast ? launch_persistent_one<256, 4, true, true, false, 8, true, 1, true>(
                            maps, p, mt, nt, g_num_sms, st)
-                     : launch_persistent_one<256, 4, true, true, false, 8, false, 1, false, true>(
+                     : launch_persistent_one<256, 4, true, true, false, 8, false, 1, true>(
                            maps, p, mt, nt, g_num_sms, st);
-      }
-      int use_tma = ENV.rms_tma;
-      if (use_tma < 0) use_tma = total <= 4 ? 1 : 0;
-      const bool tma_ok =
-          use_tma != 0 && (d->rms_ld & 7) == 0 && d->beta32 == 0 &&
-          ((((uintptr_t)d->rms_p32) | ((uintptr_t)d->rms_ms) | ((uintptr_t)d->rms_mom) |
-            ((uintptr_t)d->rms_p16)) & 15) == 0 && d->out16 == nullptr;
-      if (tma_ok) {
-        RmsMaps rm;
-        memset(&rm, 0, sizeof(rm));
-        for (int s = 0; s < d->nseg; ++s) {
-          rm.a[s] = maps.a[s];
-          rm.b[s] = maps.b[s];
-        }
-        const MapKind sk = ENV.rms_l2_256 ? MAP_F32_SW128_L2_256 : MAP_F32_SW128;
-        int rc = make_map_kind(&rm.p32, d->rms_p32, (uint64_t)d->N, (uint64_t)d->M,
-                               (uint64_t)d->rms_ld, 32, 32, sk);
-        if (!rc) rc = make_map_kind(&rm.ms, d->rms_ms, (uint64_t)d->N, (uint64_t)d->M,
-                                    (uint64_t)d->rms_ld, 32, 32, sk);
-        if (!rc) rc = make_map_kind(&rm.mom, d->rms_mom, (uint64_t)d->N, (uint64_t)d->M,
-                                    (uint64_t)d->rms_ld, 32, 32, sk);
-        if (!rc && d->rms_p16 != nullptr)
-          rc = make_map_kind(&rm.p16, d->rms_p16, (uint64_t)d->N, (uint64_t)d->M,
-                             (uint64_t)d->rms_ld, 32, 32, MAP_BF16_SW64);
-        if (rc) return rc;
-        // bit 1: bf16 weight copy written by row stores from registers instead of a TMA store
-        if (ENV.rms_p16_tma == 0) p.epi.rms_cs |= 2;
-        // bit 2: the two epilogue warps of a lane quarter interleave their 32-column blocks
-        if (ENV.rms_interleave != 0) p.epi.rms_cs |= 4;
-        // (the TMA-state kernels build their own instruction descriptor M from this one's)
-        p.idesc = (p.idesc & ~(0x1Fu << 24)) | ((uint32_t)(BM >> 4) << 24);
-        // CTA pair (cta_group::2, 256-row tiles) whenever there are at least two row tiles
-        if (p.cluster == 2 && ENV.rms_pair != 0)
-          return nfast ? launch_rms_tma<true, 2, true>(rm, p, mt, nt, g_num_sms, st)
-                       : launch_rms_tma<false, 2, true>(rm, p, mt, nt, g_num_sms, st);
-        if (p.cluster == 2)
-          return nfast ? launch_rms_tma<true, 2>(rm, p, mt, nt, g_num_sms, st)
-                       : launch_rms_tma<false, 2>(rm, p, mt, nt, g_num_sms, st);
-        return nfast ? launch_rms_tma<true, 1>(rm, p, mt, nt, g_num_sms, st)
-                     : launch_rms_tma<false, 1>(rm, p, mt, nt, g_num_sms, st);
       }
       if (nfast != 0)
         return launch_persistent_cfg<256, 3, true, true, false, 8, true>(maps, p, mt, nt, g_num_sms, st);

@@ -279,24 +279,16 @@ def test_wgrad_with_fused_rmsprop_epilogue(K, N, B):
     assert torch.equal(p32b, p32) and torch.equal(msb, ms)
 
 
-@pytest.mark.parametrize("mode", ["pair", "tma", "tma16", "reg"])
 @pytest.mark.parametrize("nfast", ["0", "1"])
 @pytest.mark.parametrize("K,N,B", [(1000, 1300, 256), (385, 2049, 96), (64, 300, 40),
                                    (700, 520, 2048)])
-def test_fused_rmsprop_epilogue_paths(K, N, B, nfast, mode, monkeypatch):
-    """The fused-optimiser epilogues -- "pair": CTA pair (tcgen05 cta_group::2, 256-row tiles)
-    with the optimiser state moved by TMA through swizzled shared memory; "tma": the same
-    epilogue on one-CTA tiles; "tma16": also the bf16 copy by TMA store; "reg": the register
-    path of the generic persistent kernel -- on both tile rasters, several row / column tiles
-    with ragged edges, a single row tile (K = 64: no cluster), a long batch reduction (32
-    k-blocks: the operand ring wraps many times), with and without the bf16 copy, with and
-    without the gradient output.  Padding must stay untouched, except that a TMA store clips at
-    16-byte granularity: up to 3 fp32 / 7 bf16 padding elements next to column N are rewritten
-    with the update of zeros, i.e. zeros (the engine's padding is zero and stays zero)."""
+def test_fused_rmsprop_epilogue_paths(K, N, B, nfast, monkeypatch):
+    """The fused-optimiser epilogue with row-major state (the register path of the generic
+    persistent kernel) on both tile rasters, several row / column tiles with ragged edges, a
+    single row tile (K = 64: no cluster), a long batch reduction (32 k-blocks: the operand ring
+    wraps many times), with and without the bf16 copy, with and without the gradient output.
+    Padding must stay untouched."""
     ops = _ops()
-    monkeypatch.setenv("CC_GEMM_RMS_TMA", "0" if mode == "reg" else "1")
-    monkeypatch.setenv("CC_GEMM_RMS_PAIR", "1" if mode == "pair" else "0")
-    monkeypatch.setenv("CC_GEMM_RMS_P16_TMA", "1" if mode == "tma16" else "0")
     monkeypatch.setenv("CC_GEMM_RMS_NFAST", nfast)
     x, dz = _rand(B, K, 90, 0.5), _rand(B, N, 91, 0.01)
     ld = ops.pad_ld(N)
@@ -337,14 +329,9 @@ def test_fused_rmsprop_epilogue_paths(K, N, B, nfast, mode, monkeypatch):
             assert float((dwf[:, N:] - 7.0).abs().sum()) == 0.0
         if with16:
             assert torch.equal(p16f[:, :N], p32f[:, :N].to(torch.bfloat16))
-        # padding columns: untouched beyond the 16-byte granule that holds column N - 1
-        for t, tma_store in ((p32f, mode != "reg"), (msf, mode != "reg"), (momf, mode != "reg"),
-                             (p16f, mode == "tma16" and with16)):
-            per16 = 16 // t.element_size()
-            edge = (N + per16 - 1) // per16 * per16 if tma_store else N
-            assert float((t[:, edge:].float() - 7.0).abs().sum()) == 0.0
-            rim = t[:, N:edge].float()
-            assert bool(((rim == 7.0) | (rim == 0.0)).all())
+        # padding columns: untouched
+        for t in (p32f, msf, momf, p16f):
+            assert float((t[:, N:].float() - 7.0).abs().sum()) == 0.0
 
 
 @pytest.mark.parametrize("nfast", ["0", "1"])
@@ -360,7 +347,6 @@ def test_fused_rmsprop_blocked_state(K0, K1, N, B, nfast, monkeypatch):
     padding rows and padding columns of the state stay zero."""
     ops = _ops()
     monkeypatch.setenv("CC_GEMM_RMS_NFAST", nfast)
-    monkeypatch.setenv("CC_GEMM_RMS_TMA", "0")
     K = K0 + K1
     R, ld = (K + 31) // 32 * 32, ops.pad_ld(N)
     lr, rho, mo, eps = 0.0075, 0.85, 0.1, 1e-7
@@ -454,19 +440,15 @@ def test_effective_tile_width(bn_eff, orient, monkeypatch):
     _check(out16, ref, K, True)
 
 
-@pytest.mark.parametrize("pair", ["1", "0"])
 @pytest.mark.parametrize("orient", ["fwd", "dgrad", "wgrad"])
 @pytest.mark.parametrize("M,N,K,segs", [(300, 1000, 200, 1), (1000, 517, 2100, 1), (257, 264, 70, 1),
                                         (640, 2300, 96, 3)])
-def test_cta_pair_mma(M, N, K, segs, orient, pair, monkeypatch):
-    """pair = "1": two SMs run one tcgen05 cta_group::2 MMA on a 256-row tile (each CTA stages
-    half of the B tile, a 6-stage operand ring); "0": the 2-CTA multicast scheme with one
-    cta_group::1 MMA per CTA.  Both against the fp32 product, and bit-identical to each other
-    (same tiles, same k order, same accumulation): all three operand-major combinations, odd
-    row-tile counts (the second CTA of the last pair idles), ragged N, a long reduction that
-    wraps the ring, and several accumulating segments."""
+def test_cluster_multicast_mma(M, N, K, segs, orient, monkeypatch):
+    """The 2-CTA multicast scheme (two CTAs on vertically adjacent tiles, each loading half of
+    the shared B tile into both) against the fp32 product: all three operand-major
+    combinations, odd row-tile counts (the second CTA of the last pair idles), ragged N, a long
+    reduction that wraps the ring, and several accumulating segments."""
     ops = _ops()
-    monkeypatch.setenv("CC_GEMM_PAIR", pair)
     monkeypatch.setenv("CC_GEMM_BN_EFF", "256")
     bias = torch.randn(N, device="cuda")
     a_list, b_list, ref = [], [], 0
@@ -490,13 +472,6 @@ def test_cta_pair_mma(M, N, K, segs, orient, pair, monkeypatch):
     want = torch.sigmoid(ref + bias.cpu())
     _check(out32, want, K * segs, False)
     _check(out16, want, K * segs, True)
-    if pair == "1":
-        monkeypatch.setenv("CC_GEMM_PAIR", "0")
-        other = ops.alloc2d(M, N, dtype=torch.float32)
-        ops.gemm(M, N, a_list, b_list, [K] * segs, am, bm, bias=bias, act=ops.ACT_SIGMOID,
-                 out32=other, use_ws=False)
-        torch.cuda.synchronize()
-        assert torch.equal(other, out32)
 
 
 def test_effective_tile_width_auto_matches_full_width(monkeypatch):
