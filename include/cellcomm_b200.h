@@ -293,6 +293,12 @@ int cc_split_bf16(const void* x, int64_t ldx, void* hi, int64_t ldhi, void* lo, 
  * mask_u8 != NULL: explicit keep mask (parity tests inject TF's masks this way).
  * mask_u8 == NULL: keep = philox(seed, *counter_dev, stream_id, r, c) >= rate;
  * the same call with the same arguments regenerates the mask in backward.
+ * The stream: u(r, c) = top 24 bits of word c % 4 of the Philox-4x32-10 block with key = seed,
+ * counter lo = r * ceil(cols / 4) + c / 4, counter hi = (stream_id << 40) ^ step (step =
+ * *counter_dev, 0 when counter_dev is NULL), times 2^-24.  It depends on the layout and the
+ * launch geometry not at all (tests/tail_ref.py holds a host port).  Limits of that counter:
+ * stream ids are distinct below 2^24 only (id + 2^24 aliases id), and a step of 2^40 or more
+ * overlaps the id bits (step 2^40 of id 0 is step 0 of id 1).
  * dtypes: x, out */
 int cc_dropout(const void* x, int64_t ldx, void* out, int64_t ldo, int64_t rows, int64_t cols,
                float rate, const uint8_t* mask_u8, int64_t ldm, uint64_t seed,
@@ -302,7 +308,9 @@ int cc_dropout(const void* x, int64_t ldx, void* out, int64_t ldo, int64_t rows,
 int cc_dropout_mask(uint8_t* mask_u8, int64_t ldm, int64_t rows, int64_t cols, float rate,
                     uint64_t seed, const uint64_t* counter_dev, uint32_t stream_id,
                     cc_stream_t stream);
-/* uniform [0,1) floats: tf.random.uniform (src/bigan_basic.py:36-37, bigan_cont.py:52-53) */
+/* uniform floats, tf.random.uniform (src/bigan_basic.py:36-37, bigan_cont.py:52-53): out32 is the
+ * dropout stream u(r, c) above, in [0, 1) on a 2^-24 grid.  out16 (may be NULL, shares ld) is
+ * bf16_rn(u), so it lies in [0, 1]: draws u >= 1 - 2^-9 (about 0.2 %) round to exactly 1.0. */
 int cc_uniform(float* out32, void* out16, int64_t ld, int64_t rows, int64_t cols, uint64_t seed,
                const uint64_t* counter_dev, uint32_t stream_id, cc_stream_t stream);
 int cc_counter_add(uint64_t* counter_dev, uint64_t inc, cc_stream_t stream);
@@ -318,7 +326,13 @@ int cc_copy2d(const void* src, int64_t lds, void* dst, int64_t ldd, int64_t rows
 
 /* BatchNormalization (Keras 2.4 defaults: eps=1e-3, momentum=0.99), SURVEY A.3.
  * stats: sums[0:cols] = sum_r x, sums[cols:2cols] = sum_r x^2 (fp32, overwritten).
- * The caller may all-reduce `sums` across ranks before cc_bn_train_apply.  dtypes: x */
+ * The caller may all-reduce `sums` across ranks before cc_bn_train_apply.  dtypes: x
+ * One pass: the variance is E[x^2] - E[x]^2 from these fp32 sums (Keras's tf.nn.moments takes
+ * two passes), so it loses about u * E[x^2] (u = 2^-24 times the additions in the chain) to
+ * cancellation.  Harmless while the mean stays within ~30x the spread (inputs in [0, 1], the
+ * networks' activations: save_rstd within 1e-3 relative); beyond that, measured on an NVIDIA
+ * B200 (1,000 W) at 2048 rows, eps 1e-3, the largest relative error of save_rstd is 2.7e-3 at
+ * mean/std 100, 2.5e-2 at 300 and 0.48 at 1000 (tests/test_tail_kernels_ref_gpu.py). */
 int cc_bn_stats(const void* x, int64_t ld, int64_t rows, int64_t cols, float* sums,
                 int32_t dtypes, cc_stream_t stream);
 int cc_bn_stats_ws(const void* x, int64_t ld, int64_t rows, int64_t cols, float* sums,
