@@ -194,8 +194,9 @@ __device__ __forceinline__ void epilogue_store32(const EpiParams& e, int r, int 
   if (ncols <= 0) return;
 #pragma unroll
   for (int j = 0; j < 32; ++j) {
-    float x = v[j] * e.alpha;
-    if (e.bias != nullptr && j < ncols) x += __ldg(e.bias + c0 + j);
+    // fmaf(v, alpha, bias), one rounding: epilogue_chunk (persistent kernel) and
+    // splitk_finalize_kernel compute the same expression, so the bits do not depend on the path
+    float x = fmaf(v[j], e.alpha, (e.bias != nullptr && j < ncols) ? __ldg(e.bias + c0 + j) : 0.f);
     if (e.act == CC_ACT_SIGMOID) x = sigmoidf_(x);
     else if (e.act == CC_ACT_RELU) x = fmaxf(x, 0.f);
     v[j] = x;
@@ -418,19 +419,23 @@ __device__ __forceinline__ void epilogue_chunk(const EpiParams& e, float* stage 
     const long long step = 4 * e.ld32;
     const unsigned last = (unsigned)e.route_world - 1u;
     const bool vec = ncol == 4 && (e.ld32 & 3) == 0 && ((c & 3) == 0);
+    auto owner_of = [&](long long rel) {
+      return min((unsigned)((unsigned long long)rel / e.route_shard), last);
+    };
 #pragma unroll
     for (int t = 0; t < 8; ++t) {
       if (t < nrow) {
         const long long rel = rel0 + t * step;
-        const unsigned owner = min((unsigned)((unsigned long long)rel / e.route_shard), last);
-        float* dst = e.route_base[owner] + rel;
         if (vec) {
-          *reinterpret_cast<float4*>(dst) = g[t];
+          // rel % 4 == 0 and route_shard % 8 == 0: the four elements have one owner
+          *reinterpret_cast<float4*>(e.route_base[owner_of(rel)] + rel) = g[t];
         } else {
-          dst[0] = g[t].x;
-          if (ncol > 1) dst[1] = g[t].y;
-          if (ncol > 2) dst[2] = g[t].z;
-          if (ncol > 3) dst[3] = g[t].w;
+          // rel % 4 != 0 when ld32 % 4 != 0: a shard boundary may fall inside the four
+          // columns, so every element finds its own owner
+          e.route_base[owner_of(rel)][rel] = g[t].x;
+          if (ncol > 1) e.route_base[owner_of(rel + 1)][rel + 1] = g[t].y;
+          if (ncol > 2) e.route_base[owner_of(rel + 2)][rel + 2] = g[t].z;
+          if (ncol > 3) e.route_base[owner_of(rel + 3)][rel + 3] = g[t].w;
         }
       }
     }
@@ -1022,8 +1027,7 @@ __global__ void splitk_finalize_kernel(const EpiParams e, const float* __restric
   const int ncols = min(4, e.N - c0);
 #pragma unroll
   for (int j = 0; j < 4; ++j) {
-    float x = v[j] * e.alpha;
-    if (e.bias != nullptr && j < ncols) x += __ldg(e.bias + c0 + j);
+    float x = fmaf(v[j], e.alpha, (e.bias != nullptr && j < ncols) ? __ldg(e.bias + c0 + j) : 0.f);
     if (e.act == CC_ACT_SIGMOID) x = sigmoidf_(x);
     else if (e.act == CC_ACT_RELU) x = fmaxf(x, 0.f);
     v[j] = x;
@@ -1327,12 +1331,16 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
                    d->out16 == nullptr && d->beta32 == 0 && d->route_world == 0 &&
                    d->force_splits <= 1 && (d->force_bn == 0 || d->force_bn == 256),
                "cc_gemm: rms_blocked is for plain weight-gradient GEMMs (X^T dZ, N > 128)");
-    CC_REQUIRE(d->rms_row0 >= 0 && (d->rms_ld & 31) == 0 &&
+    // the bf16 copies and out32 are written in whole 32-column chunks (zeros past N), so their
+    // rows must be at least round_up(N, 32) long or a chunk spills into the next row
+    const long long n32 = ((long long)d->N + 31) / 32 * 32;
+    CC_REQUIRE(d->rms_row0 >= 0 && (d->rms_ld & 31) == 0 && d->rms_ld >= n32 &&
                    ((((uintptr_t)d->rms_p32) | ((uintptr_t)d->rms_ms) | ((uintptr_t)d->rms_mom) |
                      ((uintptr_t)d->rms_p16) | ((uintptr_t)d->rms_p16_lo) | ((uintptr_t)d->out32)) & 15) == 0 &&
-                   (d->out32 == nullptr || (d->ld32 & 3) == 0),
-               "cc_gemm: rms_blocked needs 16-byte aligned blocks, rms_ld %% 32 == 0 (rms_ld=%lld)",
-               (long long)d->rms_ld);
+                   (d->out32 == nullptr || ((d->ld32 & 3) == 0 && d->ld32 >= n32)),
+               "cc_gemm: rms_blocked needs 16-byte aligned blocks, rms_ld %% 32 == 0 and rms_ld, "
+               "ld32 >= round_up(N, 32) (N=%d rms_ld=%lld ld32=%lld)",
+               d->N, (long long)d->rms_ld, (long long)d->ld32);
   }
   CC_REQUIRE(d->rms_p16_lo == nullptr || d->rms_blocked,
              "cc_gemm: rms_p16_lo is written by the blocked fused-optimiser epilogue only");
@@ -1345,7 +1353,9 @@ int gemm_impl(const cc_gemm_desc* d, cudaStream_t st) {
                "cc_gemm: route_shard=%lld route_off0=%lld", (long long)d->route_shard,
                (long long)d->route_off0);
     for (int q = 0; q < d->route_world; ++q)
-      CC_REQUIRE(d->route_base[q] != nullptr, "cc_gemm: route_base[%d] is null", q);
+      CC_REQUIRE(d->route_base[q] != nullptr && ((uintptr_t)d->route_base[q] & 15) == 0,
+                 "cc_gemm: route_base[%d]=%p is null or not 16-byte aligned", q,
+                 (const void*)d->route_base[q]);
   }
   if (g_num_sms == 0) {
     int dev = 0;

@@ -127,8 +127,8 @@ int cc_gather_rows(const int64_t* rowptr_dev, const int32_t* colidx_dev, const f
  *            = 1: B_s is stored [K_s, N] row-major (N contiguous)
  *
  * epilogue, per element (r,c), v = acc:
- *   v = alpha * v
- *   if bias:   v += bias[c]
+ *   v = fmaf(v, alpha, bias ? bias[c] : 0)   (one rounding; the same in every kernel
+ *                                            and split-K path)
  *   act:       0 none, 1 sigmoid, 2 relu
  *   if dact:   v *= act'(y[r,c])   (1: y(1-y)  2: y>0)   y = dact_y (bf16)
  *   if out32:  out32[r,c] = v + (beta32 ? out32[r,c] : 0)
@@ -184,7 +184,8 @@ typedef struct cc_gemm_desc {
    * the bucket start, = route_off0 + row*ld32 + col) belongs to rank rel / route_shard and is
    * stored to route_base[owner] + rel -- this rank's slot in the OWNER's staging buffer, a
    * peer-mapped pointer over NVLink (the own share goes to local memory).  out32 must be set
-   * (it is the local address of element (0,0)); beta32 and split-K are not available. */
+   * (it is the local address of element (0,0)); beta32 and split-K are not available.  Every
+   * route_base[q] must be 16-byte aligned: the vector path stores float4 to route_base + rel. */
   int32_t route_world;   /* 0: off */
   int64_t route_shard;   /* elements per rank, multiple of 8 */
   int64_t route_off0;    /* offset of out32[0,0] from the bucket start, multiple of 4 */
@@ -205,7 +206,9 @@ typedef struct cc_gemm_desc {
    * 512 contiguous bytes and each 32 x 32 chunk one DRAM-page-local 4 KB block per array.
    * rms_row0 is the layer row of this GEMM's row 0 (the row offset of a Concatenate segment;
    * any value >= 0).  rms_p16 (the bf16 compute copy, a TMA operand elsewhere) and out32 stay
-   * row-major views of this GEMM's own [M, N] slice. */
+   * row-major views of this GEMM's own [M, N] slice.  They, and rms_p16_lo, are written in whole
+   * 32-column chunks (zeros between N and the chunk edge), so rms_ld and ld32 must be at least
+   * round_up(N, 32). */
   int32_t rms_blocked;
   int32_t rms_row0;
   /* blocked layout only, optional: the low-order bf16 term bf16(w - float(bf16(w))) of the
