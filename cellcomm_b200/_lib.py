@@ -165,6 +165,9 @@ SIGNATURES = {
     "cc_recon_sqerr": (C.c_int, [vp, c_i64, c_i64, c_i64, vp, vp, vp, c_i64, c_f32, vp, vp]),
     "cc_col_moments": (C.c_int, [vp, c_i64, c_i64, c_i64, c_i32, vp, vp, vp, vp, c_i64, vp]),
     "cc_col_moments_ws_bytes": (c_i64, [c_i64, c_i64]),
+    "cc_log1p_features": (C.c_int, [vp, c_i64, c_i64, c_i64, c_i32, vp, c_i64, vp, vp, vp]),
+    "cc_mmd_sums": (C.c_int, [vp, c_i64, c_i64, vp, c_i32, vp, c_i64, vp, vp, c_i64, vp]),
+    "cc_mmd_sums_ws_bytes": (c_i64, [c_i64, c_i32, c_i64]),
     "cc_argmax_onehot": (C.c_int, [vp, c_i64, vp, c_i64, vp, c_i64, c_i64, c_i64, vp]),
     "cc_rmsprop_step": (C.c_int, [vp, vp, vp, vp, vp, c_i64, c_i64, c_i64, c_f32, c_f32, c_f32,
                                   c_f32, c_f32, vp]),

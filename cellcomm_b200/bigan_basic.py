@@ -114,6 +114,155 @@ def comparison_summary(comparison):
     return rows
 
 
+# two_sample_test, per group k: the cells tested on each side (int64 [K]), the lower median of
+# the pooled squared distances (float64 [K]), MMD^2 and its permutation p-value per bandwidth
+# scale of MMD_SCALES (float64 [K, 3]), and the Kolmogorov-Smirnov D of the per-cell library
+# size and genes detected, real against generated (float64 [K])
+TwoSampleTest = namedtuple("TwoSampleTest", [
+    "real_cells", "generated_cells", "sqdist_median", "mmd2", "p_value", "library_size_ks",
+    "genes_detected_ks"])
+
+MMD_SCALES = (0.5, 1.0, 2.0)      # kernel bandwidths s * median
+MAX_TEST_CELLS = 16384            # per group and side: bounds the [2n, 2n] Gram matrix
+
+
+def mmd_from_sums(n, xx, yy, xy):
+    """Unbiased MMD^2 of two samples of n cells each from their kernel sums over ordered pairs
+    i != j: XX (both in X), YY (both in Y), XY (i in X, j in Y):
+        XX / (n (n - 1)) + YY / (n (n - 1)) - 2 XY / n^2
+    Every path (the dense definition and the streamed device pass) ends here."""
+    n = float(n)
+    xx, yy, xy = (np.asarray(v, dtype=np.float64) for v in (xx, yy, xy))
+    return xx / (n * (n - 1)) + yy / (n * (n - 1)) - 2.0 * xy / (n * n)
+
+
+def permutation_p_value(mmd2):
+    """p = (1 + #{p >= 1 : MMD^2_p >= MMD^2_0}) / L over the first axis of mmd2 ([L, ...]):
+    labelling 0 is the observed one, 1..L-1 the permutations."""
+    mmd2 = np.asarray(mmd2, dtype=np.float64)
+    return (1.0 + np.sum(mmd2[1:] >= mmd2[0], axis=0)) / len(mmd2)
+
+
+def ks_statistic(a, b):
+    """Two-sample Kolmogorov-Smirnov statistic D = max |F_a - F_b| of the empirical CDFs."""
+    a = np.sort(np.asarray(a, dtype=np.float64))
+    b = np.sort(np.asarray(b, dtype=np.float64))
+    if len(a) == 0 or len(b) == 0:
+        return float("nan")
+    v = np.concatenate([a, b])
+    fa = np.searchsorted(a, v, side="right") / len(a)
+    fb = np.searchsorted(b, v, side="right") / len(b)
+    return float(np.max(np.abs(fa - fb)))
+
+
+def bf16_round(x):
+    """float32 -> the float32 value of its bf16 rounding, half to even; NaN stays NaN."""
+    u = np.ascontiguousarray(x, dtype=np.float32).view(np.uint32)
+    nan = (u & 0x7FFFFFFF) > 0x7F800000
+    r = ((u.astype(np.uint64) + 0x7FFF + ((u >> 16) & 1)) >> 16).astype(np.uint32)
+    r = np.where(nan, (u >> 16) | 0x40, r)
+    return (r << 16).astype(np.uint32).view(np.float32)
+
+
+def log1p_features(v):
+    """The test's per-gene feature bf16(float32(log1p(float64(v))))."""
+    return bf16_round(np.log1p(np.asarray(v, dtype=np.float64)).astype(np.float32))
+
+
+def two_sample_args(max_cells, permutations, seed):
+    """Checked (max_cells, permutations, seed) of two_sample_test."""
+    max_cells, permutations, seed = int(max_cells), int(permutations), int(seed)
+    if not 2 <= max_cells <= MAX_TEST_CELLS:
+        raise ValueError(f"max_cells must lie in [2, {MAX_TEST_CELLS}], got {max_cells}")
+    if permutations < 0:
+        raise ValueError(f"permutations must be >= 0, got {permutations}")
+    if seed < 0:
+        raise ValueError(f"seed must be >= 0, got {seed}")
+    return max_cells, permutations, seed
+
+
+def two_sample_cells(labels, K, max_cells, seed):
+    """Per group k, the real cells two_sample_test takes (row numbers, ascending): all of the
+    group's cells, or max_cells of them drawn with default_rng([seed, 0, k]) and sorted."""
+    picks = []
+    for k in range(K):
+        rows = np.flatnonzero(labels == k).astype(np.int64)
+        if len(rows) > max_cells:
+            rows = rows[np.sort(np.random.default_rng([seed, 0, k]).choice(
+                len(rows), max_cells, replace=False))]
+        picks.append(rows)
+    return picks
+
+
+def two_sample_labellings(n, permutations, seed, k):
+    """bool [permutations + 1, 2n]: row 0 puts the first n pooled cells in X, row p >= 1 the
+    cells rng.permutation(2n)[:n], drawn in order from rng = default_rng([seed, 1, k])."""
+    N = 2 * n
+    out = np.zeros((permutations + 1, N), dtype=bool)
+    out[0, :n] = True
+    rng = np.random.default_rng([seed, 1, k])
+    for p in range(1, permutations + 1):
+        out[p, rng.permutation(N)[:n]] = True
+    return out
+
+
+def pack_labellings(labellings):
+    """bool [L, N] -> uint32 [L, ceil(N / 32)]: bit i % 32 of word i // 32 is cell i."""
+    L, N = labellings.shape
+    W = (N + 31) // 32
+    padded = np.zeros((L, W * 32), dtype=bool)
+    padded[:, :N] = labellings
+    return np.packbits(padded, axis=1, bitorder="little").view("<u4").astype(np.uint32)
+
+
+def kernel_sums(d2, masks, scale_bandwidths):
+    """Definition of the kernel sums: fp64 [L, len(scale_bandwidths), 3] of XX, YY, XY per
+    labelling (bool masks [L, N], True = X) with k = exp(-d2 / h) for every h, summed over
+    ordered pairs i != j."""
+    d2 = np.asarray(d2, dtype=np.float64)
+    B = np.asarray(masks, dtype=np.float64)
+    out = np.empty((len(B), len(scale_bandwidths), 3))
+    for b, h in enumerate(scale_bandwidths):
+        k = np.exp(-d2 / h)
+        np.fill_diagonal(k, 0.0)
+        r = k.sum(1)
+        xx = np.einsum("pi,ip->p", B, k @ B.T)
+        rb = B @ r
+        out[:, b, 0] = xx
+        out[:, b, 1] = r.sum() - 2.0 * rb + xx
+        out[:, b, 2] = rb - xx
+    return out
+
+
+def lower_median(values):
+    v = np.sort(np.asarray(values).reshape(-1))
+    return float(v[(len(v) - 1) // 2]) if len(v) else float("nan")
+
+
+def two_sample_result(counts, medians, sums, lib, det):
+    """TwoSampleTest from per-group cell counts n_k, medians, kernel sums ([L, 3, 3] or None for
+    a group without a test) and (real, generated) pairs of per-cell library sizes and genes
+    detected.  Every path ends here."""
+    K = len(counts)
+    n = np.asarray(counts, dtype=np.int64)
+    med = np.full(K, np.nan)
+    mmd2 = np.full((K, len(MMD_SCALES)), np.nan)
+    p = np.full((K, len(MMD_SCALES)), np.nan)
+    lib_ks = np.full(K, np.nan)
+    det_ks = np.full(K, np.nan)
+    for k in range(K):
+        if n[k] < 2:
+            continue
+        med[k] = medians[k]
+        lib_ks[k] = ks_statistic(*lib[k])
+        det_ks[k] = ks_statistic(*det[k])
+        if sums[k] is not None and med[k] > 0:
+            stats = mmd_from_sums(n[k], sums[k][..., 0], sums[k][..., 1], sums[k][..., 2])
+            mmd2[k] = stats[0]
+            p[k] = permutation_p_value(stats)
+    return TwoSampleTest(n, n.copy(), med, mmd2, p, lib_ks, det_ks)
+
+
 class BasicBiGan:
     def __init__(self, encoding_size, gene_size,
                  generator_factory: Callable[[int, int], object],
@@ -243,6 +392,55 @@ class BasicBiGan:
         """Generated-cell encodings for compare_cells, counts[k] of them for group k in group
         order: random_encoding_vector over all of them."""
         return self.random_encoding_vector(int(np.sum(counts)))
+
+    def two_sample_test(self, cell_data, max_cells=4096, permutations=1000, seed=0):
+        """Kernel two-sample test of real against generated cells, per group -> TwoSampleTest.
+        Groups come from _comparison_groups.  Group k tests its real cells (max_cells of them,
+        two_sample_cells, when it has more) against as many generated ones; the generated
+        cells are drawn as compare_cells draws them (_comparison_encodings for every group,
+        then random_uniform_vector(total), generate_cells).  Per cell, the features are
+        log1p_features(v) over genes (v the count; the generator's rounded output), and the
+        pooled Gram matrix G = F F^T (real cells first) gives d2_ij = max(G_ii + G_jj - 2 G_ij,
+        0).  With m the lower median of d2 over i < j, MMD^2 (mmd_from_sums) is taken for
+        k(i, j) = exp(-d2_ij / (s m)), s in MMD_SCALES, on the observed split and on
+        `permutations` random ones (two_sample_labellings), giving permutation_p_value.  KS D
+        of the library size and genes detected per cell closes the result.  Groups with fewer
+        than 2 cells report their counts and NaN; a zero median gives NaN MMD^2 and p.  The
+        subsample and labellings are seeded from `seed` alone.  This is the definition, dense
+        fp64 numpy; engine-backed subclasses stream it on the device."""
+        max_cells, permutations, seed = two_sample_args(max_cells, permutations, seed)
+        x = np.asarray(cell_data, dtype=np.float64)
+        if x.ndim != 2:
+            raise ValueError(f"expected cells of shape (n, genes), got {x.shape}")
+        if np.any(x < 0):
+            raise ValueError("two_sample_test: the cells hold negative counts")
+        labels, K = self._comparison_groups(cell_data)
+        picks = two_sample_cells(labels, K, max_cells, seed)
+        counts = [len(p) for p in picks]
+        encodings = self._comparison_encodings(counts)
+        noise = self.random_uniform_vector(len(encodings))
+        generated = np.asarray(self.generate_cells(encodings, noise), dtype=np.float64)
+        medians, sums, lib, det = [], [], [], []
+        off = 0
+        for k in range(K):
+            n = counts[k]
+            real, gen = x[picks[k]], generated[off:off + n]
+            off += n
+            lib.append((real.sum(1), gen.sum(1)))
+            det.append((np.count_nonzero(real, axis=1), np.count_nonzero(gen, axis=1)))
+            if n < 2:
+                medians.append(np.nan)
+                sums.append(None)
+                continue
+            F = np.concatenate([log1p_features(real), log1p_features(gen)]).astype(np.float64)
+            G = F @ F.T
+            g = np.diag(G)
+            d2 = np.maximum(g[:, None] + g[None, :] - 2.0 * G, 0.0)
+            m = lower_median(d2[np.triu_indices(2 * n, 1)])
+            medians.append(m)
+            sums.append(kernel_sums(d2, two_sample_labellings(n, permutations, seed, k),
+                                    [s * m for s in MMD_SCALES]) if m > 0 else None)
+        return two_sample_result(counts, medians, sums, lib, det)
 
     @abstractmethod
     def trainings_step(self, sampled_batch):

@@ -15,14 +15,18 @@ from typing import Callable
 import numpy as np
 
 try:
-    from .bigan_basic import (BasicBiGan, CellScores, group_labels, require_sorted,
-                              statistics_from_sums)
+    from .bigan_basic import (BasicBiGan, CellScores, MMD_SCALES, group_labels,
+                              pack_labellings, require_sorted, statistics_from_sums,
+                              two_sample_args, two_sample_cells, two_sample_labellings,
+                              two_sample_result)
     from . import engine as _engine
     from .models import NetModel, RMSprop, losses, activations  # noqa: F401
     from .cell_type_training import CellBatch, CellMatrix
 except ImportError:  # imported as top-level modules (PYTHONPATH=src style)
-    from bigan_basic import (BasicBiGan, CellScores, group_labels, require_sorted,
-                             statistics_from_sums)
+    from bigan_basic import (BasicBiGan, CellScores, MMD_SCALES, group_labels,
+                             pack_labellings, require_sorted, statistics_from_sums,
+                             two_sample_args, two_sample_cells, two_sample_labellings,
+                             two_sample_result)
     from cellcomm_b200 import engine as _engine
     from cellcomm_b200.models import NetModel, RMSprop, losses, activations  # noqa: F401
     from cellcomm_b200.cell_type_training import CellBatch, CellMatrix
@@ -469,6 +473,53 @@ class ClassifyCellBiGan(BasicBiGan):
                                            r32=np.asarray(random_in, dtype=np.float32),
                                            tile_rows=self.PREDICT_TILE)
         return statistics_from_sums(counts, *(t.cpu().numpy() for t in sums))
+
+    def two_sample_test(self, cell_data, max_cells=4096, permutations=1000, seed=0):
+        """BasicBiGan.two_sample_test, streamed on the device: the generated cells of every
+        group are one features_stream over the generator (tiled like generate_cells, so the
+        same bits), each group's real cells one features_stream over the device CSR, and
+        BiGanEngine.mmd_sums forms the Gram matrix with cc_gemm, the median with kthvalue and
+        the kernel sums of all labellings with cc_mmd_sums.  Only the medians, the per-cell
+        library sizes and genes detected and the [L, 3, 3] sums come back to the host.  A
+        CellMatrix is read as it is; anything else is first wrapped with
+        CellMatrix.from_dense.  Rank-local in data-parallel runs (no collective)."""
+        if self._engine is None:
+            return super().two_sample_test(cell_data, max_cells, permutations, seed)
+        max_cells, permutations, seed = two_sample_args(max_cells, permutations, seed)
+        mat = cell_data if isinstance(cell_data, CellMatrix) else CellMatrix.from_dense(cell_data)
+        if mat.shape[1] != self.gene_size:
+            raise ValueError(f"expected cells with {self.gene_size} genes, got {mat.shape[1]}")
+        if np.any(mat.values64 < 0):
+            raise ValueError("two_sample_test: the cells hold negative counts")
+        labels, K = self._comparison_groups(mat)
+        picks = two_sample_cells(labels, K, max_cells, seed)
+        counts = [len(p) for p in picks]
+        encodings = np.asarray(self._comparison_encodings(counts), dtype=np.float32)
+        noise = self.random_uniform_vector(len(encodings))
+        eng = self._engine
+        gen_f, gen_lib, gen_det = eng.features_stream(z32=encodings, r32=noise,
+                                                      tile_rows=self.PREDICT_TILE)
+        gen_lib, gen_det = gen_lib.cpu().numpy(), gen_det.cpu().numpy()
+        csr = mat.device_csr(eng.device)
+        medians, sums, lib, det = [], [], [], []
+        off = 0
+        for k in range(K):
+            n = counts[k]
+            fx, x_lib, x_det = eng.features_stream(csr=csr, order=picks[k],
+                                                   tile_rows=self.PREDICT_TILE)
+            lib.append((x_lib.cpu().numpy(), gen_lib[off:off + n]))
+            det.append((x_det.cpu().numpy(), gen_det[off:off + n]))
+            if n < 2:
+                medians.append(np.nan)
+                sums.append(None)
+            else:
+                masks = pack_labellings(two_sample_labellings(n, permutations, seed, k))
+                m, s = eng.mmd_sums(fx, gen_f[off:off + n], MMD_SCALES, masks)
+                medians.append(m)
+                sums.append(s)
+            off += n
+            del fx
+        return two_sample_result(counts, medians, sums, lib, det)
 
     def _comparison_groups(self, cell_data):
         """compare_cells' grouping: K = encoding_size classes, a cell's class the argmax of its

@@ -2286,6 +2286,115 @@ class BiGanEngine:
                                     round=True, ws=ws)
         return sums, sumsq, nonzero
 
+    def features_stream(self, *, csr=None, order=None, z32=None, r32=None,
+                        tile_rows=GENERATE_TILE):
+        """log1p features of real or generated cells -> device tensors
+            features       [n, gene_size] bf16  view of a [n, pad_ld(gene_size)] buffer whose
+                                                padding columns are zero (a GEMM operand)
+            library_size   [n] fp64             sum over genes of v
+            genes_detected [n] int32            #{genes : v != 0}
+        with features = bf16(float(log1p(double(v)))) (cc_log1p_features).  The two modes of
+        moments_stream: real cells are the rows `order` (host or device int64) of the device CSR
+        `csr`, gathered tile by tile with cc_gather_rows(row_idx=...), v the exact fp32 count;
+        generated cells are the rows of z32 / r32 ([n, Z] fp32), v = rint(G.predict(z, r)),
+        tiled from row 0 like G.predict, so they are generate_cells' cells bit for bit.
+        Device memory: one fp32 tile and the outputs.  Engine state is not touched and no
+        collective is issued."""
+        dev = self.device
+        if dev.type != "cuda":
+            raise RuntimeError("features_stream needs a CUDA device (no host fallback)")
+        if (csr is None) == (z32 is None):
+            raise ValueError("features_stream: give either csr and order (real cells) or z32 "
+                             "and r32 (generated cells)")
+        if csr is not None:
+            order = torch.as_tensor(order, dtype=torch.int64).to(dev)
+            if order.dim() != 1:
+                raise ValueError("features_stream: order must be a vector of row numbers")
+            n = order.numel()
+        else:
+            z32 = torch.as_tensor(z32, dtype=torch.float32).to(dev)
+            r32 = torch.as_tensor(r32, dtype=torch.float32).to(dev)
+            n = z32.shape[0]
+            if z32.dim() != 2 or tuple(z32.shape) != (n, self.Z) or tuple(r32.shape) != (n, self.Z):
+                raise ValueError(f"features_stream: z32 / r32 must both be [n, {self.Z}]")
+        tile_rows = int(tile_rows)
+        if tile_rows < 1:
+            raise ValueError("features_stream: tile_rows must be >= 1")
+        Gn = self.Gn
+        feats = ops.alloc2d(n, Gn, dtype=torch.bfloat16, device=dev, zero=False)
+        lib = torch.zeros(n, dtype=torch.float64, device=dev)
+        det = torch.zeros(n, dtype=torch.int32, device=dev)
+        if n == 0:
+            return feats, lib, det
+        T = max(1, min(tile_rows, n))
+        tile = ops.alloc2d(T, Gn, dtype=torch.float32, device=dev, zero=False)
+        for s in range(0, n, T):
+            m = min(T, n - s)
+            if csr is not None:
+                rowptr, colidx, values = csr
+                ops.gather_rows(rowptr, colidx, values, Gn, row_idx=order[s:s + m],
+                                out32=tile[:m])
+            else:
+                self.set_latents(z32[s:s + m], r32[s:s + m], m)
+                self.generate(m, out32=tile[:m])
+            ops.log1p_features(tile[:m], feats[s:s + m], lib[s:s + m], det[s:s + m],
+                               round=csr is None)
+        return feats, lib, det
+
+    MEDIAN_ROWS = 1024        # rows of d^2 formed at a time for the median
+
+    def mmd_sums(self, fx, fy, scales, masks):
+        """Kernel sums of an MMD permutation test on two device feature blocks fx, fy ([n, K]
+        bf16, rows of features_stream) -> (median, sums):
+            median  the lower median of d2_ij = max((G_ii + G_jj) - 2 G_ij, 0), i < j, over the
+                    pooled cells (fx rows first), G their fp32 Gram matrix
+            sums    host fp64 [L, len(scales), 3]: XX, YY, XY of k = exp(-d2 / (s * median)) per
+                    labelling (cc_mmd_sums; XX, YY, XY as in mmd_from_sums)
+        masks: uint32 [L, ceil(2n / 32)] (host), bit i = pooled cell i is in X.  The Gram
+        matrix is three cc_gemm calls (XX, XY and YY quadrants; the YX quadrant is never read),
+        the median a torch kthvalue over the upper triangle formed with the kernel's fp32
+        expression.  Device memory: the [2n, 2n] fp32 Gram matrix, the upper triangle of d2 and
+        the workspace; nothing of size (n, genes) in fp32.  Rank-local, no collective.
+        A zero median (most pairs identical) gives median 0 and NaN sums."""
+        import numpy as np
+        dev = self.device
+        n, K = fx.shape
+        if tuple(fy.shape) != (n, K):
+            raise ValueError("mmd_sums: fx and fy must have the same shape")
+        N = 2 * n
+        masks = np.ascontiguousarray(masks, dtype=np.uint32)
+        L = masks.shape[0]
+        if masks.ndim != 2 or masks.shape[1] != (N + 31) // 32:
+            raise ValueError(f"mmd_sums: masks must be [L, {(N + 31) // 32}]")
+        if not 1 <= len(scales) <= 4:
+            raise ValueError("mmd_sums: 1 to 4 bandwidth scales")
+        if n < 1:
+            raise ValueError("mmd_sums: needs at least one cell per block")
+        G = ops.alloc2d(N, N, dtype=torch.float32, device=dev, zero=False)
+        ops.gemm(n, n, [fx], [fx], [K], 0, 0, out32=G[:n, :n])
+        ops.gemm(n, n, [fx], [fy], [K], 0, 0, out32=G[:n, n:])
+        ops.gemm(n, n, [fy], [fy], [K], 0, 0, out32=G[n:, n:])
+        diag = torch.diagonal(G).clone()
+        upper = []
+        cols = torch.arange(N, device=dev)
+        for s in range(0, N - 1, self.MEDIAN_ROWS):
+            e = min(N - 1, s + self.MEDIAN_ROWS)
+            d2 = torch.clamp_min((diag[s:e, None] + diag[None, :]) - 2.0 * G[s:e], 0.0)
+            upper.append(d2[cols[None, :] > torch.arange(s, e, device=dev)[:, None]])
+            del d2
+        upper = torch.cat(upper)
+        m = upper.numel()
+        median = float(torch.kthvalue(upper, (m - 1) // 2 + 1).values) if m else float("nan")
+        del upper
+        out = np.full((L, len(scales), 3), np.nan)
+        if not median > 0:
+            return median, out
+        inv = [1.0 / (float(s) * median) for s in scales]
+        sums = torch.empty((L, len(scales), 3), dtype=torch.float64, device=dev)
+        ws = torch.empty(ops.mmd_sums_ws_bytes(N, len(scales), L), dtype=torch.uint8, device=dev)
+        ops.mmd_sums(G, inv, torch.from_numpy(masks.view(np.int32)).to(dev), sums, ws=ws)
+        return median, sums.cpu().numpy()
+
     def discriminate(self, z16, x16, out32):
         """D.predict -> probabilities (fp32 [rows,1])."""
         return self.D.forward({"z": z16, "cell": x16}, x16.shape[0], bn_train=False, dropout="off",

@@ -526,6 +526,58 @@ def col_moments(x32, sum64, sumsq64, nonzero64, *, round=False, ws):
                                      _p(ws), 0 if ws is None else ws.numel(), _stream()))
 
 
+def log1p_features(x32, f16, library_size, genes_detected, *, round=False):
+    """f16[r, c] = bf16(float(log1p(double(v)))), library_size[r] = sum_c v (fp64) and
+    genes_detected[r] = #{c : v != 0} (int32) for the rows of a dense fp32 tile, v = x32[r, c]
+    or rint(x32[r, c]) with round=True (cc_log1p_features).  f16 is [rows, cols] bf16 whose
+    leading dimension is at least cols rounded up to 64; those padding columns are zeroed."""
+    _req(x32, torch.float32, "x32")
+    _req(f16, torch.bfloat16, "f16")
+    _req(library_size, torch.float64, "library_size")
+    _req(genes_detected, torch.int32, "genes_detected")
+    if x32.dim() != 2 or tuple(f16.shape) != tuple(x32.shape):
+        raise ValueError("log1p_features: x32 and f16 must both be [rows, cols]")
+    rows = x32.shape[0]
+    for t in (library_size, genes_detected):
+        if t.numel() != rows or not t.is_contiguous():
+            raise ValueError(f"log1p_features: the row outputs must hold {rows} contiguous values")
+    check(_lib.load().cc_log1p_features(_p(x32), _ld(x32), rows, x32.shape[1], int(bool(round)),
+                                        _p(f16), _ld(f16), library_size.data_ptr(),
+                                        genes_detected.data_ptr(), _stream()))
+
+
+def mmd_sums_ws_bytes(n_cells, n_bandwidths, labellings):
+    """Bytes of an mmd_sums workspace for n_cells cells, n_bandwidths and labellings."""
+    return int(_lib.load().cc_mmd_sums_ws_bytes(int(n_cells), int(n_bandwidths),
+                                                int(labellings)))
+
+
+def mmd_sums(gram32, inv_bandwidths, masks, out64, *, ws):
+    """XX, YY, XY kernel sums of every labelling and bandwidth (cc_mmd_sums): gram32 [N, N] fp32
+    (only i <= j is read), inv_bandwidths 1 to 4 host floats, masks int32 [L, ceil(N / 32)]
+    (the bits of uint32 words), out64 fp64 [L, len(inv_bandwidths), 3].  ws: a uint8 buffer of
+    at least mmd_sums_ws_bytes bytes."""
+    _req(gram32, torch.float32, "gram32")
+    _req(masks, torch.int32, "masks")
+    _req(out64, torch.float64, "out64")
+    _req(ws, torch.uint8, "ws")
+    N = gram32.shape[0]
+    if gram32.dim() != 2 or gram32.shape[1] != N:
+        raise ValueError("mmd_sums: gram32 must be [N, N]")
+    g = [float(v) for v in inv_bandwidths]
+    L = masks.shape[0]
+    if masks.dim() != 2 or masks.shape[1] != (N + 31) // 32 or not masks.is_contiguous():
+        raise ValueError(f"mmd_sums: masks must be contiguous [L, {(N + 31) // 32}]")
+    if tuple(out64.shape) != (L, len(g), 3) or not out64.is_contiguous():
+        raise ValueError(f"mmd_sums: out64 must be contiguous [{L}, {len(g)}, 3]")
+    if ws is not None and not ws.is_contiguous():
+        raise ValueError("mmd_sums: ws must be contiguous")
+    arr = (C.c_float * max(1, len(g)))(*g)
+    check(_lib.load().cc_mmd_sums(_p(gram32), _ld(gram32), N, C.cast(arr, C.c_void_p), len(g),
+                                  _p(masks), L, out64.data_ptr(), _p(ws),
+                                  0 if ws is None else ws.numel(), _stream()))
+
+
 def argmax_onehot(p32, out16=None, out32=None):
     _req(p32, torch.float32, "p32")
     check(_lib.load().cc_argmax_onehot(_p(p32), _ld(p32), _p(out16), _ld(out16), _p(out32),

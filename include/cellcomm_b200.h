@@ -452,6 +452,38 @@ int cc_col_moments(const float* x, int64_t ld, int64_t rows, int64_t cols,
                    int32_t round_half_even, double* sum, double* sumsq, int64_t* nonzero,
                    void* ws, int64_t ws_bytes, cc_stream_t stream);
 int64_t cc_col_moments_ws_bytes(int64_t rows, int64_t cols);
+/* log1p features for the two-sample pass (csrc/twosample.cu).  For every row r of the fp32 tile
+ * x ([rows, ldx]) and column c < cols, with v = x[r, c] or rint(x[r, c]) (round half to even)
+ * when round_half_even != 0:
+ *   features[r, c] = bf16_rn(float(log1p(double(v))))   (bf16, row-major, leading dim ldf)
+ *   library_size[r] = sum_c v (fp64),  genes_detected[r] = #{c : v != 0}
+ * Columns [cols, round_up(cols, 64)) of the features are written as zero, so the output is a
+ * GEMM operand as it stands; ldf must be a multiple of 8 and at least round_up(cols, 64), and
+ * features 16-byte aligned.  Nothing at or past `cols` of x is read.  -0.0 gives -0.0 and is
+ * not detected; a NaN gives a quiet NaN with its sign.  The row sums combine in a fixed order,
+ * so identical inputs give identical bits, and integer counts give exact sums.  rows == 0 is a
+ * no-op. */
+int cc_log1p_features(const float* x, int64_t ldx, int64_t rows, int64_t cols,
+                      int32_t round_half_even, void* features, int64_t ldf,
+                      double* library_size, int32_t* genes_detected, cc_stream_t stream);
+/* Kernel sums of an MMD permutation test (csrc/twosample.cu).  gram is the fp32 Gram matrix
+ * [n_cells, ldg] of the pooled cells (only elements G[i][j] with i <= j are read: the upper
+ * triangle and the diagonal), inv_bandwidths (host) holds 1 to 4 values g_b, and masks
+ * (uint32 [labellings, ceil(n_cells / 32)], bit i % 32 of word i / 32 set = cell i is in X) one
+ * labelling per row.  With d2 = max((G[i][i] + G[j][j]) - 2 G[i][j], 0) in fp32 (no FMA
+ * contraction) and k_b = expf(-(d2 g_b)), it writes for every labelling p and bandwidth b
+ *   sums[(p * n_bandwidths + b) * 3 + {0, 1, 2}] = XX, YY, XY      (fp64)
+ * the sums of k_b over ordered pairs i != j with both cells in X, both in Y, and i in X, j in Y.
+ * ldg must be a multiple of 4 and gram 16-byte aligned.  Per-thread partials are fp32 over 32
+ * terms, everything above them fp64 in a fixed order (a grid that depends on n_cells alone, no
+ * float atomics), so identical inputs give identical bits on any GPU.  Workspace contract: ws
+ * holds ws_bytes bytes, 8-byte aligned, at least cc_mmd_sums_ws_bytes(n_cells, n_bandwidths,
+ * labellings); a smaller one fails (cc_last_error).  It needs no zeroing.  One workspace per
+ * stream.  n_cells < 2 writes zeros; labellings == 0 is a no-op. */
+int cc_mmd_sums(const float* gram, int64_t ldg, int64_t n_cells, const float* inv_bandwidths,
+                int32_t n_bandwidths, const uint32_t* masks, int64_t labellings, double* sums,
+                void* ws, int64_t ws_bytes, cc_stream_t stream);
+int64_t cc_mmd_sums_ws_bytes(int64_t n_cells, int32_t n_bandwidths, int64_t labellings);
 /* to_categorical(argmax(p,-1)): src/bigan_classify.py:121-124 */
 int cc_argmax_onehot(const float* p32, int64_t ldp, void* out16, int64_t ldo, float* out32,
                      int64_t ldo32, int64_t rows, int64_t cols, cc_stream_t stream);
