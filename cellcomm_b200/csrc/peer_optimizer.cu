@@ -187,24 +187,43 @@ __global__ void peer_wait_kernel(const uint32_t* flags, const int n, const uint3
 
 using namespace cc;
 
+// the kernel moves 8 elements per thread as 16-byte vectors (fp32 float4 pairs, one bf16 uint4)
+static bool vec16_at(const void* base, long long start, int elem_bytes) {
+  return base == nullptr || (((uintptr_t)base + (uintptr_t)(start * elem_bytes)) & 15) == 0;
+}
+
 extern "C" int cc_peer_rmsprop(const cc_peer_rmsprop_desc* d, cc_stream_t stream) {
   CC_REQUIRE(d != nullptr, "cc_peer_rmsprop: null descriptor");
   CC_REQUIRE(d->world >= 1 && d->world <= CC_PEER_MAX, "cc_peer_rmsprop: world=%d", d->world);
-  CC_REQUIRE(d->count >= 0 && (d->count & 7) == 0 && (d->start & 3) == 0,
+  CC_REQUIRE(d->rank >= 0 && d->rank < d->world, "cc_peer_rmsprop: rank=%d of world=%d", d->rank,
+             d->world);
+  CC_REQUIRE(d->count >= 0 && (d->count & 7) == 0 && (d->start & 7) == 0,
              "cc_peer_rmsprop: range [%lld, +%lld) must be 8-element granular",
              (long long)d->start, (long long)d->count);
   if (d->count == 0) return 0;
+  const long long st = d->start;
+  CC_REQUIRE(d->p32 && d->ms && d->mom && d->ready, "cc_peer_rmsprop: null p32/ms/mom/ready");
+  CC_REQUIRE(vec16_at(d->p32, st, 4) && vec16_at(d->ms, st, 4) && vec16_at(d->mom, st, 4),
+             "cc_peer_rmsprop: p32/ms/mom must be 16-byte aligned at start=%lld", st);
+  CC_REQUIRE(vec16_at(d->p16_multicast, st, 2) && vec16_at(d->p16lo_multicast, st, 2),
+             "cc_peer_rmsprop: multicast pointers must be 16-byte aligned at start=%lld", st);
+  const bool has_lo = d->p16lo[0] != nullptr;
   PeerPtrs pp;
   for (int q = 0; q < CC_PEER_MAX; ++q) {
     pp.g[q] = q < d->world ? d->grad[q] : nullptr;
     pp.p16[q] = q < d->world ? (bf16*)d->p16[q] : nullptr;
-    CC_REQUIRE(q >= d->world || (pp.g[q] != nullptr && pp.p16[q] != nullptr),
+    CC_REQUIRE(q >= d->world || (pp.g[q] != nullptr && pp.p16[q] != nullptr &&
+                                 (!has_lo || d->p16lo[q] != nullptr)),
                "cc_peer_rmsprop: missing peer pointer %d", q);
+    CC_REQUIRE(q >= d->world || (vec16_at(pp.g[q], st, 4) && vec16_at(pp.p16[q], st, 2) &&
+                                 vec16_at(d->p16lo[q], st, 2)),
+               "cc_peer_rmsprop: grad/p16/p16lo of rank %d must be 16-byte aligned at start=%lld",
+               q, st);
   }
   if (!d->broadcast) pp.p16[0] = (bf16*)d->p16[d->rank];
   PeerLo lo;
   for (int q = 0; q < CC_PEER_MAX; ++q) lo.p16lo[q] = q < d->world ? (bf16*)d->p16lo[q] : nullptr;
-  if (lo.p16lo[0] != nullptr && !d->broadcast) lo.p16lo[0] = (bf16*)d->p16lo[d->rank];
+  if (has_lo && !d->broadcast) lo.p16lo[0] = (bf16*)d->p16lo[d->rank];
   lo.mc = (bf16*)d->p16lo_multicast;
   for (int k = 0; k < 2; ++k) {
     lo.begin[k] = d->lo_begin[k];

@@ -617,6 +617,8 @@ def peer_rmsprop(world, rank, grad_ptrs, p16_ptrs, p32, ms, mom, start, count, b
     for t, name in ((p32, "p32"), (ms, "ms"), (mom, "mom")):
         _req(t, torch.float32, name)
     d = _lib.PeerRmspropDesc()
+    if not 0 <= world <= len(d.grad):
+        raise ValueError(f"peer_rmsprop: world={world} (at most {len(d.grad)} ranks)")
     d.world, d.rank = int(world), int(rank)
     for q in range(world):
         d.grad[q], d.p16[q] = int(grad_ptrs[q]), int(p16_ptrs[q])

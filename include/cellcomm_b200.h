@@ -503,8 +503,11 @@ int cc_rmsprop_step(float* p32, void* p16, const float* g, float* ms, float* mom
  * library only sees device pointers).  cc_peer_rmsprop fuses
  *     reduce-scatter (P2P loads) -> Keras RMSprop on this rank's shard -> all-gather of the
  *     bf16 weights (P2P stores)
- * for the element range [start, start+count) of the flat buffers.  The reference has no
- * counterpart (single process); under data parallelism this is the gradient exchange around
+ * for the element range [start, start+count) of the flat buffers.  start and count are
+ * multiples of 8, 0 <= rank < world, and every fp32 / bf16 buffer (grad, p16, p16lo, p32, ms,
+ * mom and the multicast addresses) is 16-byte aligned at `start`: the kernel moves 8 elements
+ * per thread in 16-byte vectors.  Anything else is rejected before the launch.  The reference
+ * has no counterpart (single process); under data parallelism this is the gradient exchange around
  * `optimizer.apply_gradients` of src/bigan_classify.py:88,144-155.
  *   grad[q], p16[q] : rank q's buffers (q < world), the same flat layout on every rank
  *   broadcast = 1   : sharded update, bf16 result stored to all ranks;
