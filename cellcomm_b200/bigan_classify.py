@@ -245,21 +245,10 @@ class ClassifyCellBiGan(BasicBiGan):
         lo, hi = min(N, r * per), min(N, (r + 1) * per)
         piece = torch.zeros((per, Z), dtype=torch.float32, device=eng.device)
         if hi > lo:
-            self._encode_rows(mat, lo, hi, piece[:hi - lo])
+            eng.encode_stream(*mat.device_csr(eng.device), lo, hi, piece[:hi - lo])
         full = torch.empty((W * per, Z), dtype=torch.float32, device=eng.device)
         eng.dist.all_gather(full.view(-1), piece.view(-1))
         return full[:N].cpu().numpy()
-
-    def _encode_rows(self, mat, lo, hi, out):
-        """E.predict on rows [lo, hi) of a device-resident CellMatrix -> out (fp32, device)."""
-        eng = self._engine
-        if eng.device.type == "cuda" and os.environ.get("CELLCOMM_B200_ENCODE_STREAM", "1") != "0":
-            rowptr, colidx, values = mat.device_csr(eng.device)
-            eng.encode_stream(rowptr, colidx, values, lo, hi, out)
-            return
-        for s in range(lo, hi, self.PREDICT_TILE):
-            m = min(self.PREDICT_TILE, hi - s)
-            eng.encode(self._stage_cells(mat, s, m), out32=out[s - lo:s - lo + m])
 
     # ------------------------------------------------------------------ checkpoint / resume
     def save_checkpoint(self, path, extra=None):
@@ -294,7 +283,7 @@ class ClassifyCellBiGan(BasicBiGan):
                                "CUDA engine is unavailable and there is no host fallback")
         return self._engine
 
-    def _stage_cells(self, cells, row_start=0, rows=None):
+    def _stage_cells(self, cells):
         """[n, gene_size] bf16 device tile for `cells`: a CellBatch / CellMatrix is gathered
         from the device-resident CSR (cc_gather_rows); anything array-like (DataFrame, ndarray,
         list, torch tensor) is uploaded as float32 and cast on the device."""
@@ -305,16 +294,13 @@ class ClassifyCellBiGan(BasicBiGan):
         if isinstance(cells, (CellBatch, CellMatrix)):
             mat = cells.matrix if isinstance(cells, CellBatch) else cells
             rowptr, colidx, values = mat.device_csr(dev)
+            out = self._tile(len(cells))
             if isinstance(cells, CellBatch):
-                n = len(cells)
                 idx = torch.from_numpy(cells.positions).to(dev, non_blocking=True)
-                out = self._tile(n)
                 ops.gather_rows(rowptr, colidx, values, mat.shape[1], row_idx=idx, out16=out)
             else:
-                n = len(mat) - row_start if rows is None else rows
-                out = self._tile(n)
-                ops.gather_rows(rowptr, colidx, values, mat.shape[1], row_start=row_start,
-                                n_rows=n, out16=out)
+                ops.gather_rows(rowptr, colidx, values, mat.shape[1], n_rows=len(mat),
+                                out16=out)
             return out
         if isinstance(cells, torch.Tensor):
             t = cells
@@ -322,8 +308,6 @@ class ClassifyCellBiGan(BasicBiGan):
             arr = cells.values if hasattr(cells, "values") and not isinstance(cells, np.ndarray) \
                 else cells
             t = torch.as_tensor(np.ascontiguousarray(np.asarray(arr, dtype=np.float32)))
-        if rows is not None:
-            t = t[row_start:row_start + rows]
         t = t.to(dev, dtype=torch.float32, non_blocking=True)
         if t.dim() != 2 or t.shape[1] != self.gene_size:
             raise ValueError(f"expected cells of shape (n, {self.gene_size}), got {tuple(t.shape)}")
@@ -338,13 +322,12 @@ class ClassifyCellBiGan(BasicBiGan):
             setattr(self, name, buf)
         return buf[:n]
 
-    PREDICT_TILE = 4096
-
     def _predict(self, role, x):
-        """Model.predict for G / E / D in inference mode -> float32 host array."""
+        """Model.predict for G / E / D in inference mode -> float32 host array, in the engine's
+        PREDICT_TILE-row tiles."""
         import torch
         eng = self._require_engine()
-        dev = eng.device
+        dev, T = eng.device, eng.PREDICT_TILE
         if role == "E":
             if isinstance(x, CellMatrix):
                 # the encode-all-cells pass (src/intercepts/db_recorder.py:85)
@@ -352,31 +335,33 @@ class ClassifyCellBiGan(BasicBiGan):
                     self._announce("encode_all")
                     return self._encode_all_sharded(x)
                 out = torch.empty((len(x), self.encoding_size), dtype=torch.float32, device=dev)
-                self._encode_rows(x, 0, len(x), out)
+                eng.encode_stream(*x.device_csr(dev), 0, len(x), out)
                 return out.cpu().numpy()
             n = len(x)
             out = torch.empty((n, self.encoding_size), dtype=torch.float32, device=dev)
-            for s in range(0, n, self.PREDICT_TILE):
-                m = min(self.PREDICT_TILE, n - s)
+            for s in range(0, n, T):
+                m = min(T, n - s)
                 eng.encode(self._stage_cells(_rows(x, s, s + m)), out32=out[s:s + m])
             return out.cpu().numpy()
         enc, second = x
         z = torch.as_tensor(np.asarray(enc, dtype=np.float32)).to(dev)
         n = z.shape[0]
         if role == "G":
-            r = torch.as_tensor(np.asarray(second, dtype=np.float32)).to(dev)
+            z, r = eng._latents("G.predict", z, np.asarray(second, dtype=np.float32))
             out = torch.empty((n, self.gene_size), dtype=torch.float32, device=dev)
-            for s in range(0, n, self.PREDICT_TILE):
-                m = min(self.PREDICT_TILE, n - s)
-                eng.set_latents(z[s:s + m], r[s:s + m], m)
-                eng.generate(m, out32=out[s:s + m])
+            for _ in eng._generated_tiles(z, r, T, out):
+                pass
             return out.cpu().numpy()
         out = torch.empty((n, 1), dtype=torch.float32, device=dev)
-        for s in range(0, n, self.PREDICT_TILE):
-            m = min(self.PREDICT_TILE, n - s)
-            tile = self._stage_cells(second, s, m) if isinstance(second, CellMatrix) \
-                else self._stage_cells(_rows(second, s, s + m))
-            eng.discriminate(z[s:s + m].contiguous(), tile, out[s:s + m])
+        if n == 0:
+            return out.cpu().numpy()
+        if isinstance(second, CellMatrix):
+            cells = eng._real_tiles(second.device_csr(dev), (0, n), self._tile(min(T, n)))
+        else:
+            cells = ((s, min(T, n - s), self._stage_cells(_rows(second, s, s + T)))
+                     for s in range(0, n, T))
+        for s, m, x16 in cells:
+            eng.discriminate(z[s:s + m].contiguous(), x16, out[s:s + m])
         return out.cpu().numpy()
 
     def generate_cell_matrix(self, encoding_in, random_in=None, columns=None):
@@ -400,7 +385,7 @@ class ClassifyCellBiGan(BasicBiGan):
             random_in = self.random_uniform_vector(len(encoding_in))
         enc = np.asarray(encoding_in, dtype=np.float32)
         rowptr, colidx, values = self._engine.generate_csr(
-            enc, np.asarray(random_in, dtype=np.float32), self.PREDICT_TILE)
+            enc, np.asarray(random_in, dtype=np.float32))
         return CellMatrix(rowptr, colidx, values, np.arange(1, len(enc) + 1), columns)
 
     def score_cells(self, cell_data, random_in=None):
@@ -429,7 +414,7 @@ class ClassifyCellBiGan(BasicBiGan):
         d_real = torch.empty(n, dtype=torch.float32, device=dev)
         rowptr, colidx, values = mat.device_csr(dev)
         eng.score_stream(rowptr, colidx, values, 0, n, np.asarray(random_in, dtype=np.float32),
-                         enc, mse, d_real, self.PREDICT_TILE)
+                         enc, mse, d_real)
         return CellScores(enc.cpu().numpy(), mse.cpu().numpy(), d_real.cpu().numpy())
 
     def gene_statistics(self, cell_data, groups=None, n_groups=None):
@@ -450,7 +435,7 @@ class ClassifyCellBiGan(BasicBiGan):
         bounds = np.concatenate([[0], np.cumsum(counts)])
         order = np.argsort(labels, kind="stable").astype(np.int64)
         sums = self._engine.moments_stream(bounds, csr=mat.device_csr(self._engine.device),
-                                           order=order, tile_rows=self.PREDICT_TILE)
+                                           order=order)
         return statistics_from_sums(counts, *(t.cpu().numpy() for t in sums))
 
     def generated_gene_statistics(self, encoding_in, random_in=None, groups=None,
@@ -470,8 +455,7 @@ class ClassifyCellBiGan(BasicBiGan):
         counts = np.bincount(labels, minlength=K)
         bounds = np.concatenate([[0], np.cumsum(counts)])
         sums = self._engine.moments_stream(bounds, z32=enc,
-                                           r32=np.asarray(random_in, dtype=np.float32),
-                                           tile_rows=self.PREDICT_TILE)
+                                           r32=np.asarray(random_in, dtype=np.float32))
         return statistics_from_sums(counts, *(t.cpu().numpy() for t in sums))
 
     def two_sample_test(self, cell_data, max_cells=4096, permutations=1000, seed=0):
@@ -497,16 +481,14 @@ class ClassifyCellBiGan(BasicBiGan):
         encodings = np.asarray(self._comparison_encodings(counts), dtype=np.float32)
         noise = self.random_uniform_vector(len(encodings))
         eng = self._engine
-        gen_f, gen_lib, gen_det = eng.features_stream(z32=encodings, r32=noise,
-                                                      tile_rows=self.PREDICT_TILE)
+        gen_f, gen_lib, gen_det = eng.features_stream(z32=encodings, r32=noise)
         gen_lib, gen_det = gen_lib.cpu().numpy(), gen_det.cpu().numpy()
         csr = mat.device_csr(eng.device)
         medians, sums, lib, det = [], [], [], []
         off = 0
         for k in range(K):
             n = counts[k]
-            fx, x_lib, x_det = eng.features_stream(csr=csr, order=picks[k],
-                                                   tile_rows=self.PREDICT_TILE)
+            fx, x_lib, x_det = eng.features_stream(csr=csr, order=picks[k])
             lib.append((x_lib.cpu().numpy(), gen_lib[off:off + n]))
             det.append((x_det.cpu().numpy(), gen_det[off:off + n]))
             if n < 2:

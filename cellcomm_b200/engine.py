@@ -1917,19 +1917,89 @@ class BiGanEngine:
         return gs
 
     # ------------------------------------------------------------------ inference
+    PREDICT_TILE = 4096       # rows per tile of every pass over cells (see _generated_tiles)
+
+    def _tiling(self, name, tile_rows, cuda=True):
+        """Rows per tile of the pass `name`: tile_rows, or PREDICT_TILE when None."""
+        if cuda and self.device.type != "cuda":
+            raise RuntimeError(f"{name} needs a CUDA device (no host fallback)")
+        tile_rows = self.PREDICT_TILE if tile_rows is None else int(tile_rows)
+        if tile_rows < 1:
+            raise ValueError(f"{name}: tile_rows must be >= 1")
+        return tile_rows
+
+    def _latents(self, name, z32, r32, n=None):
+        """z32 / r32 ([n, Z] fp32, host or device; n = z32's rows when None) on the device."""
+        z32 = torch.as_tensor(z32, dtype=torch.float32).to(self.device)
+        r32 = torch.as_tensor(r32, dtype=torch.float32).to(self.device)
+        n = z32.shape[0] if n is None else n
+        if tuple(z32.shape) != (n, self.Z) or tuple(r32.shape) != (n, self.Z):
+            raise ValueError(f"{name}: z32 / r32 must both be [{n}, {self.Z}]")
+        return z32, r32
+
+    def _cells(self, name, csr, order, z32, r32, n=None):
+        """The cells of a pass over real or generated ones: the rows `order` (host or device
+        int64) of the device CSR `csr`, or the generator's output for z32 / r32.  Exactly one
+        of the two must be given, with n cells when n is given -> (n, order, z32, r32), the
+        given pair on the device and the other None."""
+        if (csr is None) == (z32 is None):
+            raise ValueError(f"{name}: give either csr and order (real cells) or z32 and r32 "
+                             "(generated cells)")
+        if csr is None:
+            z32, r32 = self._latents(name, z32, r32, n)
+            return z32.shape[0], None, z32, r32
+        order = torch.as_tensor(order, dtype=torch.int64).to(self.device)
+        if order.dim() != 1 or n not in (None, order.numel()):
+            raise ValueError(f"{name}: order must be a vector of row numbers"
+                             + ("" if n is None else f", {n} of them"))
+        return order.numel(), order, None, None
+
+    def _generated_tiles(self, z32, r32, tile_rows, out):
+        """Generated cells tile by tile: for rows [s, s + m) of z32 / r32 ([n, Z] fp32 on the
+        device), from row 0 in tiles of tile_rows rows, set_latents + generate() into
+        x = out[s:s + m] when out ([n, gene_size] fp32) holds every row, else into x = out[:m]
+        of one fp32 tile buffer; yields (s, m, x).
+
+        This is G.predict's tiling, and the only one that reproduces generate_cells bit for
+        bit: the generator's GEMMs choose their split-K from the row count.  Every pass over
+        generated cells takes its tiles from here."""
+        n = z32.shape[0]
+        for s in range(0, n, tile_rows):
+            m = min(tile_rows, n - s)
+            x = out[s:s + m] if out.shape[0] == n else out[:m]
+            self.set_latents(z32[s:s + m], r32[s:s + m], m)
+            self.generate(m, out32=x)
+            yield s, m, x
+
+    def _real_tiles(self, csr, rows, tile):
+        """Real cells tile by tile: for cells [s, s + m) of `rows` of the device CSR
+        csr = (rowptr, colidx, values) with gene_size columns, in tiles of tile's rows,
+        cc_gather_rows into x = tile[:m] (bf16 or fp32); yields (s, m, x).  rows: a row range
+        (row_begin, row_end), gathered by row_start / n_rows, or an int64 device vector of row
+        numbers, gathered by row_idx."""
+        T, key = tile.shape[0], "out16" if tile.dtype == ops.COMPUTE_DTYPE else "out32"
+        ranged = isinstance(rows, tuple)
+        n = rows[1] - rows[0] if ranged else rows.numel()
+        for s in range(0, n, T):
+            m = min(T, n - s)
+            x = tile[:m]
+            if ranged:
+                ops.gather_rows(*csr, self.Gn, row_start=rows[0] + s, n_rows=m, **{key: x})
+            else:
+                ops.gather_rows(*csr, self.Gn, row_idx=rows[s:s + m], **{key: x})
+            yield s, m, x
+
     def encode(self, x16, out32=None):
         """E.predict on a [rows, gene_size] bf16 tile; fp32 result in out32 when given."""
         return self.E.forward({"cell": x16}, x16.shape[0], bn_train=False, dropout="off",
                               out32=out32)
-
-    ENCODE_TILE = 4096
 
     def encode_plan(self, tile_rows=None):
         """cc_encode_plan for this engine's encoder: the op list Net.forward(bn_train=False,
         dropout="off") would launch for one tile (same kernels, same precision policy), over
         scratch slots.  None when a layer has width 0 (the 5-gene fixture's Dense(0))."""
         from . import _lib
-        tile_rows = int(tile_rows or self.ENCODE_TILE)
+        tile_rows = int(tile_rows or self.PREDICT_TILE)
         cached = getattr(self, "_enc_plan", None)
         if cached is not None and cached[0] == tile_rows:
             return cached[1]
@@ -2032,35 +2102,30 @@ class BiGanEngine:
     def encode_stream(self, rowptr, colidx, values, row_begin, row_end, out32, tile_rows=None):
         """encoding_prediction for rows [row_begin, row_end) of a device CSR in ONE C call
         (cc_encode_stream): gather + encoder forward per tile, no Python between tiles.  Falls
-        back to the tile loop over encode() for encoders the plan cannot express."""
+        back to the tile loop over encode() off CUDA and for encoders the plan cannot express."""
         self.E._wait_optimizer()
-        plan = self.encode_plan(tile_rows)
-        if plan is None:
-            tile = int(tile_rows or self.ENCODE_TILE)
-            buf = ops.alloc2d(min(tile, max(1, row_end - row_begin)), self.Gn, device=self.device)
-            for s in range(row_begin, row_end, tile):
-                m = min(tile, row_end - s)
-                ops.gather_rows(rowptr, colidx, values, self.Gn, row_start=s, n_rows=m,
-                                out16=buf[:m])
-                self.encode(buf[:m], out32=out32[s - row_begin:s - row_begin + m])
+        tile_rows = self._tiling("encode_stream", tile_rows, cuda=False)
+        plan = self.encode_plan(tile_rows) if self.device.type == "cuda" else None
+        if plan is not None:
+            ops.encode_stream(rowptr, colidx, values, row_begin, row_end, plan, out32)
             return
-        ops.encode_stream(rowptr, colidx, values, row_begin, row_end, plan, out32)
+        tile = ops.alloc2d(min(tile_rows, max(1, row_end - row_begin)), self.Gn,
+                           device=self.device)
+        for s, m, x in self._real_tiles((rowptr, colidx, values), (row_begin, row_end), tile):
+            self.encode(x, out32=out32[s:s + m])
 
     def generate(self, rows, out32=None):
         """G.predict on the staged latents (first `rows`)."""
         return self.G.forward({"z": self.z32[:rows], "r": self.r32[:rows]}, rows, bn_train=False,
                               dropout="off", out32=out32)
 
-    GENERATE_TILE = 4096      # = ClassifyCellBiGan.PREDICT_TILE: split-K depends on M, so the
-                              # streamed pass must tile exactly like G.predict to match its bits
-
-    def generate_csr(self, z32, r32, tile_rows=GENERATE_TILE, consume=None):
+    def generate_csr(self, z32, r32, tile_rows=None, consume=None):
         """rint(G.predict(z, r)) for every row of z32 / r32 ([n, Z] fp32, host or device) as a
-        CSR, without ever holding the dense (n, genes) output.  Per tile of `tile_rows` rows
-        (from row 0, like G.predict): the generator forward (the kernels generate() runs) into
-        one fp32 tile, cc_round_csr_count, a read-back of the tile's nnz, cc_round_csr_fill,
-        and cudaMemcpyAsync of the entries into pinned host staging on a side stream, so that
-        the copy of tile i overlaps the forward of tile i+1 (two staging sets, events).
+        CSR, without ever holding the dense (n, genes) output.  Per generated tile
+        (_generated_tiles, into one fp32 tile): cc_round_csr_count, a read-back of the tile's
+        nnz, cc_round_csr_fill, and cudaMemcpyAsync of the entries into pinned host staging on
+        a side stream, so that the copy of tile i overlaps the forward of tile i+1 (two staging
+        sets, events).
         Device memory: the fp32 tile plus the largest tile's entries.
 
         Engine state (weights, BN statistics, RNG counter, loss_buf) is not touched; like
@@ -2073,16 +2138,9 @@ class BiGanEngine:
         (rowptr int64 [n + 1], colidx int32 [nnz], values float32 [nnz]) as numpy arrays."""
         import numpy as np
         dev = self.device
-        if dev.type != "cuda":
-            raise RuntimeError("generate_csr needs a CUDA device (no host fallback)")
-        z32 = torch.as_tensor(z32, dtype=torch.float32).to(dev)
-        r32 = torch.as_tensor(r32, dtype=torch.float32).to(dev)
-        n = int(z32.shape[0])
-        if tuple(z32.shape) != (n, self.Z) or tuple(r32.shape) != (n, self.Z):
-            raise ValueError(f"generate_csr: z32 / r32 must both be [n, {self.Z}]")
-        tile_rows = int(tile_rows)
-        if tile_rows < 1:
-            raise ValueError("generate_csr: tile_rows must be >= 1")
+        tile_rows = self._tiling("generate_csr", tile_rows)
+        z32, r32 = self._latents("generate_csr", z32, r32)
+        n = z32.shape[0]
         parts = None
         if consume is None:
             rowptr_out = np.zeros(n + 1, dtype=np.int64)
@@ -2112,11 +2170,9 @@ class BiGanEngine:
             copied[slot].synchronize()
             consume(row0, rp, stage[slot][0][:nnz], stage[slot][1][:nnz])
 
-        for i, s in enumerate(range(0, n, T)):
-            m, slot = min(T, n - s), i % 2
-            self.set_latents(z32[s:s + m], r32[s:s + m], m)
-            self.generate(m, out32=tile[:m])
-            ops.round_csr_count(tile[:m], rowptr_d[:m + 1])
+        for i, (s, m, x) in enumerate(self._generated_tiles(z32, r32, T, tile)):
+            slot = i % 2
+            ops.round_csr_count(x, rowptr_d[:m + 1])
             rowptr_h[:m + 1].copy_(rowptr_d[:m + 1], non_blocking=True)
             counted = torch.cuda.Event()
             counted.record(main)
@@ -2131,7 +2187,7 @@ class BiGanEngine:
                 cap = max(nnz, 1)
                 ent_d = (torch.empty(cap, dtype=torch.int32, device=dev),
                          torch.empty(cap, dtype=torch.float32, device=dev))
-            ops.round_csr_fill(tile[:m], rowptr_d[:m + 1], ent_d[0][:nnz], ent_d[1][:nnz])
+            ops.round_csr_fill(x, rowptr_d[:m + 1], ent_d[0][:nnz], ent_d[1][:nnz])
             filled = torch.cuda.Event()
             filled.record(main)
             if stage[slot] is None or stage[slot][0].numel() < nnz:
@@ -2158,25 +2214,24 @@ class BiGanEngine:
         return rowptr_out, colidx, values
 
     def score_stream(self, rowptr, colidx, values, row_begin, row_end, r32, enc_out, mse_out,
-                     d_out, tile_rows=GENERATE_TILE):
+                     d_out, tile_rows=None):
         """Per-cell scores of rows [row_begin, row_end) of a device CSR with gene_size columns:
             enc_out[i] = E.predict(x)                      ([n, Z] fp32, device)
             mse_out[i] = mean_c (G.predict(z, r) - x)^2    ([n] fp32, device; G's fp32 output
                                                             against the exact fp32 counts)
             d_out[i]   = D.predict(z, x)                   ([n] or [n, 1] fp32, device)
         with z = enc_out[i] and r = r32[i] ([n, Z] fp32, host or device).  Per tile of
-        `tile_rows` rows from row_begin (the tiling of E / G / D.predict, so the bits match):
-        encode_stream into z, set_latents(z, r) + generate() into one fp32 tile,
-        cc_recon_sqerr with scale 1 / gene_size, cc_gather_rows into one bf16 cell tile, and
-        discriminate(z, x).  Device memory: those two tiles and the nets' activations for
-        tile_rows rows; nothing of size (n, genes).
+        `tile_rows` rows from row_begin (the tiling of E / G / D.predict, so the bits match;
+        see _generated_tiles): encode_stream into z, set_latents(z, r) + generate() into one
+        fp32 tile, cc_recon_sqerr with scale 1 / gene_size, cc_gather_rows into one bf16 cell
+        tile (_real_tiles), and discriminate(z, x).  Device memory: those two tiles and the
+        nets' activations for tile_rows rows; nothing of size (n, genes).
 
         Engine state (weights, BN statistics, RNG counter, loss_buf) is not touched; every
         forward orders itself after pending side-stream optimiser updates of its net, and the
         pass issues no collective."""
         dev = self.device
-        if dev.type != "cuda":
-            raise RuntimeError("score_stream needs a CUDA device (no host fallback)")
+        tile_rows = self._tiling("score_stream", tile_rows)
         row_begin, row_end = int(row_begin), int(row_end)
         n = row_end - row_begin
         if row_begin < 0 or n < 0 or row_end > rowptr.shape[0] - 1:
@@ -2187,14 +2242,12 @@ class BiGanEngine:
             raise ValueError(f"score_stream: r32 and enc_out must be [{n}, {self.Z}]")
         if mse_out.numel() != n or d_out.numel() != n:
             raise ValueError(f"score_stream: mse_out and d_out must hold {n} values")
-        tile_rows = int(tile_rows)
-        if tile_rows < 1:
-            raise ValueError("score_stream: tile_rows must be >= 1")
         if n == 0:
             return
         T = min(tile_rows, n)
         pred = ops.alloc2d(T, self.Gn, dtype=torch.float32, device=dev, zero=False)
-        cells = ops.alloc2d(T, self.Gn, device=dev)     # zero padding, like the predict tiles
+        cells = self._real_tiles((rowptr, colidx, values), (row_begin, row_end),
+                                 ops.alloc2d(T, self.Gn, device=dev))   # zero padding
         mse, d = mse_out.view(n), d_out.view(n, 1)
         for s in range(0, n, T):
             m, row = min(T, n - s), row_begin + s
@@ -2204,12 +2257,11 @@ class BiGanEngine:
             self.generate(m, out32=pred[:m])
             ops.recon_sqerr(pred[:m], rowptr, colidx, values, row, mse[s:s + m],
                             scale=1.0 / self.Gn)
-            ops.gather_rows(rowptr, colidx, values, self.Gn, row_start=row, n_rows=m,
-                            out16=cells[:m])
-            self.discriminate(z, cells[:m], d[s:s + m])
+            _, _, x = next(cells)           # the gather of these rows, after the generator
+            self.discriminate(z, x, d[s:s + m])
 
     def moments_stream(self, bounds, *, csr=None, order=None, z32=None, r32=None,
-                       tile_rows=GENERATE_TILE):
+                       tile_rows=None):
         """Per-group column moments of real or generated cells, for K groups given by `bounds`
         (K + 1 non-decreasing host ints from 0) -> device tensors
             sum     [K, gene_size] fp64   sum over the group's cells of v
@@ -2218,76 +2270,48 @@ class BiGanEngine:
         Real cells: csr = (rowptr, colidx, values) of a device CSR with gene_size columns and
         `order` (host or device int64) its row numbers sorted by group; group k is the rows
         order[bounds[k]:bounds[k + 1]] and v the exact fp32 count.  Per tile of at most
-        tile_rows positions of one group: cc_gather_rows(row_idx=...) into the fp32 tile, then
-        cc_col_moments into that group's accumulators.
+        tile_rows positions of one group (_real_tiles into the fp32 tile): cc_col_moments into
+        that group's accumulators.
         Generated cells: z32 / r32 ([n, Z] fp32, host or device, n = bounds[-1]) sorted by
         group; group k is rows [bounds[k], bounds[k + 1]) and v = rint(G.predict(z, r)).  Per
-        tile of tile_rows rows from row 0 (the tiling of G.predict, whose split-K depends on
-        the row count, so the cells are generate_cells' bit for bit): set_latents + generate()
-        into the fp32 tile, then one cc_col_moments(round_half_even=1) per group segment inside
-        the tile.
+        generated tile (_generated_tiles into the fp32 tile, so the cells are generate_cells'
+        bit for bit): one cc_col_moments(round_half_even=1) per group segment inside the tile.
         Device memory: the fp32 tile, the accumulators and the cc_col_moments workspace;
         nothing of size (n, genes).  Engine state (weights, BN statistics, RNG counter,
         loss_buf) is not touched; the generator forward orders itself after pending side-stream
         optimiser updates, and the pass issues no collective."""
         dev = self.device
-        if dev.type != "cuda":
-            raise RuntimeError("moments_stream needs a CUDA device (no host fallback)")
+        tile_rows = self._tiling("moments_stream", tile_rows)
         bounds = [int(b) for b in bounds]
         K = len(bounds) - 1
         if K < 1 or bounds[0] != 0 or any(b > e for b, e in zip(bounds, bounds[1:])):
             raise ValueError("moments_stream: bounds must be K + 1 >= 2 non-decreasing "
                              "offsets from 0")
-        if (csr is None) == (z32 is None):
-            raise ValueError("moments_stream: give either csr and order (real cells) or z32 "
-                             "and r32 (generated cells)")
-        n = bounds[-1]
-        tile_rows = int(tile_rows)
-        if tile_rows < 1:
-            raise ValueError("moments_stream: tile_rows must be >= 1")
+        n, order, z32, r32 = self._cells("moments_stream", csr, order, z32, r32, bounds[-1])
         Gn = self.Gn
         sums = torch.zeros((K, Gn), dtype=torch.float64, device=dev)
         sumsq = torch.zeros((K, Gn), dtype=torch.float64, device=dev)
         nonzero = torch.zeros((K, Gn), dtype=torch.int64, device=dev)
-        if csr is not None:
-            rowptr, colidx, values = csr
-            order = torch.as_tensor(order, dtype=torch.int64).to(dev)
-            if order.dim() != 1 or order.numel() != n:
-                raise ValueError(f"moments_stream: order must hold bounds[-1] = {n} row numbers")
-            T = max(1, min(tile_rows, max((e - b for b, e in zip(bounds, bounds[1:])),
-                                          default=1)))
-        else:
-            z32 = torch.as_tensor(z32, dtype=torch.float32).to(dev)
-            r32 = torch.as_tensor(r32, dtype=torch.float32).to(dev)
-            if tuple(z32.shape) != (n, self.Z) or tuple(r32.shape) != (n, self.Z):
-                raise ValueError(f"moments_stream: z32 / r32 must both be [{n}, {self.Z}]")
-            T = max(1, min(tile_rows, n))
         if n == 0:
             return sums, sumsq, nonzero
+        T = min(tile_rows, n if csr is None else max(e - b for b, e in zip(bounds, bounds[1:])))
         tile = ops.alloc2d(T, Gn, dtype=torch.float32, device=dev, zero=False)
         ws_bytes = ops.col_moments_ws_bytes(T, Gn)
         ws = torch.zeros(ws_bytes, dtype=torch.uint8, device=dev) if ws_bytes else None
         if csr is not None:
             for k in range(K):
-                for s in range(bounds[k], bounds[k + 1], T):
-                    m = min(T, bounds[k + 1] - s)
-                    ops.gather_rows(rowptr, colidx, values, Gn, row_idx=order[s:s + m],
-                                    out32=tile[:m])
-                    ops.col_moments(tile[:m], sums[k], sumsq[k], nonzero[k], ws=ws)
+                for _, _, x in self._real_tiles(csr, order[bounds[k]:bounds[k + 1]], tile):
+                    ops.col_moments(x, sums[k], sumsq[k], nonzero[k], ws=ws)
             return sums, sumsq, nonzero
-        for s in range(0, n, T):
-            m = min(T, n - s)
-            self.set_latents(z32[s:s + m], r32[s:s + m], m)
-            self.generate(m, out32=tile[:m])
+        for s, m, x in self._generated_tiles(z32, r32, tile_rows, tile):
             for k in range(K):
                 lo, hi = max(bounds[k], s), min(bounds[k + 1], s + m)
                 if lo < hi:
-                    ops.col_moments(tile[lo - s:hi - s], sums[k], sumsq[k], nonzero[k],
+                    ops.col_moments(x[lo - s:hi - s], sums[k], sumsq[k], nonzero[k],
                                     round=True, ws=ws)
         return sums, sumsq, nonzero
 
-    def features_stream(self, *, csr=None, order=None, z32=None, r32=None,
-                        tile_rows=GENERATE_TILE):
+    def features_stream(self, *, csr=None, order=None, z32=None, r32=None, tile_rows=None):
         """log1p features of real or generated cells -> device tensors
             features       [n, gene_size] bf16  view of a [n, pad_ld(gene_size)] buffer whose
                                                 padding columns are zero (a GEMM operand)
@@ -2295,50 +2319,24 @@ class BiGanEngine:
             genes_detected [n] int32            #{genes : v != 0}
         with features = bf16(float(log1p(double(v)))) (cc_log1p_features).  The two modes of
         moments_stream: real cells are the rows `order` (host or device int64) of the device CSR
-        `csr`, gathered tile by tile with cc_gather_rows(row_idx=...), v the exact fp32 count;
-        generated cells are the rows of z32 / r32 ([n, Z] fp32), v = rint(G.predict(z, r)),
-        tiled from row 0 like G.predict, so they are generate_cells' cells bit for bit.
-        Device memory: one fp32 tile and the outputs.  Engine state is not touched and no
-        collective is issued."""
+        `csr` (_real_tiles), v the exact fp32 count; generated cells are the rows of z32 / r32
+        ([n, Z] fp32), v = rint(G.predict(z, r)) (_generated_tiles, so they are generate_cells'
+        cells bit for bit).  Device memory: one fp32 tile and the outputs.  Engine state is not
+        touched and no collective is issued."""
         dev = self.device
-        if dev.type != "cuda":
-            raise RuntimeError("features_stream needs a CUDA device (no host fallback)")
-        if (csr is None) == (z32 is None):
-            raise ValueError("features_stream: give either csr and order (real cells) or z32 "
-                             "and r32 (generated cells)")
-        if csr is not None:
-            order = torch.as_tensor(order, dtype=torch.int64).to(dev)
-            if order.dim() != 1:
-                raise ValueError("features_stream: order must be a vector of row numbers")
-            n = order.numel()
-        else:
-            z32 = torch.as_tensor(z32, dtype=torch.float32).to(dev)
-            r32 = torch.as_tensor(r32, dtype=torch.float32).to(dev)
-            n = z32.shape[0]
-            if z32.dim() != 2 or tuple(z32.shape) != (n, self.Z) or tuple(r32.shape) != (n, self.Z):
-                raise ValueError(f"features_stream: z32 / r32 must both be [n, {self.Z}]")
-        tile_rows = int(tile_rows)
-        if tile_rows < 1:
-            raise ValueError("features_stream: tile_rows must be >= 1")
-        Gn = self.Gn
-        feats = ops.alloc2d(n, Gn, dtype=torch.bfloat16, device=dev, zero=False)
+        tile_rows = self._tiling("features_stream", tile_rows)
+        n, order, z32, r32 = self._cells("features_stream", csr, order, z32, r32)
+        feats = ops.alloc2d(n, self.Gn, dtype=torch.bfloat16, device=dev, zero=False)
         lib = torch.zeros(n, dtype=torch.float64, device=dev)
         det = torch.zeros(n, dtype=torch.int32, device=dev)
         if n == 0:
             return feats, lib, det
-        T = max(1, min(tile_rows, n))
-        tile = ops.alloc2d(T, Gn, dtype=torch.float32, device=dev, zero=False)
-        for s in range(0, n, T):
-            m = min(T, n - s)
-            if csr is not None:
-                rowptr, colidx, values = csr
-                ops.gather_rows(rowptr, colidx, values, Gn, row_idx=order[s:s + m],
-                                out32=tile[:m])
-            else:
-                self.set_latents(z32[s:s + m], r32[s:s + m], m)
-                self.generate(m, out32=tile[:m])
-            ops.log1p_features(tile[:m], feats[s:s + m], lib[s:s + m], det[s:s + m],
-                               round=csr is None)
+        tile = ops.alloc2d(min(tile_rows, n), self.Gn, dtype=torch.float32, device=dev,
+                           zero=False)
+        tiles = (self._real_tiles(csr, order, tile) if csr is not None
+                 else self._generated_tiles(z32, r32, tile_rows, tile))
+        for s, m, x in tiles:
+            ops.log1p_features(x, feats[s:s + m], lib[s:s + m], det[s:s + m], round=csr is None)
         return feats, lib, det
 
     MEDIAN_ROWS = 1024        # rows of d^2 formed at a time for the median

@@ -155,12 +155,12 @@ def _cells(n, G, seed, per_row=60, scale=1):
 
 @pytest.mark.parametrize("variant", ["cont", "classify"])
 def test_two_sample_test_streams_the_definition(variant):
-    """33,694 genes; a generator tile of 1,024 rows here (PREDICT_TILE is what generate_cells
-    and the stream both tile by), so generation crosses tiles while the host definition stays
-    affordable"""
+    """33,694 genes; a generator tile of 1,024 rows here (the engine's PREDICT_TILE is what
+    generate_cells and the stream both tile by), so generation crosses tiles while the host
+    definition stays affordable"""
     G, n, P = 33694, 1500, 40
     net = _expressive(_net(variant, G, seed=5))
-    net.PREDICT_TILE = 1024
+    net._engine.PREDICT_TILE = 1024
     mat = _cells(n, G, 7)
     state = net._prior_rng.bit_generator.state
     np_state = np.random.get_state()
